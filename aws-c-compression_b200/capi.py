@@ -15,6 +15,9 @@ AWS_ERROR_COMPRESSION_DEVICE_FAILURE = 3073
 AWS_ERROR_COMPRESSION_INVALID_CODE_TABLE = 3074
 AWS_ERROR_COMPRESSION_INVALID_PADDING = 3075
 HPACK_HUFFMAN_SMALLEST, HPACK_HUFFMAN_NEVER, HPACK_HUFFMAN_ALWAYS = 0, 1, 2
+# enum aws_hpack_field_kind
+(HPACK_FIELD_INDEXED, HPACK_FIELD_LITERAL_INCREMENTAL, HPACK_FIELD_LITERAL_WITHOUT_INDEXING,
+ HPACK_FIELD_LITERAL_NEVER_INDEXED, HPACK_FIELD_TABLE_SIZE_UPDATE) = range(5)
 
 
 class CodecError(RuntimeError):
@@ -78,6 +81,20 @@ class aws_huffman_batch(C.Structure):
     ]
 
 
+class aws_hpack_header_lists(C.Structure):
+    _fields_ = [
+        ("n", C.c_size_t),
+        ("field_offsets", C.c_void_p),
+        ("field_capacity", C.c_uint64),
+        ("field_kind", C.c_void_p),
+        ("field_index", C.c_void_p),
+        ("never_indexed", C.c_void_p),
+        ("strings", C.c_void_p),
+        ("strings_capacity", C.c_uint64),
+        ("string_offsets", C.c_void_p),
+    ]
+
+
 class aws_huffman_table_coder(C.Structure):
     _fields_ = [("coder", aws_huffman_symbol_coder), ("codes", aws_huffman_code * 256),
                 ("lut_entries", C.c_void_p), ("lut_count", C.c_uint32), ("lut_root_bits", C.c_uint8)]
@@ -128,6 +145,8 @@ EXPORTED_SYMBOLS = [
     "aws_huffman_encode_batch_multi", "aws_huffman_decode_batch_multi", "aws_huffman_batch_ctx_synchronize",
     "aws_huffman_batch_ctx_stream", "aws_huffman_batch_ctx_device", "aws_huffman_batch_ctx_launch_count",
     "aws_huffman_batch_plan_shards", "aws_huffman_batch_concat_offsets",
+    "aws_hpack_header_block_decode_batch", "aws_hpack_header_block_encode_batch",
+    "aws_hpack_header_block_decode_batch_device", "aws_hpack_header_block_encode_batch_device",
 ]
 
 
@@ -218,6 +237,18 @@ class Library:
         L.aws_huffman_batch_plan_shards.restype = C.c_int
         L.aws_huffman_batch_concat_offsets.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]
         L.aws_huffman_batch_concat_offsets.restype = C.c_int
+        L.aws_hpack_header_block_decode_batch.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p,
+                                                          P(aws_hpack_header_lists), C.c_void_p]
+        L.aws_hpack_header_block_encode_batch.argtypes = [C.c_void_p, P(aws_hpack_header_lists), C.c_int, C.c_void_p,
+                                                          C.c_uint64, C.c_void_p]
+        L.aws_hpack_header_block_decode_batch_device.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_uint64,
+                                                                 P(aws_hpack_header_lists), C.c_void_p, C.c_void_p]
+        L.aws_hpack_header_block_encode_batch_device.argtypes = [C.c_void_p, P(aws_hpack_header_lists), C.c_uint64,
+                                                                 C.c_uint64, C.c_int, C.c_void_p, C.c_uint64, C.c_void_p,
+                                                                 C.c_void_p]
+        for name in ("aws_hpack_header_block_decode_batch", "aws_hpack_header_block_encode_batch",
+                     "aws_hpack_header_block_decode_batch_device", "aws_hpack_header_block_encode_batch_device"):
+            getattr(L, name).restype = C.c_int
 
     def last_error(self):
         return self.lib.aws_last_error()
@@ -516,6 +547,72 @@ class BatchContext:
                     _ptr(out_offsets), _ptr(status), stream or 0)
         if rc != 0:
             raise CodecError(self.library.last_error(), "aws_hpack_string_%s_batch_device" % ("encode" if encode else "decode"))
+
+    # ---- HPACK header blocks (hpack_header_block_batch.h) ----
+    def _blocks_call(self, fn_name, *args):
+        rc = getattr(self.library.lib, fn_name)(self.handle, *args)
+        if rc != 0:
+            raise CodecError(self.library.last_error(), fn_name)
+
+    def hpack_decode_blocks(self, data, in_offsets, field_capacity=None, strings_capacity=None):
+        """Host buffers. Capacities default to the documented bounds (in_size fields, 28 * in_size octets). On
+        failure the CodecError carries the arrays as `result` (offsets are complete on AWS_ERROR_SHORT_BUFFER)."""
+        data = np.ascontiguousarray(data, dtype=np.uint8)
+        in_offsets = np.ascontiguousarray(in_offsets, dtype=np.uint64)
+        n = len(in_offsets) - 1
+        in_size = int(in_offsets[-1])
+        field_capacity = in_size if field_capacity is None else int(field_capacity)
+        strings_capacity = 28 * in_size if strings_capacity is None else int(strings_capacity)
+        res = {"field_offsets": np.zeros(n + 1, dtype=np.uint64), "field_kind": np.zeros(max(field_capacity, 1), np.uint8),
+               "field_index": np.zeros(max(field_capacity, 1), np.uint64),
+               "strings": np.zeros(max(strings_capacity, 1), np.uint8),
+               "string_offsets": np.zeros(2 * field_capacity + 1, np.uint64), "status": np.zeros(n, np.int32)}
+        lists = aws_hpack_header_lists(n, _ptr(res["field_offsets"]), field_capacity, _ptr(res["field_kind"]),
+                                       _ptr(res["field_index"]), None, _ptr(res["strings"]), strings_capacity,
+                                       _ptr(res["string_offsets"]))
+        try:
+            self._blocks_call("aws_hpack_header_block_decode_batch", n, _ptr(data), _ptr(in_offsets), C.byref(lists),
+                              _ptr(res["status"]))
+        except CodecError as err:
+            err.result = res
+            raise
+        return res
+
+    def hpack_encode_blocks(self, field_offsets, strings, string_offsets, out_capacity, mode=HPACK_HUFFMAN_SMALLEST,
+                            never_indexed=None):
+        """Host buffers: header lists in, header blocks out ({"out", "out_offsets"})."""
+        field_offsets = np.ascontiguousarray(field_offsets, dtype=np.uint64)
+        strings = np.ascontiguousarray(strings, dtype=np.uint8)
+        string_offsets = np.ascontiguousarray(string_offsets, dtype=np.uint64)
+        if never_indexed is not None:
+            never_indexed = np.ascontiguousarray(never_indexed, dtype=np.uint8)
+        n = len(field_offsets) - 1
+        res = {"out": np.zeros(max(int(out_capacity), 1), dtype=np.uint8), "out_offsets": np.zeros(n + 1, dtype=np.uint64)}
+        lists = aws_hpack_header_lists(n, _ptr(field_offsets), 0, None, None, _ptr(never_indexed), _ptr(strings), 0,
+                                       _ptr(string_offsets))
+        try:
+            self._blocks_call("aws_hpack_header_block_encode_batch", C.byref(lists), mode, _ptr(res["out"]),
+                              int(out_capacity), _ptr(res["out_offsets"]))
+        except CodecError as err:
+            err.result = res
+            raise
+        return res
+
+    def hpack_decode_blocks_device(self, n, in_, in_offsets, in_size, field_offsets, field_kind, field_index, strings,
+                                   string_offsets, status=None, stream=None):
+        """Torch CUDA tensors; capacities are the tensors' sizes (string_offsets: 2 * field_capacity + 1)."""
+        field_capacity = (string_offsets.numel() - 1) // 2
+        lists = aws_hpack_header_lists(n, _ptr(field_offsets), field_capacity, _ptr(field_kind), _ptr(field_index), None,
+                                       _ptr(strings), strings.numel(), _ptr(string_offsets))
+        self._blocks_call("aws_hpack_header_block_decode_batch_device", n, _ptr(in_), _ptr(in_offsets), int(in_size),
+                          C.byref(lists), _ptr(status), stream or 0)
+
+    def hpack_encode_blocks_device(self, n, field_offsets, num_fields, strings, string_offsets, strings_size, out,
+                                   out_offsets, mode=HPACK_HUFFMAN_SMALLEST, never_indexed=None, stream=None):
+        lists = aws_hpack_header_lists(n, _ptr(field_offsets), 0, None, None, _ptr(never_indexed), _ptr(strings), 0,
+                                       _ptr(string_offsets))
+        self._blocks_call("aws_hpack_header_block_encode_batch_device", C.byref(lists), int(num_fields),
+                          int(strings_size), mode, _ptr(out), out.numel(), _ptr(out_offsets), stream or 0)
 
     def encode(self, data, in_offsets, out_capacity, **kw):
         return self._host(True, data, in_offsets, out_capacity, **kw)

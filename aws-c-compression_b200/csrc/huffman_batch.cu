@@ -6,6 +6,7 @@
 // AWS_ERROR_COMPRESSION_DEVICE_FAILURE.
 #include <aws/compression/huffman_batch.h>
 #include <aws/compression/hpack_string_batch.h>
+#include <aws/compression/hpack_header_block_batch.h>
 #include <aws/compression/huffman_table_builder.h>
 
 #include "../host/huffman_lut.h"
@@ -15,6 +16,7 @@
 #include "encode_slots.cuh"
 #include "encode_strings.cuh"
 #include "hpack_literals.cuh"
+#include "hpack_blocks.cuh"
 #include "decode_fast.cuh"
 #include "decode_rows.cuh"
 #include "decode_slots.cuh"
@@ -109,6 +111,26 @@ struct Lane {
         stream = nullptr;
     }
 };
+// HPACK header blocks (hpack_blocks.cuh): per-block counts and bases, parsed fields, literal spans and the decoded
+// literals, encode plans, and the staging of the host entry points' extra arrays.
+struct BlockBufs {
+    GrowBuf num_fields, num_lits, lit_bytes, struct_status, out_fields, status, field_base, lit_base, lit_byte_base,
+        f_kind, f_index, f_block, f_lits, lit_src, lit_offsets, lits, dec, dec_offsets, lit_status, str_lens, plan,
+        plan_index, field_lens, field_pos, framed, framed_offsets, s_field_offsets, s_never, s_kind, s_index,
+        s_string_offsets;
+    uint64_t *h_totals = nullptr;  // pinned: fields, literals, literal octets
+    void release() {
+        GrowBuf *all[] = {&num_fields, &num_lits,      &lit_bytes,  &struct_status, &out_fields,      &status,
+                          &field_base, &lit_base,      &lit_byte_base, &f_kind,     &f_index,         &f_block,
+                          &f_lits,     &lit_src,       &lit_offsets, &lits,         &dec,             &dec_offsets,
+                          &lit_status, &str_lens,      &plan,       &plan_index,    &field_lens,      &field_pos,
+                          &framed,     &framed_offsets, &s_field_offsets, &s_never, &s_kind,          &s_index,
+                          &s_string_offsets};
+        for (GrowBuf *g : all) g->release();
+        if (h_totals) cudaFreeHost(h_totals);
+        h_totals = nullptr;
+    }
+};
 }  // namespace hb_host
 using hb_host::GrowBuf;
 using hb_host::Lane;
@@ -140,6 +162,7 @@ struct aws_huffman_batch_ctx {
     // HPACK string literals (hpack_literals.cuh): packed payloads between the framing and the codec, per-item plans
     GrowBuf hp_pay, hp_pay_off, hp_dec, hp_dec_off, hp_huff, hp_prefix, hp_lens, hp_pay_lens, hp_dec_status, hp_left_bits,
         hp_left_num, hp_status;
+    hb_host::BlockBufs blk;
     uint64_t *h_scalar = nullptr;  // pinned
     // The *_device entry points enqueue on the caller's stream but share ctx->scratch (tile descriptors, ...).
     // `scratch_free` is recorded after every such call; a call on ANOTHER stream waits for it first, so two calls
@@ -1360,6 +1383,290 @@ int hpack_run_host(
 }
 
 // ---------------------------------------------------------------------------------------------
+// HPACK header blocks (hpack_blocks.cuh) over the literal layer above. Device pointers in, device pointers out.
+// ---------------------------------------------------------------------------------------------
+// Device pointers of an aws_hpack_header_lists (decode side).
+struct BlockLists {
+    uint64_t *field_offsets;
+    uint64_t field_capacity;
+    uint8_t *kind;
+    uint64_t *index;
+    uint8_t *strings;
+    uint64_t strings_capacity;
+    uint64_t *string_offsets;
+};
+
+inline unsigned grid_of(uint64_t items, uint64_t per_block) { return (unsigned)std::max<uint64_t>(1, (items + per_block - 1) / per_block); }
+
+// stage: `o` holds host pointers' shapes only; the per-field outputs go to context staging sized from the totals
+// (the host entry point copies them back).
+int hpack_blocks_decode_on_device(
+    aws_huffman_batch_ctx *ctx, uint64_t n, const uint8_t *in, const uint64_t *in_off, BlockLists o, int32_t *status,
+    bool stage, cudaStream_t st) {
+    hb_host::BlockBufs &B = ctx->blk;
+    if (n == 0) {
+        HB_CUDA_TRY(cudaMemsetAsync(o.field_offsets, 0, sizeof(uint64_t), st));
+        if (o.string_offsets && !stage) HB_CUDA_TRY(cudaMemsetAsync(o.string_offsets, 0, sizeof(uint64_t), st));
+        return AWS_OP_SUCCESS;
+    }
+    const unsigned flat = grid_of(n, 256);
+    HB_CUDA_TRY(B.num_fields.reserve(n * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.num_lits.reserve(n * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.lit_bytes.reserve(n * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.out_fields.reserve(n * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.struct_status.reserve(n * sizeof(int32_t)));
+    HB_CUDA_TRY(B.field_base.reserve((n + 1) * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.lit_base.reserve((n + 1) * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.lit_byte_base.reserve((n + 1) * sizeof(uint64_t)));
+    if (!status) {
+        HB_CUDA_TRY(B.status.reserve(n * sizeof(int32_t)));
+        status = B.status.as<int32_t>();
+    }
+    if (!B.h_totals) HB_CUDA_TRY(cudaHostAlloc(reinterpret_cast<void **>(&B.h_totals), 3 * sizeof(uint64_t), cudaHostAllocDefault));
+    uint64_t *field_base = B.field_base.as<uint64_t>(), *lit_base = B.lit_base.as<uint64_t>();
+    uint64_t *lit_byte_base = B.lit_byte_base.as<uint64_t>();
+
+    // 1. structure, counts; 2. their bases, and the totals the later launches are sized from
+    hb::hpack_block_scan_kernel<<<flat, 256, 0, st>>>(
+        n, in, in_off, B.num_fields.as<uint64_t>(), B.num_lits.as<uint64_t>(), B.lit_bytes.as<uint64_t>(), B.struct_status.as<int32_t>());
+    ++ctx->launches;
+    if (launch_scan(ctx, ctx->scratch, B.num_fields.as<uint64_t>(), field_base, n, st)) return AWS_OP_ERR;
+    if (launch_scan(ctx, ctx->scratch, B.num_lits.as<uint64_t>(), lit_base, n, st)) return AWS_OP_ERR;
+    if (launch_scan(ctx, ctx->scratch, B.lit_bytes.as<uint64_t>(), lit_byte_base, n, st)) return AWS_OP_ERR;
+    HB_CUDA_TRY(cudaMemcpyAsync(B.h_totals + 0, field_base + n, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    HB_CUDA_TRY(cudaMemcpyAsync(B.h_totals + 1, lit_base + n, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    HB_CUDA_TRY(cudaMemcpyAsync(B.h_totals + 2, lit_byte_base + n, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    HB_CUDA_TRY(cudaStreamSynchronize(st));
+    const uint64_t parsed = B.h_totals[0], num_lits = B.h_totals[1], lit_total = B.h_totals[2];
+    const uint64_t kept = std::min(parsed, o.field_capacity);  // field slots that can be written
+    const uint32_t min_len = std::max<uint32_t>(1, ctx->tables.min_len);
+    const uint64_t dec_cap = lit_total * 8 / min_len + 64;
+    if (stage) {
+        // (a field's strings are its decoded literals or at most 28 octets of Appendix A)
+        o.strings_capacity = std::min(o.strings_capacity, dec_cap + 28 * kept);
+        HB_CUDA_TRY(B.s_kind.reserve(kept + 1));
+        HB_CUDA_TRY(B.s_index.reserve((kept + 1) * sizeof(uint64_t)));
+        HB_CUDA_TRY(B.s_string_offsets.reserve((2 * kept + 1) * sizeof(uint64_t)));
+        HB_CUDA_TRY(ctx->s_out.reserve(o.strings_capacity + 16));
+        o.kind = B.s_kind.as<uint8_t>();
+        o.index = B.s_index.as<uint64_t>();
+        o.string_offsets = B.s_string_offsets.as<uint64_t>();
+        o.strings = ctx->s_out.as<uint8_t>();
+    }
+    HB_CUDA_TRY(B.f_kind.reserve(parsed + 1));
+    HB_CUDA_TRY(B.f_index.reserve((parsed + 1) * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.f_block.reserve((parsed + 1) * sizeof(uint32_t)));
+    HB_CUDA_TRY(B.f_lits.reserve((2 * parsed + 1) * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.lit_src.reserve((num_lits + 1) * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.lit_offsets.reserve((num_lits + 1) * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.lit_status.reserve((num_lits + 1) * sizeof(int32_t)));
+    HB_CUDA_TRY(B.dec_offsets.reserve((num_lits + 1) * sizeof(uint64_t)));
+    uint8_t *f_kind = B.f_kind.as<uint8_t>();
+    uint64_t *f_index = B.f_index.as<uint64_t>(), *f_lits = B.f_lits.as<uint64_t>();
+    uint32_t *f_block = B.f_block.as<uint32_t>();
+    uint64_t *dec_offsets = B.dec_offsets.as<uint64_t>();
+    int32_t *lit_status = B.lit_status.as<int32_t>();
+
+    // 3. field records and literal spans in parsed order; 4. the literals, packed; 5. decoded by the literal path
+    if (parsed || num_lits) {
+        hb::hpack_block_split_kernel<<<flat, 256, 0, st>>>(
+            n, in, in_off, field_base, lit_base, lit_byte_base, f_kind, f_index, f_block, f_lits, B.lit_src.as<uint64_t>(),
+            B.lit_offsets.as<uint64_t>());
+        ++ctx->launches;
+    }
+    if (num_lits) {
+        HB_CUDA_TRY(B.lits.reserve(lit_total + 64));
+        HB_CUDA_TRY(B.dec.reserve(dec_cap + 64));
+        hb::hpack_lit_gather_kernel<<<grid_of(num_lits, 256), 256, 0, st>>>(
+            num_lits, in, B.lit_src.as<uint64_t>(), B.lit_offsets.as<uint64_t>(), B.lits.as<uint8_t>());
+        ++ctx->launches;
+        if (hpack_decode_on_device(ctx, num_lits, B.lits.as<uint8_t>(), B.lit_offsets.as<uint64_t>(), lit_total,
+                                   B.dec.as<uint8_t>(), dec_cap, dec_offsets, lit_status, st))
+            return AWS_OP_ERR;
+    }
+    // 6. final status per block, field offsets; 7. records, string lengths, string offsets, strings
+    hb::hpack_block_finish_kernel<<<flat, 256, 0, st>>>(
+        n, lit_base, lit_status, B.struct_status.as<int32_t>(), B.num_fields.as<uint64_t>(), status, B.out_fields.as<uint64_t>());
+    ++ctx->launches;
+    if (launch_scan(ctx, ctx->scratch, B.out_fields.as<uint64_t>(), o.field_offsets, n, st)) return AWS_OP_ERR;
+    if (!kept) {
+        HB_CUDA_TRY(cudaMemsetAsync(o.string_offsets, 0, sizeof(uint64_t), st));
+        HB_CUDA_TRY(cudaGetLastError());
+        return AWS_OP_SUCCESS;
+    }
+    HB_CUDA_TRY(B.str_lens.reserve(2 * kept * sizeof(uint64_t)));
+    HB_CUDA_TRY(cudaMemsetAsync(B.str_lens.ptr, 0, 2 * kept * sizeof(uint64_t), st));
+    const uint8_t *dec = B.dec.as<uint8_t>();
+    hb::hpack_field_records_kernel<<<grid_of(parsed, 256), 256, 0, st>>>(
+        parsed, f_kind, f_index, f_block, f_lits, field_base, status, o.field_offsets, o.field_capacity, dec, dec_offsets,
+        o.kind, o.index, B.str_lens.as<uint64_t>());
+    ++ctx->launches;
+    if (launch_scan(ctx, ctx->scratch, B.str_lens.as<uint64_t>(), o.string_offsets, 2 * kept, st)) return AWS_OP_ERR;
+    hb::hpack_compose_kernel<<<grid_of(2 * parsed, 256), 256, 0, st>>>(
+        parsed, f_kind, f_index, f_block, f_lits, field_base, status, o.field_offsets, o.field_capacity, dec, dec_offsets,
+        o.strings, o.strings_capacity, o.string_offsets);
+    ++ctx->launches;
+    HB_CUDA_TRY(cudaGetLastError());
+    return AWS_OP_SUCCESS;
+}
+
+int hpack_blocks_encode_on_device(
+    aws_huffman_batch_ctx *ctx, uint64_t n, const uint64_t *field_offsets, uint64_t num_fields, const uint8_t *never_indexed,
+    const uint8_t *strings, const uint64_t *string_offsets, uint64_t strings_size, uint32_t mode, uint8_t *out,
+    uint64_t out_capacity, uint64_t *out_offsets, cudaStream_t st) {
+    hb_host::BlockBufs &B = ctx->blk;
+    if (n == 0 || num_fields == 0) {
+        HB_CUDA_TRY(cudaMemsetAsync(out_offsets, 0, (n + 1) * sizeof(uint64_t), st));
+        return AWS_OP_SUCCESS;
+    }
+    const uint64_t F = num_fields;
+    // framed names and values: raw or Huffman, whichever `mode` picks, behind a prefix of at most 10 octets
+    const uint64_t expand = mode == hb::kHpackAlways ? (std::max<uint32_t>(1, ctx->tables.max_len) + 7) / 8 : 1;
+    const uint64_t framed_cap = strings_size * expand + 2 * F * 10 + 64;
+    HB_CUDA_TRY(B.framed.reserve(framed_cap + 64));
+    HB_CUDA_TRY(B.framed_offsets.reserve((2 * F + 1) * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.plan.reserve(F));
+    HB_CUDA_TRY(B.plan_index.reserve(F));
+    HB_CUDA_TRY(B.field_lens.reserve(F * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.field_pos.reserve((F + 1) * sizeof(uint64_t)));
+    const uint64_t *framed_offsets = B.framed_offsets.as<uint64_t>();
+    uint64_t *field_pos = B.field_pos.as<uint64_t>();
+
+    // 1. every name and value framed (indexed names too: simpler than a compacted batch); 2. representation and size
+    // per field; 3. wire positions of fields and blocks; 4. prefixes and literals
+    if (hpack_encode_on_device(ctx, 2 * F, strings, string_offsets, strings_size, mode, B.framed.as<uint8_t>(), framed_cap,
+                               B.framed_offsets.as<uint64_t>(), st))
+        return AWS_OP_ERR;
+    hb::hpack_field_plan_kernel<<<grid_of(F, 256), 256, 0, st>>>(
+        F, strings, string_offsets, never_indexed, framed_offsets, B.plan.as<uint8_t>(), B.plan_index.as<uint8_t>(),
+        B.field_lens.as<uint64_t>());
+    ++ctx->launches;
+    if (launch_scan(ctx, ctx->scratch, B.field_lens.as<uint64_t>(), field_pos, F, st)) return AWS_OP_ERR;
+    hb::hpack_block_offsets_kernel<<<grid_of(n + 1, 256), 256, 0, st>>>(n, field_offsets, field_pos, out_offsets);
+    ++ctx->launches;
+    hb::hpack_field_emit_kernel<<<grid_of(F, 256), 256, 0, st>>>(
+        F, B.plan.as<uint8_t>(), B.plan_index.as<uint8_t>(), B.framed.as<uint8_t>(), framed_offsets, field_pos, out,
+        out_capacity);
+    ++ctx->launches;
+    HB_CUDA_TRY(cudaGetLastError());
+    return AWS_OP_SUCCESS;
+}
+
+int check_block_lists(const aws_hpack_header_lists *l, bool decode) {
+    if (!l || (l->n && !l->field_offsets) || !l->string_offsets || l->n > 0xffffffffull)
+        return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    if (decode && ((l->field_capacity && (!l->field_kind || !l->field_index)) || (l->strings_capacity && !l->strings)))
+        return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    return AWS_OP_SUCCESS;
+}
+
+// Offsets from the caller's memory, read before any kernel trusts them: a decreasing pair would send a walk or a
+// copy outside the arrays.
+bool offsets_sorted(const uint64_t *offsets, uint64_t count) {
+    for (uint64_t i = 1; i < count; ++i)
+        if (offsets[i] < offsets[i - 1]) return false;
+    return true;
+}
+
+BlockLists block_lists(const aws_hpack_header_lists *l) {
+    return BlockLists{l->field_offsets, l->field_capacity, l->field_kind, l->field_index, l->strings, l->strings_capacity,
+                      l->string_offsets};
+}
+
+// Host pointers: stage in, run, stage out (the way hpack_run_host does).
+int hpack_blocks_decode_host(
+    aws_huffman_batch_ctx *ctx, size_t n, const uint8_t *in, const uint64_t *in_off, aws_hpack_header_lists *out,
+    int32_t *status) {
+    if (!ctx || (n && !in_off) || check_block_lists(out, true) || out->n != n) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    if (n == 0) {
+        out->field_offsets[0] = 0;
+        out->string_offsets[0] = 0;
+        return AWS_OP_SUCCESS;
+    }
+    const uint64_t total_in = in_off[n];
+    if ((total_in && !in) || !offsets_sorted(in_off, n + 1)) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    HB_CUDA_TRY(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    hb_host::BlockBufs &B = ctx->blk;
+    HB_CUDA_TRY(ctx->s_in.reserve(total_in + 16));
+    HB_CUDA_TRY(ctx->s_in_off.reserve((n + 1) * sizeof(uint64_t)));
+    HB_CUDA_TRY(ctx->s_status.reserve(n * sizeof(int32_t)));
+    HB_CUDA_TRY(B.s_field_offsets.reserve((n + 1) * sizeof(uint64_t)));
+    if (total_in) HB_CUDA_TRY(cudaMemcpyAsync(ctx->s_in.ptr, in, total_in, cudaMemcpyHostToDevice, st));
+    HB_CUDA_TRY(cudaMemcpyAsync(ctx->s_in_off.ptr, in_off, (n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
+    BlockLists o = block_lists(out);
+    o.field_offsets = B.s_field_offsets.as<uint64_t>();
+    if (hpack_blocks_decode_on_device(ctx, n, ctx->s_in.as<uint8_t>(), ctx->s_in_off.as<uint64_t>(), o,
+                                      ctx->s_status.as<int32_t>(), true, st))
+        return AWS_OP_ERR;
+    HB_CUDA_TRY(cudaMemcpyAsync(out->field_offsets, o.field_offsets, (n + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    if (status) HB_CUDA_TRY(cudaMemcpyAsync(status, ctx->s_status.ptr, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    HB_CUDA_TRY(cudaStreamSynchronize(st));
+    const uint64_t fields = out->field_offsets[n];
+    if (fields > out->field_capacity) return aws_raise_error(AWS_ERROR_SHORT_BUFFER);
+    HB_CUDA_TRY(cudaMemcpyAsync(out->string_offsets, B.s_string_offsets.ptr, (2 * fields + 1) * sizeof(uint64_t),
+                                cudaMemcpyDeviceToHost, st));
+    HB_CUDA_TRY(cudaStreamSynchronize(st));
+    const uint64_t total = out->string_offsets[2 * fields];
+    if (total > out->strings_capacity) return aws_raise_error(AWS_ERROR_SHORT_BUFFER);
+    if (fields) {
+        HB_CUDA_TRY(cudaMemcpyAsync(out->field_kind, B.s_kind.ptr, fields, cudaMemcpyDeviceToHost, st));
+        HB_CUDA_TRY(cudaMemcpyAsync(out->field_index, B.s_index.ptr, fields * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    }
+    if (total) HB_CUDA_TRY(cudaMemcpyAsync(out->strings, ctx->s_out.ptr, total, cudaMemcpyDeviceToHost, st));
+    HB_CUDA_TRY(cudaStreamSynchronize(st));
+    return AWS_OP_SUCCESS;
+}
+
+int hpack_blocks_encode_host(
+    aws_huffman_batch_ctx *ctx, const aws_hpack_header_lists *in, uint32_t mode, uint8_t *out, uint64_t out_capacity,
+    uint64_t *out_off) {
+    if (!ctx || check_block_lists(in, false) || !out_off || (out_capacity && !out)) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    const uint64_t n = in->n;
+    if (n == 0) {
+        out_off[0] = 0;
+        return AWS_OP_SUCCESS;
+    }
+    // (fields are numbered from 0 and every one is encoded: lists start at field 0, strings at octet 0)
+    if (in->field_offsets[0] != 0 || !offsets_sorted(in->field_offsets, n + 1)) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    const uint64_t F = in->field_offsets[n];
+    if (in->string_offsets[0] != 0 || !offsets_sorted(in->string_offsets, 2 * F + 1))
+        return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    const uint64_t S = in->string_offsets[2 * F];
+    if (S && !in->strings) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    HB_CUDA_TRY(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    hb_host::BlockBufs &B = ctx->blk;
+    HB_CUDA_TRY(B.s_field_offsets.reserve((n + 1) * sizeof(uint64_t)));
+    HB_CUDA_TRY(ctx->s_in.reserve(S + 16));
+    HB_CUDA_TRY(ctx->s_in_off.reserve((2 * F + 1) * sizeof(uint64_t)));
+    HB_CUDA_TRY(ctx->s_out.reserve(out_capacity + 16));
+    HB_CUDA_TRY(ctx->s_out_off.reserve((n + 1) * sizeof(uint64_t)));
+    HB_CUDA_TRY(cudaMemcpyAsync(B.s_field_offsets.ptr, in->field_offsets, (n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
+    if (S) HB_CUDA_TRY(cudaMemcpyAsync(ctx->s_in.ptr, in->strings, S, cudaMemcpyHostToDevice, st));
+    HB_CUDA_TRY(cudaMemcpyAsync(ctx->s_in_off.ptr, in->string_offsets, (2 * F + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
+    const uint8_t *never = nullptr;
+    if (in->never_indexed && F) {
+        HB_CUDA_TRY(B.s_never.reserve(F));
+        HB_CUDA_TRY(cudaMemcpyAsync(B.s_never.ptr, in->never_indexed, F, cudaMemcpyHostToDevice, st));
+        never = B.s_never.as<uint8_t>();
+    }
+    if (hpack_blocks_encode_on_device(ctx, n, B.s_field_offsets.as<uint64_t>(), F, never, ctx->s_in.as<uint8_t>(),
+                                      ctx->s_in_off.as<uint64_t>(), S, mode, ctx->s_out.as<uint8_t>(), out_capacity,
+                                      ctx->s_out_off.as<uint64_t>(), st))
+        return AWS_OP_ERR;
+    HB_CUDA_TRY(cudaMemcpyAsync(out_off, ctx->s_out_off.ptr, (n + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    HB_CUDA_TRY(cudaStreamSynchronize(st));
+    const uint64_t total = out_off[n];
+    if (total > out_capacity) return aws_raise_error(AWS_ERROR_SHORT_BUFFER);
+    if (total) {
+        HB_CUDA_TRY(cudaMemcpyAsync(out, ctx->s_out.ptr, total, cudaMemcpyDeviceToHost, st));
+        HB_CUDA_TRY(cudaStreamSynchronize(st));
+    }
+    return AWS_OP_SUCCESS;
+}
+
+// ---------------------------------------------------------------------------------------------
 // Byte histogram (SURVEY.md 8f.4: the counts a code table is built from). HBM-bound by construction: 16 bytes per
 // lane and load, and a block-wide histogram with ONE COLUMN PER LANE (hist[value][lane]): the 32 lanes of a
 // shared-memory atomic never meet in an address and every lane stays in its own bank, however skewed the
@@ -1654,6 +1961,7 @@ void aws_huffman_batch_ctx_destroy(struct aws_huffman_batch_ctx *ctx) {
                        &ctx->hp_left_bits, &ctx->hp_left_num, &ctx->hp_status};
     for (GrowBuf *g : bufs) g->release();
     if (ctx->h_scalar) cudaFreeHost(ctx->h_scalar);
+    ctx->blk.release();
     ctx->scratch.release();
     for (Lane &lane : ctx->lanes) lane.release();
     (void)cudaGetLastError();
@@ -1788,6 +2096,44 @@ int aws_hpack_string_decode_batch_device(
     if (device_call_begin(ctx, cuda_stream, &st)) return AWS_OP_ERR;
     return device_call_end(
         ctx, st, hpack_decode_on_device(ctx, n, in, in_offsets, in_size, out, out_capacity, out_offsets, status, st));
+}
+
+int aws_hpack_header_block_decode_batch(
+    struct aws_huffman_batch_ctx *ctx, size_t n, const uint8_t *in, const uint64_t *in_offsets,
+    struct aws_hpack_header_lists *out, int32_t *status) {
+    return hpack_blocks_decode_host(ctx, n, in, in_offsets, out, status);
+}
+
+int aws_hpack_header_block_encode_batch(
+    struct aws_huffman_batch_ctx *ctx, const struct aws_hpack_header_lists *in, enum aws_hpack_huffman_mode mode,
+    uint8_t *out, uint64_t out_capacity, uint64_t *out_offsets) {
+    if ((unsigned)mode > (unsigned)AWS_HPACK_HUFFMAN_ALWAYS) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    return hpack_blocks_encode_host(ctx, in, (uint32_t)mode, out, out_capacity, out_offsets);
+}
+
+int aws_hpack_header_block_decode_batch_device(
+    struct aws_huffman_batch_ctx *ctx, size_t n, const uint8_t *in, const uint64_t *in_offsets, uint64_t in_size,
+    struct aws_hpack_header_lists *out, int32_t *status, void *cuda_stream) {
+    if (!ctx || (n && !in_offsets) || (in_size && !in) || check_block_lists(out, true) || out->n != n)
+        return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    cudaStream_t st;
+    if (device_call_begin(ctx, cuda_stream, &st)) return AWS_OP_ERR;
+    return device_call_end(ctx, st, hpack_blocks_decode_on_device(ctx, n, in, in_offsets, block_lists(out), status, false, st));
+}
+
+int aws_hpack_header_block_encode_batch_device(
+    struct aws_huffman_batch_ctx *ctx, const struct aws_hpack_header_lists *in, uint64_t num_fields,
+    uint64_t strings_size, enum aws_hpack_huffman_mode mode, uint8_t *out, uint64_t out_capacity, uint64_t *out_offsets,
+    void *cuda_stream) {
+    if (!ctx || check_block_lists(in, false) || !out_offsets || (out_capacity && !out) || (strings_size && !in->strings) ||
+        (unsigned)mode > (unsigned)AWS_HPACK_HUFFMAN_ALWAYS)
+        return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    cudaStream_t st;
+    if (device_call_begin(ctx, cuda_stream, &st)) return AWS_OP_ERR;
+    return device_call_end(ctx, st,
+                           hpack_blocks_encode_on_device(ctx, in->n, in->field_offsets, num_fields, in->never_indexed, in->strings,
+                                                         in->string_offsets, strings_size, (uint32_t)mode, out, out_capacity,
+                                                         out_offsets, st));
 }
 
 int aws_huffman_get_encoded_length_batch(
