@@ -641,11 +641,7 @@ __device__ __forceinline__ Lut2Hit lut2_lookup(const Lut2 &t, uint32_t window) {
 }
 __device__ __forceinline__ uint32_t lut2_len1(uint32_t x) { return (x >> 16) & 63u; }
 
-// kInPlace: the row being written overlays the stream being read (decode_slots.cuh: the writer never passes the
-// reader, but what was read is gone): a lane that meets a hole cannot start over from here — it returns
-// kTermTrapped and the caller redoes the string from global memory — and nothing is stored beyond the last symbol.
-constexpr uint32_t kTermTrapped = 3;
-template <bool kEmit, bool kPadded, bool kSkipHoles, bool kInPlace = false, bool kRaw = false>
+template <bool kEmit, bool kPadded, bool kSkipHoles, bool kRaw = false>
 __device__ __forceinline__ SpanS decode_span_lean(
     const uint32_t *s_in, const Lut2 &t, uint32_t root_bits, uint32_t pos, uint32_t stop, uint32_t end, uint32_t out_addr) {
     constexpr uint32_t kParked = 0x80000000u;
@@ -851,21 +847,11 @@ __device__ __forceinline__ SpanS decode_span_lean(
         }
 #endif
         if (pos & kParked) {
-            if (kInPlace) {
-                r.term = kTermTrapped;
-                r.pos = pos0;
-                r.nsym = 0;
-                return r;
-            }
             pos = pos0;
             out_addr = out0;
             c.template init<kPadded>(in_addr, pos);
-        } else if (kEmit && (out_addr & 3u)) {
-            if (kInPlace) {  // the symbols still in `acc`, and not a byte more
-                for (uint32_t k = 0; k < (out_addr & 3u); ++k) sts_u8((out_addr & ~3u) + k, acc >> (8 * k));
-            } else {         // (the bytes above them are spare: rows have slack)
-                asm volatile("st.shared.u32 [%0], %1;" ::"r"(out_addr & ~3u), "r"(acc) : "memory");
-            }
+        } else if (kEmit && (out_addr & 3u)) {  // (the bytes above the symbols in `acc` are spare: rows have slack)
+            asm volatile("st.shared.u32 [%0], %1;" ::"r"(out_addr & ~3u), "r"(acc) : "memory");
         }
         // the rest of the span (or all of it, after a trap): one lookup at a time with the end-of-stream rules (the
         // window is the stream zero-extended, huffman.c:196-211; a code that does not fit ends the stream,
@@ -1342,7 +1328,7 @@ __global__ void __launch_bounds__(kDecTeams * kDecBlock, 1) decode_batch_kernel(
                     }
                 } else if (staged) {
                     const uint32_t ib = s_start[it], ie = ib + nbytes * 8;
-                    const SpanS r = decode_span_lean<true, false, false, false, kRaw>(s_in, lut2, a.root_bits, ib, ie, ie, rows_addr + s_row[it]);
+                    const SpanS r = decode_span_lean<true, false, false, kRaw>(s_in, lut2, a.root_bits, ib, ie, ie, rows_addr + s_row[it]);
                     cbits = r.pos - ib;
                     nsym = r.nsym;
                     term = r.term;

@@ -278,33 +278,4 @@ __device__ __forceinline__ uint64_t lookback_exclusive(uint64_t *tile_state, uin
     return exclusive;
 }
 
-// Whole block: copies n bytes from `src` (16-byte aligned, with >= 32 readable bytes after n: a block's
-// slot of the deferred-output scratch, read through L2) to `dst` (any alignment) with 128-bit stores.
-__device__ __forceinline__ void block_copy_realign(const uint8_t *src, uint8_t *dst, uint32_t n, uint32_t tid, uint32_t nthreads) {
-    const uint32_t head = min(n, (16u - (uint32_t)(reinterpret_cast<uintptr_t>(dst) & 15)) & 15u);
-    const uint32_t nvec = (n - head) >> 4;
-    const uint4 *sv = reinterpret_cast<const uint4 *>(src);
-    uint4 *dv = reinterpret_cast<uint4 *>(dst + head);
-    const uint32_t tw = head >> 2, r8 = (head & 3u) * 8u;  // the body starts `head` bytes into the image
-    for (uint32_t v = tid; v < nvec; v += nthreads) {
-        const uint4 a = __ldcg(sv + v), b = __ldcg(sv + v + 1);
-        uint32_t w0, w1, w2, w3, w4;
-        switch (tw) {  // (uniform)
-            case 0: w0 = a.x; w1 = a.y; w2 = a.z; w3 = a.w; w4 = b.x; break;
-            case 1: w0 = a.y; w1 = a.z; w2 = a.w; w3 = b.x; w4 = b.y; break;
-            case 2: w0 = a.z; w1 = a.w; w2 = b.x; w3 = b.y; w4 = b.z; break;
-            default: w0 = a.w; w1 = b.x; w2 = b.y; w3 = b.z; w4 = b.w; break;
-        }
-        uint4 o;
-        o.x = __funnelshift_r(w0, w1, r8);
-        o.y = __funnelshift_r(w1, w2, r8);
-        o.z = __funnelshift_r(w2, w3, r8);
-        o.w = __funnelshift_r(w3, w4, r8);
-        dv[v] = o;
-    }
-    if (tid < head) dst[tid] = __ldcg(src + tid);
-    const uint32_t tail0 = head + 16u * nvec;
-    if (tid >= 32 && tid - 32 < n - tail0) dst[tail0 + tid - 32] = __ldcg(src + tail0 + tid - 32);
-}
-
 }  // namespace hb

@@ -18,8 +18,6 @@
 #include "hpack_literals.cuh"
 #include "hpack_blocks.cuh"
 #include "decode_fast.cuh"
-#include "decode_rows.cuh"
-#include "decode_slots.cuh"
 
 #include <algorithm>
 #include <cstdio>
@@ -81,16 +79,17 @@ struct GrowBuf {
 // Per-launch kernel scratch (tile descriptors, chunk records, ...). One per concurrent stream.
 struct Scratch {
     GrowBuf lens, tile_state, tile_first, chunks, chunk_lens, chunk_offsets, fused, slot_base, deferred, str_ctl, str_state,
-        str_tiles, str_bits, str_bits_first, rows, row_pos, row_cnt, rows_ctl;
+        str_tiles, str_bits, str_bits_first;
     void release() {
-        GrowBuf *all[] = {&lens,          &tile_state, &tile_first,  &chunks,   &chunk_lens, &chunk_offsets,
-                          &fused,         &slot_base,  &deferred,    &str_ctl,  &str_state,  &str_tiles,
-                          &str_bits,      &str_bits_first, &rows,       &row_pos,     &row_cnt,  &rows_ctl};
+        GrowBuf *all[] = {&lens,     &tile_state, &tile_first, &chunks,  &chunk_lens, &chunk_offsets, &fused,
+                          &slot_base, &deferred,  &str_ctl,    &str_state, &str_tiles, &str_bits,     &str_bits_first};
         for (GrowBuf *g : all) g->release();
     }
 };
 
-constexpr int kLanes = 8;
+// lanes of the pipelined host path (round 2, 12 MiB sub-batches: retired one issue later with 4 lanes 60.9,
+// two issues later with 5 lanes 59.7, one issue later with 3 lanes 59.6 GB/s end to end)
+constexpr size_t kLanes = 4;
 struct Lane {
     cudaStream_t stream = nullptr;
     cudaEvent_t kernels_done = nullptr, retired = nullptr;
@@ -158,7 +157,7 @@ struct aws_huffman_batch_ctx {
     int str_blocks_per_sm[3] = {0, 0, 0};  // str_bits_kernel, str_pack_kernel, str_scan_kernel
     // staging for the host entry points
     GrowBuf s_in, s_in_off, s_out, s_out_off, s_caps, s_status, s_consumed, s_ovf_pattern, s_ovf_bits, s_left_bits,
-        s_left_num, s_chain;
+        s_left_num;
     // HPACK string literals (hpack_literals.cuh): packed payloads between the framing and the codec, per-item plans
     GrowBuf hp_pay, hp_pay_off, hp_dec, hp_dec_off, hp_huff, hp_prefix, hp_lens, hp_pay_lens, hp_dec_status, hp_left_bits,
         hp_left_num, hp_status;
@@ -171,10 +170,8 @@ struct aws_huffman_batch_ctx {
     cudaStream_t scratch_stream = nullptr;
     bool scratch_busy = false;
     // switches, read once at context creation (DESIGN.md 6b)
-    bool force_generic = false, no_slots = false, no_strings = false, no_fused_stream = false, no_rows = false;
-    int rows_blocks_per_sm = 0, compact_blocks_per_sm = 0;
-    bool no_slots_decode = false;
-    size_t slots_static_smem = 0, dec_static_smem[2] = {0, 0};
+    bool force_generic = false, no_slots = false, no_strings = false, no_fused_stream = false;
+    size_t dec_static_smem[2] = {0, 0};
 };
 
 namespace {
@@ -562,121 +559,6 @@ int decode_batch_fast(
     return AWS_OP_SUCCESS;
 }
 
-// Packed layout, many strings: decode_slots_kernel (decode_slots.cuh) — decode_batch_kernel with stage and rows in
-// one place, larger tiles for the same shared memory, rows straight to global memory.
-int decode_batch_slots(
-    aws_huffman_batch_ctx *ctx, Scratch &sc, const hb::BatchView &v, uint64_t total_in, cudaStream_t stream) {
-    if (!ctx->slots_static_smem) {
-        cudaFuncAttributes attr{};
-        HB_CUDA_TRY(cudaFuncGetAttributes(&attr, decode_slots_kernel));
-        ctx->slots_static_smem = attr.sharedSizeBytes;
-        // (the limit belongs to the kernel, not to the context: set to what the device allows, launches ask for less)
-        HB_CUDA_TRY(cudaFuncSetAttribute(
-            decode_slots_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(227 * 1024 - 1024 - attr.sharedSizeBytes)));
-    }
-    DecSlotsArgs a{};
-    a.b = v;
-    a.lut2 = ctx->d_lut2;
-    a.lut2_count = ctx->lut2_count;
-    a.lut2_trap = ctx->lut2_trap;
-    a.root_bits = ctx->tables.lut_root_bits;
-    a.min_len = std::min<uint32_t>(8, std::max<uint32_t>(1, ctx->tables.min_len));
-    const size_t lut_bytes = (size_t)a.lut2_count * 8;
-    const size_t avail = (size_t)227 * 1024 - 1024 - ctx->slots_static_smem - lut_bytes;
-    const size_t region = (avail / kDecTeams) & ~size_t(15);
-    a.region_bytes = (uint32_t)region;
-    // strings per tile: as many slots as fit the region at the batch's average length with 15 % to spare, in whole
-    // warps (a tile that does not fit takes the two-pass global route and every tile behind it waits for its count)
-    {
-        const double avg = std::max(1.0, (double)total_in / (double)v.n);
-        const uint64_t fit = (uint64_t)std::max(32.0, (double)region / (1.15 * (avg * 8.0 / a.min_len + kSlotSlack)));
-        a.items_per_tile = (uint32_t)std::min<uint64_t>(kSlotItemsPerTile, fit & ~uint64_t(31));
-    }
-    const uint64_t num_tiles = (v.n + a.items_per_tile - 1) / a.items_per_tile;
-    const size_t state_bytes = num_tiles * sizeof(uint64_t) + 256;
-    HB_CUDA_TRY(sc.tile_state.reserve(state_bytes));
-    HB_CUDA_TRY(cudaMemsetAsync(sc.tile_state.ptr, 0, state_bytes, stream));
-    a.tile_state = sc.tile_state.as<uint64_t>();
-    a.ticket = reinterpret_cast<uint32_t *>(a.tile_state + num_tiles);
-    a.num_tiles = (uint32_t)num_tiles;
-    const size_t smem = lut_bytes + kDecTeams * region;
-    const unsigned blocks = (unsigned)std::min<uint64_t>((num_tiles + kDecTeams - 1) / kDecTeams, (uint64_t)ctx->sm_count);
-    decode_slots_kernel<<<blocks, kDecTeams * kDecBlock, smem, stream>>>(a);
-    ++ctx->launches;
-    HB_CUDA_TRY(cudaGetLastError());
-    return AWS_OP_SUCCESS;
-}
-
-// Packed layout, many strings: decode into worst-case spaced rows of a global scratch (decode_rows_kernel), then
-// counts -> offsets and rows -> dense output (compact_rows_kernel). decode_rows.cuh.
-constexpr size_t kCompactStageBytes = 56 * 1024, kCompactImageBytes = 42 * 1024;  // two blocks per SM
-int decode_batch_rows(
-    aws_huffman_batch_ctx *ctx, Scratch &sc, const hb::BatchView &v, uint64_t total_in, cudaStream_t stream) {
-    const uint32_t min_len = std::max<uint32_t>(1, ctx->tables.min_len);
-    const uint64_t rows_bytes = 16ull * (total_in / (2ull * min_len) + 1) + (uint64_t)kRowsSlack * v.n + 256;
-    const uint64_t num_pools = (v.n + kRowsPool - 1) / kRowsPool;
-    // strings per compaction tile: as many as fit the stage (rows at their worst-case spacing) with 15 % to spare, and
-    // the image if strings of average length decode to 85 % of their worst case (8 / min_len symbols per byte; the
-    // benchmark's data: 1.36 of 1.6); even. A tile that does not fit takes the slow route.
-    const double avg_row = std::max(1.0, (double)total_in * 8.0 / min_len / (double)v.n);
-    uint64_t per_tile = (uint64_t)std::min((double)kCompactStageBytes / (1.15 * (avg_row + kRowsSlack)),
-                                           (double)(kCompactImageBytes - 64) / (0.85 * 1.15 * avg_row));
-    per_tile = std::max<uint64_t>(2, std::min<uint64_t>(kCompactMaxItems, per_tile & ~uint64_t(1)));
-    const uint64_t num_tiles = (v.n + per_tile - 1) / per_tile;
-    if (num_pools >= 0xffffffffull || num_tiles >= 0xffffffffull) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
-    HB_CUDA_TRY(sc.rows.reserve(rows_bytes));
-    HB_CUDA_TRY(sc.row_pos.reserve(v.n * sizeof(uint64_t)));
-    HB_CUDA_TRY(sc.row_cnt.reserve((v.n + 2) * sizeof(uint32_t)));
-    // [look-back descriptors of the compaction: num_tiles][tickets: 2 words (+ pad)]
-    const size_t ctl_bytes = num_tiles * sizeof(uint64_t) + 64;
-    HB_CUDA_TRY(sc.rows_ctl.reserve(ctl_bytes));
-    HB_CUDA_TRY(cudaMemsetAsync(sc.rows_ctl.ptr, 0, ctl_bytes, stream));
-    uint32_t *tickets = reinterpret_cast<uint32_t *>(sc.rows_ctl.as<uint64_t>() + num_tiles);
-    DecRowsArgs a{};
-    a.b = v;
-    a.total_in = total_in;
-    a.lut2 = ctx->d_lut2;
-    a.lut2_count = ctx->lut2_count;
-    a.lut2_trap = ctx->lut2_trap;
-    a.root_bits = ctx->tables.lut_root_bits;
-    a.min_len = min_len;
-    a.rows = sc.rows.as<uint8_t>();
-    a.row_pos = sc.row_pos.as<uint64_t>();
-    a.cnt = sc.row_cnt.as<uint32_t>();
-    a.ticket = tickets;
-    a.num_pools = (uint32_t)num_pools;
-    const size_t rows_smem = (size_t)ctx->lut2_count * 8 + 1024 + (size_t)kRowsWarps * kRowsRingBytes;
-    if (!ctx->rows_blocks_per_sm) {
-        // (the attribute belongs to the kernel, not to the context, and tables differ in size: the limit is set to
-        // what the device allows once, the launches ask for what they need)
-        int per_sm = 0;
-        HB_CUDA_TRY(cudaFuncSetAttribute(decode_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 216 * 1024));
-        HB_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, decode_rows_kernel, kRowsThreads, rows_smem));
-        ctx->rows_blocks_per_sm = std::max(1, per_sm);
-        HB_CUDA_TRY(cudaFuncSetAttribute(compact_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(kCompactStageBytes + kCompactImageBytes)));
-        HB_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, compact_rows_kernel, kCompactThreads, kCompactStageBytes + kCompactImageBytes));
-        ctx->compact_blocks_per_sm = std::max(1, per_sm);
-    }
-    const unsigned grid_r = (unsigned)std::min<uint64_t>(num_pools, (uint64_t)ctx->sm_count * ctx->rows_blocks_per_sm);
-    decode_rows_kernel<<<grid_r, kRowsThreads, rows_smem, stream>>>(a);
-    CompactArgs c{};
-    c.b = v;
-    c.rows = a.rows;
-    c.row_pos = a.row_pos;
-    c.cnt = a.cnt;
-    c.tile_state = sc.rows_ctl.as<uint64_t>();
-    c.ticket = tickets + 1;
-    c.num_tiles = (uint32_t)num_tiles;
-    c.items_per_tile = (uint32_t)per_tile;
-    c.stage_bytes = (uint32_t)kCompactStageBytes;
-    c.image_bytes = (uint32_t)kCompactImageBytes;
-    const unsigned grid_c = (unsigned)std::min<uint64_t>(num_tiles, (uint64_t)ctx->sm_count * ctx->compact_blocks_per_sm);
-    compact_rows_kernel<<<grid_c, kCompactThreads, kCompactStageBytes + kCompactImageBytes, stream>>>(c);
-    ctx->launches += 2;
-    HB_CUDA_TRY(cudaGetLastError());
-    return AWS_OP_SUCCESS;
-}
-
 // Packed layout, one long stream: chunked speculative decode. The fused single-pass kernel does the
 // work; the multi-kernel path behind it only runs (on the device's own decision, no host round trip)
 // when the fused kernel raised its `fail` flag: a stream that does not self-synchronise, or that stops
@@ -763,7 +645,6 @@ int decode_stream_fast(
     return AWS_OP_SUCCESS;
 }
 
-inline bool num_tiles_ok(uint64_t n) { return n / 32 < 0xfffffff0ull; }
 constexpr uint64_t kStreamMinBytes = 64 * 1024;  // shorter single items go through the batch kernel
 
 int decode_on_device(
@@ -772,8 +653,6 @@ int decode_on_device(
     const bool force_generic = ctx->force_generic;
     if (!v.resume && !v.out_caps && ctx->tables.lut_count <= kDecLutMaxSmem && !force_generic) {
         if (v.n == 1 && total_in >= kStreamMinBytes) return decode_stream_fast(ctx, sc, v, total_in, stream);
-        if (!ctx->no_rows) return decode_batch_rows(ctx, sc, v, total_in, stream);
-        if (!ctx->no_slots_decode && num_tiles_ok(v.n)) return decode_batch_slots(ctx, sc, v, total_in, stream);
         return decode_batch_fast(ctx, sc, v, total_in, stream);
     }
     if (!v.out_lens) {
@@ -805,34 +684,6 @@ __global__ void add_base_kernel(uint64_t *offsets, uint64_t count, uint64_t base
     if (i < count) offsets[i] += base;
 }
 
-// Sub-batch j of the pipelined host path leaves the device WITHOUT the host knowing its size: this kernel reads the
-// sub-batch's size and the running output position (written by sub-batch j - 1's instance; the streams are ordered
-// by an event), publishes the next position, rebases the sub-batch's packed offsets and copies its payload straight
-// into the caller's pinned buffer (`dst`: the device's alias of it) with 128-bit stores.
-constexpr int kChainBlocks = 96, kChainThreads = 256;
-constexpr uint32_t kChainSegment = 16 * 1024;  // bytes a block moves per turn (multiple of 16)
-__global__ void __launch_bounds__(kChainThreads) d2h_chain_kernel(
-    const uint8_t *src, uint64_t *out_off, uint64_t nj, const uint64_t *base_in, uint64_t *base_out, uint8_t *dst,
-    uint64_t capacity, uint32_t *overflow) {
-    const uint64_t base = base_in ? *base_in : 0;
-    const uint64_t total = out_off[nj];
-    const bool fits = base + total <= capacity;
-    if (blockIdx.x == 0 && threadIdx.x == 0) {
-        *base_out = base + total;
-        if (!fits) *overflow = 1u;
-    }
-    if (fits) {
-        for (uint64_t seg = (uint64_t)blockIdx.x * kChainSegment; seg < total; seg += (uint64_t)gridDim.x * kChainSegment)
-            hb::block_copy_realign(src + seg, dst + base + seg, (uint32_t)min((uint64_t)kChainSegment, total - seg), threadIdx.x, kChainThreads);
-    }
-    if (base)
-        for (uint64_t i = (uint64_t)blockIdx.x * kChainThreads + threadIdx.x; i < nj; i += (uint64_t)gridDim.x * kChainThreads)
-            out_off[i] += base;
-}
-
-template <typename T>
-T *mapped_alias(T *p, uint64_t size);
-
 int lane_prepare(Lane &lane) {
     if (lane.stream) return AWS_OP_SUCCESS;
     HB_CUDA_TRY(cudaStreamCreateWithFlags(&lane.stream, cudaStreamNonBlocking));
@@ -842,10 +693,37 @@ int lane_prepare(Lane &lane) {
     return AWS_OP_SUCCESS;
 }
 
-constexpr uint64_t kZeroCopyMinBytes = 4096;          // pinned payload buffers: kernels work on them in place
 constexpr uint64_t kPipelineMinBytes = 8ull << 20;   // below this one shot is as good
 constexpr uint64_t kPipelineShardBytes = 12ull << 20;  // measured on PCIe Gen5 x16: 4 / 6 / 8 / 12 / 16 MiB: 53.2 / 57.0 / 58.3 / 60.4 / 59.6 GB/s
                                                        // end to end (round 1, slower kernels: 8 MiB)
+// A sub-batch is retired (its D2H copies queued) one issue after it was issued, and its lane takes the next
+// sub-batch kLanes issues after it took this one. A lane must not be re-used before its sub-batch was retired; with
+// one lane more than that, re-using a lane never has to wait for a D2H copy that is still running, so uploads of
+// later sub-batches and downloads of earlier ones stay concurrent.
+constexpr size_t kRetireLag = 1;
+static_assert(hb_host::kLanes >= kRetireLag + 2, "lanes must outnumber the issue-to-retire distance by two");
+
+// Copies the per-item arrays of items [first, first + count) from the device view `v` into the caller's batch `b`.
+// `v` holds an array exactly when the caller asked for it.
+int copy_item_arrays_to_host(const aws_huffman_batch *b, const hb::BatchView &v, size_t first, size_t count, cudaStream_t st) {
+    if (v.out_lens)
+        HB_CUDA_TRY(cudaMemcpyAsync(b->out_lens + first, v.out_lens, count * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    if (v.status)
+        HB_CUDA_TRY(cudaMemcpyAsync(b->status + first, v.status, count * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    if (v.consumed)
+        HB_CUDA_TRY(cudaMemcpyAsync(b->consumed + first, v.consumed, count * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    if (v.overflow_pattern)
+        HB_CUDA_TRY(cudaMemcpyAsync(
+            b->overflow_pattern + first, v.overflow_pattern, count * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    if (v.overflow_num_bits)
+        HB_CUDA_TRY(cudaMemcpyAsync(b->overflow_num_bits + first, v.overflow_num_bits, count, cudaMemcpyDeviceToHost, st));
+    if (v.leftover_working_bits)
+        HB_CUDA_TRY(cudaMemcpyAsync(
+            b->leftover_working_bits + first, v.leftover_working_bits, count * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    if (v.leftover_num_bits)
+        HB_CUDA_TRY(cudaMemcpyAsync(b->leftover_num_bits + first, v.leftover_num_bits, count, cudaMemcpyDeviceToHost, st));
+    return AWS_OP_SUCCESS;
+}
 
 // Packed layout with many items: the batch is cut into sub-batches (contiguous item ranges balanced by
 // bytes) that flow through kLanes lanes, so the host->device copy of one sub-batch, the kernels of the
@@ -855,9 +733,7 @@ constexpr uint64_t kPipelineShardBytes = 12ull << 20;  // measured on PCIe Gen5 
 int run_host_batch_pipelined(aws_huffman_batch_ctx *ctx, const aws_huffman_batch *b, bool encode) {
     const size_t n = b->n;
     const uint64_t total_in = b->in_offsets[n];
-    uint64_t shard_bytes = kPipelineShardBytes;
-    if (const char *mb = getenv("AWS_HUFFMAN_BATCH_SHARD_MB")) shard_bytes = std::max<uint64_t>(1, atoi(mb)) << 20;
-    size_t shards = (size_t)std::min<uint64_t>(256, std::max<uint64_t>(2, total_in / shard_bytes));
+    size_t shards = (size_t)std::min<uint64_t>(256, std::max<uint64_t>(2, total_in / kPipelineShardBytes));
     shards = std::min(shards, n);
     std::vector<size_t> begin(shards + 1);
     if (aws_huffman_batch_plan_shards(b->in_offsets, n, shards, begin.data())) return AWS_OP_ERR;
@@ -868,42 +744,18 @@ int run_host_batch_pipelined(aws_huffman_batch_ctx *ctx, const aws_huffman_batch
     shards = begin.size() - 1;
     // (cutting the first and last sub-batches smaller, to shorten pipeline fill and drain, was measured: no
     // effect — 59.5 vs 60.2 GB/s end to end)
-    std::vector<uint64_t> shard_base(shards + 1, 0);
+    std::vector<hb::BatchView> views(shards);  // sub-batch j's arrays on the device, read back by retire(j)
 
     for (Lane &lane : ctx->lanes)
         if (lane_prepare(lane)) return AWS_OP_ERR;
 
     const uint32_t max_len = std::max<uint32_t>(1, ctx->tables.max_len);
     const uint32_t min_len = std::max<uint32_t>(1, ctx->tables.min_len);
-    // a sub-batch is retired `depth` issues after it was issued; more lanes than that keep re-use from waiting
-    size_t depth = 1, lanes_used = 4;  // (round 2, 12 MiB sub-batches: depth 1 / 4 lanes 60.9, depth 2 / 5 lanes 59.7, depth 1 / 3 lanes 59.6 GB/s)
-    if (const char *d = getenv("AWS_HUFFMAN_BATCH_PIPE_DEPTH")) depth = std::min<size_t>(6, std::max(1, atoi(d)));
-    if (const char *l = getenv("AWS_HUFFMAN_BATCH_PIPE_LANES")) lanes_used = std::min<size_t>(hb_host::kLanes, std::max(2, atoi(l)));
-    lanes_used = std::max(lanes_used, depth + 2);
-    lanes_used = std::min<size_t>(lanes_used, hb_host::kLanes);
     uint64_t base_out = 0;
     bool overflow = false;
-    // CHAINED mode (opt-in: AWS_HUFFMAN_BATCH_CHAIN=1 and a pinned output buffer): the host never learns a sub-batch's size
-    // while the call runs. A small kernel behind each sub-batch's codec kernels (d2h_chain_kernel) reads the size on the
-    // device, takes the running output position from its predecessor (streams ordered by an event), and writes the
-    // payload straight into the caller's buffer; the fixed-size arrays follow by ordinary copies. No
-    // cudaEventSynchronize per sub-batch, no copy that waits for the host to have seen a size, no drain of late
-    // sub-batches at the end. Correct (tests/test_gpu_multi.py) and MEASURED SLOWER than the copy engines: 53.6 GB/s end
-    // to end against 60.4 on the 1M-string batch (4 / 6 / 8 lanes: 56.5 / 53.6 / 48 GB/s: the more sub-batches in
-    // flight, the worse — kernel-issued PCIe writes hold their SMs while the copy engines work for free). Round 1
-    // measured the same for whole kernels working on pinned buffers; it holds for a dedicated copy kernel too.
-    uint8_t *const zout = getenv("AWS_HUFFMAN_BATCH_CHAIN") ? mapped_alias(b->out, b->out_capacity) : nullptr;
-    const bool chained = zout != nullptr;
-    uint64_t *chain = nullptr;      // [0 .. shards]: output position before sub-batch j; [shards + 1]: overflow flag
-    cudaEvent_t prev_copied = nullptr;
-    if (chained) {
-        HB_CUDA_TRY(ctx->s_chain.reserve((shards + 2) * sizeof(uint64_t)));
-        chain = ctx->s_chain.as<uint64_t>();
-        HB_CUDA_TRY(cudaMemsetAsync(chain + shards + 1, 0, sizeof(uint64_t), ctx->lanes[0].stream));
-    }
 
     auto issue = [&](size_t j) -> int {
-        Lane &lane = ctx->lanes[j % lanes_used];
+        Lane &lane = ctx->lanes[j % hb_host::kLanes];
         if (lane.in_flight) {
             HB_CUDA_TRY(cudaEventSynchronize(lane.retired));
             lane.in_flight = false;
@@ -930,7 +782,7 @@ int run_host_batch_pipelined(aws_huffman_batch_ctx *ctx, const aws_huffman_batch
         rebase_offsets_kernel<<<(unsigned)((nj + 1 + 255) / 256), 256, 0, lane.stream>>>(
             lane.in_off.as<uint64_t>(), nj + 1, in0, lane.in_off.as<uint64_t>());
         ++ctx->launches;
-        hb::BatchView v{};
+        hb::BatchView &v = views[j];
         v.n = nj;
         v.in = lane.in.as<uint8_t>();
         v.in_offsets = lane.in_off.as<uint64_t>();
@@ -950,38 +802,6 @@ int run_host_batch_pipelined(aws_huffman_batch_ctx *ctx, const aws_huffman_batch
         if ((encode ? encode_on_device(ctx, lane.scratch, v, bytes_in, lane.stream)
                     : decode_on_device(ctx, lane.scratch, v, bytes_in, lane.stream)) != AWS_OP_SUCCESS)
             return AWS_OP_ERR;
-        if (chained) {
-            cudaStream_t st = lane.stream;
-            if (prev_copied) HB_CUDA_TRY(cudaStreamWaitEvent(st, prev_copied, 0));
-            d2h_chain_kernel<<<kChainBlocks, kChainThreads, 0, st>>>(
-                lane.out.as<uint8_t>(), lane.out_off.as<uint64_t>(), nj, j ? chain + j : nullptr, chain + j + 1, zout,
-                b->out_capacity, reinterpret_cast<uint32_t *>(chain + shards + 1));
-            ++ctx->launches;
-            HB_CUDA_TRY(cudaGetLastError());
-            HB_CUDA_TRY(cudaEventRecord(lane.kernels_done, st));
-            prev_copied = lane.kernels_done;
-            HB_CUDA_TRY(cudaMemcpyAsync(b->out_offsets + a, lane.out_off.ptr, nj * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-            if (b->out_lens)
-                HB_CUDA_TRY(cudaMemcpyAsync(b->out_lens + a, lane.lens.ptr, nj * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-            if (b->status)
-                HB_CUDA_TRY(cudaMemcpyAsync(b->status + a, lane.status.ptr, nj * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-            if (b->consumed)
-                HB_CUDA_TRY(cudaMemcpyAsync(b->consumed + a, lane.consumed.ptr, nj * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-            if (encode) {
-                if (b->overflow_pattern)
-                    HB_CUDA_TRY(cudaMemcpyAsync(b->overflow_pattern + a, lane.aux32.ptr, nj * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-                if (b->overflow_num_bits)
-                    HB_CUDA_TRY(cudaMemcpyAsync(b->overflow_num_bits + a, lane.aux8.ptr, nj, cudaMemcpyDeviceToHost, st));
-            } else {
-                if (b->leftover_working_bits)
-                    HB_CUDA_TRY(cudaMemcpyAsync(b->leftover_working_bits + a, lane.aux64.ptr, nj * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-                if (b->leftover_num_bits)
-                    HB_CUDA_TRY(cudaMemcpyAsync(b->leftover_num_bits + a, lane.aux8.ptr, nj, cudaMemcpyDeviceToHost, st));
-            }
-            HB_CUDA_TRY(cudaEventRecord(lane.retired, st));
-            lane.in_flight = true;
-            return AWS_OP_SUCCESS;
-        }
         HB_CUDA_TRY(cudaMemcpyAsync(
             lane.h_total, lane.out_off.as<uint64_t>() + nj, sizeof(uint64_t), cudaMemcpyDeviceToHost, lane.stream));
         HB_CUDA_TRY(cudaEventRecord(lane.kernels_done, lane.stream));
@@ -990,11 +810,10 @@ int run_host_batch_pipelined(aws_huffman_batch_ctx *ctx, const aws_huffman_batch
     };
 
     auto retire = [&](size_t j) -> int {
-        Lane &lane = ctx->lanes[j % lanes_used];
+        Lane &lane = ctx->lanes[j % hb_host::kLanes];
         const size_t a = begin[j], nj = begin[j + 1] - a;
         HB_CUDA_TRY(cudaEventSynchronize(lane.kernels_done));
         const uint64_t total = *lane.h_total;
-        shard_base[j] = base_out;
         cudaStream_t st = lane.stream;
         if (base_out + total > b->out_capacity) overflow = true;
         if (!overflow && total)
@@ -1005,32 +824,12 @@ int run_host_batch_pipelined(aws_huffman_batch_ctx *ctx, const aws_huffman_batch
             ++ctx->launches;
         }
         HB_CUDA_TRY(cudaMemcpyAsync(b->out_offsets + a, lane.out_off.ptr, nj * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-        if (b->out_lens)
-            HB_CUDA_TRY(cudaMemcpyAsync(b->out_lens + a, lane.lens.ptr, nj * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-        if (b->status)
-            HB_CUDA_TRY(cudaMemcpyAsync(b->status + a, lane.status.ptr, nj * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-        if (b->consumed)
-            HB_CUDA_TRY(cudaMemcpyAsync(b->consumed + a, lane.consumed.ptr, nj * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-        if (encode) {
-            if (b->overflow_pattern)
-                HB_CUDA_TRY(cudaMemcpyAsync(b->overflow_pattern + a, lane.aux32.ptr, nj * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-            if (b->overflow_num_bits)
-                HB_CUDA_TRY(cudaMemcpyAsync(b->overflow_num_bits + a, lane.aux8.ptr, nj, cudaMemcpyDeviceToHost, st));
-        } else {
-            if (b->leftover_working_bits)
-                HB_CUDA_TRY(cudaMemcpyAsync(b->leftover_working_bits + a, lane.aux64.ptr, nj * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-            if (b->leftover_num_bits)
-                HB_CUDA_TRY(cudaMemcpyAsync(b->leftover_num_bits + a, lane.aux8.ptr, nj, cudaMemcpyDeviceToHost, st));
-        }
+        if (copy_item_arrays_to_host(b, views[j], a, nj, st)) return AWS_OP_ERR;
         HB_CUDA_TRY(cudaEventRecord(lane.retired, st));
         base_out += total;
         return AWS_OP_SUCCESS;
     };
 
-    // A sub-batch is retired (its D2H copies queued) two issues after it was issued; with more lanes than
-    // that, re-using a lane never has to wait for a D2H copy that is still running, so uploads of later
-    // sub-batches and downloads of earlier ones stay concurrent.
-    static_assert(hb_host::kLanes > 3, "lanes must outnumber the issue-to-retire distance");
     // On an error no copy into the caller's buffers may still be running when the call returns.
     auto drain = [&]() {
         for (Lane &lane : ctx->lanes) {
@@ -1039,10 +838,8 @@ int run_host_batch_pipelined(aws_huffman_batch_ctx *ctx, const aws_huffman_batch
         }
         (void)cudaGetLastError();
     };
-    if (chained) depth = 0;  // (nothing to retire: a sub-batch is complete once issued)
-    if (chained && !getenv("AWS_HUFFMAN_BATCH_PIPE_LANES")) lanes_used = 6;  // (a lane is re-used only when everything of its last sub-batch has left)
-    for (size_t j = 0; j < shards + depth; ++j) {
-        if ((j < shards && issue(j)) || (!chained && j >= depth && j - depth < shards && retire(j - depth))) {
+    for (size_t j = 0; j < shards + kRetireLag; ++j) {
+        if ((j < shards && issue(j)) || (j >= kRetireLag && retire(j - kRetireLag))) {
             const int err = aws_last_error();
             drain();
             return aws_raise_error(err ? err : AWS_ERROR_COMPRESSION_DEVICE_FAILURE);
@@ -1051,12 +848,6 @@ int run_host_batch_pipelined(aws_huffman_batch_ctx *ctx, const aws_huffman_batch
     for (Lane &lane : ctx->lanes) {
         if (lane.in_flight) HB_CUDA_TRY(cudaEventSynchronize(lane.retired));
         lane.in_flight = false;
-    }
-    if (chained) {
-        uint64_t tail[2] = {0, 0};  // the output position behind the last sub-batch, the overflow flag
-        HB_CUDA_TRY(cudaMemcpy(tail, chain + shards, sizeof(tail), cudaMemcpyDeviceToHost));
-        base_out = tail[0];
-        overflow = tail[1] != 0;
     }
     b->out_offsets[n] = base_out;
     if (overflow) return aws_raise_error(AWS_ERROR_SHORT_BUFFER);
@@ -1070,26 +861,6 @@ int check_resume(const aws_huffman_batch *b, bool encode) {
         (encode ? (!b->overflow_pattern || !b->overflow_num_bits) : (!b->leftover_working_bits || !b->leftover_num_bits)))
         return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
     return AWS_OP_SUCCESS;
-}
-
-// The device's alias of [p, p + size) when the range lies in pinned (page-locked, mapped) host memory, else
-// nullptr. Kernels can then read and write the caller's buffers in place over PCIe (zero copy).
-template <typename T>
-T *mapped_alias(T *p, uint64_t size) {
-    if (!p || !size) return nullptr;
-    cudaPointerAttributes first{}, last{};
-    if (cudaPointerGetAttributes(&first, p) != cudaSuccess ||
-        cudaPointerGetAttributes(&last, reinterpret_cast<const uint8_t *>(p) + size - 1) != cudaSuccess) {
-        cudaGetLastError();
-        return nullptr;
-    }
-    if (first.type != cudaMemoryTypeHost || last.type != cudaMemoryTypeHost || !first.devicePointer || !last.devicePointer)
-        return nullptr;
-    // one allocation: the aliases are as far apart as the host addresses
-    if (reinterpret_cast<const uint8_t *>(last.devicePointer) - reinterpret_cast<const uint8_t *>(first.devicePointer) !=
-        (ptrdiff_t)(size - 1))
-        return nullptr;
-    return reinterpret_cast<T *>(first.devicePointer);
 }
 
 int run_host_batch(aws_huffman_batch_ctx *ctx, const aws_huffman_batch *b, bool encode, bool resume = false) {
@@ -1106,30 +877,13 @@ int run_host_batch(aws_huffman_batch_ctx *ctx, const aws_huffman_batch *b, bool 
     const uint64_t total_in = b->in_offsets[n];
     const bool slotted = b->out_caps != nullptr;
     if ((total_in && !b->in) || (b->out_capacity && !b->out)) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
-    // ZERO COPY (opt-in: AWS_HUFFMAN_BATCH_ZEROCOPY=1, AWS_HUFFMAN_BATCH_ZC_MODE = 1 input, 2 output, 3 both):
-    // payload buffers in pinned host memory are read and written by the kernels themselves, in place, over
-    // PCIe; only the small per-item arrays are staged. Correct (tests/test_gpu_batch.py::test_zero_copy_host_path)
-    // but MEASURED SLOWER than the copy engines on B200 / PCIe Gen5: kernel-issued reads of host memory run at
-    // 18 GB/s, kernel-issued writes at 48 GB/s, against 55 / 57 GB/s for cudaMemcpyAsync; end to end
-    // 41.8 vs 58.5 GB/s on the 1M-string batch and 26.6 vs 52.1 GB/s on the 1 GiB stream. Kept for callers
-    // with small latency-bound batches and as the measured record of why the host path stages its copies.
-    const uint8_t *zin = nullptr;
-    uint8_t *zout = nullptr;
-    if (!resume && !slotted && total_in >= kZeroCopyMinBytes && getenv("AWS_HUFFMAN_BATCH_ZEROCOPY")) {
-        zin = mapped_alias(b->in, total_in);
-        zout = zin ? mapped_alias(b->out, b->out_capacity) : nullptr;
-    }
-    int zc_mode = 3;
-    if (const char *m = getenv("AWS_HUFFMAN_BATCH_ZC_MODE")) zc_mode = atoi(m);
-    const bool zc_possible = zin && zout;
-    const bool zero_copy_in = zc_possible && (zc_mode & 1), zero_copy_out = zc_possible && (zc_mode & 2);
-    const bool zero_copy = zero_copy_in || zero_copy_out;
-    if (!zero_copy && !resume && !slotted && n >= 2 && total_in >= kPipelineMinBytes && !getenv("AWS_HUFFMAN_BATCH_NO_PIPELINE"))
-        return run_host_batch_pipelined(ctx, b, encode);
+    // (payloads are always staged through device memory, pinned caller buffers too: kernels that read and write pinned
+    // host memory over PCIe measured slower end to end than the copy engines, DESIGN.md 6)
+    if (!resume && !slotted && n >= 2 && total_in >= kPipelineMinBytes) return run_host_batch_pipelined(ctx, b, encode);
 
-    if (!zero_copy_in) HB_CUDA_TRY(ctx->s_in.reserve(total_in + 16));
+    HB_CUDA_TRY(ctx->s_in.reserve(total_in + 16));
     HB_CUDA_TRY(ctx->s_in_off.reserve((n + 1) * sizeof(uint64_t)));
-    if (!zero_copy_out) HB_CUDA_TRY(ctx->s_out.reserve(b->out_capacity + 16));
+    HB_CUDA_TRY(ctx->s_out.reserve(b->out_capacity + 16));
     HB_CUDA_TRY(ctx->s_out_off.reserve((n + 1) * sizeof(uint64_t)));
     HB_CUDA_TRY(ctx->scratch.lens.reserve(n * sizeof(uint64_t)));
     if (slotted) HB_CUDA_TRY(ctx->s_caps.reserve(n * sizeof(uint64_t)));
@@ -1140,7 +894,7 @@ int run_host_batch(aws_huffman_batch_ctx *ctx, const aws_huffman_batch *b, bool 
     if (!encode && b->leftover_working_bits) HB_CUDA_TRY(ctx->s_left_bits.reserve(n * sizeof(uint64_t)));
     if (!encode && b->leftover_num_bits) HB_CUDA_TRY(ctx->s_left_num.reserve(n));
 
-    if (total_in && !zero_copy_in) HB_CUDA_TRY(cudaMemcpyAsync(ctx->s_in.ptr, b->in, total_in, cudaMemcpyHostToDevice, st));
+    if (total_in) HB_CUDA_TRY(cudaMemcpyAsync(ctx->s_in.ptr, b->in, total_in, cudaMemcpyHostToDevice, st));
     HB_CUDA_TRY(cudaMemcpyAsync(ctx->s_in_off.ptr, b->in_offsets, (n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
     if (slotted) {
         HB_CUDA_TRY(cudaMemcpyAsync(ctx->s_out_off.ptr, b->out_offsets, n * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
@@ -1163,9 +917,9 @@ int run_host_batch(aws_huffman_batch_ctx *ctx, const aws_huffman_batch *b, bool 
     hb::BatchView v{};
     v.resume = resume;
     v.n = n;
-    v.in = zero_copy_in ? zin : ctx->s_in.as<uint8_t>();
+    v.in = ctx->s_in.as<uint8_t>();
     v.in_offsets = ctx->s_in_off.as<uint64_t>();
-    v.out = zero_copy_out ? zout : ctx->s_out.as<uint8_t>();
+    v.out = ctx->s_out.as<uint8_t>();
     v.out_capacity = b->out_capacity;
     v.out_offsets = ctx->s_out_off.as<uint64_t>();
     v.out_caps = slotted ? ctx->s_caps.as<uint64_t>() : nullptr;
@@ -1185,24 +939,7 @@ int run_host_batch(aws_huffman_batch_ctx *ctx, const aws_huffman_batch *b, bool 
                 : decode_on_device(ctx, ctx->scratch, v, total_in, st)) != AWS_OP_SUCCESS)
         return AWS_OP_ERR;
 
-    if (b->out_lens)
-        HB_CUDA_TRY(cudaMemcpyAsync(b->out_lens, ctx->scratch.lens.ptr, n * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-    if (b->status) HB_CUDA_TRY(cudaMemcpyAsync(b->status, v.status, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    if (b->consumed)
-        HB_CUDA_TRY(cudaMemcpyAsync(b->consumed, v.consumed, n * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-    if (encode) {
-        if (b->overflow_pattern)
-            HB_CUDA_TRY(cudaMemcpyAsync(
-                b->overflow_pattern, v.overflow_pattern, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-        if (b->overflow_num_bits)
-            HB_CUDA_TRY(cudaMemcpyAsync(b->overflow_num_bits, v.overflow_num_bits, n, cudaMemcpyDeviceToHost, st));
-    } else {
-        if (b->leftover_working_bits)
-            HB_CUDA_TRY(cudaMemcpyAsync(
-                b->leftover_working_bits, v.leftover_working_bits, n * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-        if (b->leftover_num_bits)
-            HB_CUDA_TRY(cudaMemcpyAsync(b->leftover_num_bits, v.leftover_num_bits, n, cudaMemcpyDeviceToHost, st));
-    }
+    if (copy_item_arrays_to_host(b, v, 0, n, st)) return AWS_OP_ERR;
 
     if (slotted) {
         if (b->out_capacity)
@@ -1216,7 +953,7 @@ int run_host_batch(aws_huffman_batch_ctx *ctx, const aws_huffman_batch *b, bool 
     HB_CUDA_TRY(cudaStreamSynchronize(st));
     const uint64_t total_out = b->out_offsets[n];
     if (total_out > b->out_capacity) return aws_raise_error(AWS_ERROR_SHORT_BUFFER);
-    if (total_out && !zero_copy_out) {
+    if (total_out) {
         HB_CUDA_TRY(cudaMemcpyAsync(b->out, v.out, total_out, cudaMemcpyDeviceToHost, st));
         HB_CUDA_TRY(cudaStreamSynchronize(st));
     }
@@ -1842,8 +1579,6 @@ static int hb_ctx_from_codes(
     ctx->no_slots = getenv("AWS_HUFFMAN_BATCH_NO_SLOTS") != nullptr;
     ctx->no_strings = getenv("AWS_HUFFMAN_BATCH_NO_STRINGS") != nullptr;
     ctx->no_fused_stream = getenv("AWS_HUFFMAN_BATCH_NO_FUSED_STREAM") != nullptr;
-    ctx->no_slots_decode = getenv("AWS_HUFFMAN_BATCH_SLOTS_DECODE") == nullptr;  // (opt-in: measured slower, decode_slots.cuh)
-    ctx->no_rows = getenv("AWS_HUFFMAN_BATCH_ROWS") == nullptr;  // (the two-kernel decoder is opt-in: measured slower, decode_rows.cuh)
     HB_CTX_TRY(cudaMalloc(&ctx->d_enc, sizeof(enc)));
     HB_CTX_TRY(cudaMalloc(&ctx->d_lut, (size_t)lut.count * sizeof(uint32_t)));
     HB_CTX_TRY(cudaMemcpy(ctx->d_enc, enc, sizeof(enc), cudaMemcpyHostToDevice));
@@ -1955,7 +1690,7 @@ void aws_huffman_batch_ctx_destroy(struct aws_huffman_batch_ctx *ctx) {
     if (ctx->d_lut2) cudaFree(ctx->d_lut2);
     GrowBuf *bufs[] = {&ctx->s_in,       &ctx->s_in_off,      &ctx->s_out,      &ctx->s_out_off,
                        &ctx->s_caps,     &ctx->s_status,      &ctx->s_consumed, &ctx->s_ovf_pattern,
-                       &ctx->s_ovf_bits, &ctx->s_left_bits,   &ctx->s_left_num, &ctx->s_chain, &ctx->hp_pay,
+                       &ctx->s_ovf_bits, &ctx->s_left_bits,   &ctx->s_left_num, &ctx->hp_pay,
                        &ctx->hp_pay_off, &ctx->hp_dec,        &ctx->hp_dec_off, &ctx->hp_huff,
                        &ctx->hp_prefix,  &ctx->hp_lens,       &ctx->hp_pay_lens, &ctx->hp_dec_status,
                        &ctx->hp_left_bits, &ctx->hp_left_num, &ctx->hp_status};

@@ -167,44 +167,10 @@ def test_seeded_fuzz_runs(script, args):
     print(proc.stdout.strip().splitlines()[-1])
 
 
-def test_rows_decoder_matches_the_oracle(pkg, coders, oracle, oracle_tables, monkeypatch):
-    """The opt-in two-kernel decoder (decode_rows.cuh: rows in a global scratch + compaction pass; the recorded A/B
-    partner of decode_batch_kernel) against the oracle: ragged lengths incl. empty and long strings, corrupted
-    bytes (unknown symbols, bad padding), both tables, every per-item output array."""
-    monkeypatch.setenv("AWS_HUFFMAN_BATCH_ROWS", "1")
-    rng = np.random.default_rng(4242)
-    for table in ("hpack", "test"):
-        ctx = pkg.BatchContext(coders.coder(table), eos_padding=0xFF, device=0)
-        try:
-            for shape in range(4):
-                n = int(rng.integers(1, 5000))
-                lens = [rng.integers(0, 300, size=n), rng.integers(0, 12, size=n), rng.integers(200, 3000, size=n),
-                        np.where(rng.random(n) < 0.3, 0, rng.integers(1, 600, size=n))][shape]
-                offs = np.zeros(n + 1, dtype=np.uint64)
-                offs[1:] = np.cumsum(lens)
-                sampler = refcodec.zipf_symbol_sampler(refcodec.table_arrays(table)[1])
-                data = sampler[rng.integers(0, 65536, size=int(offs[-1]))]
-                enc = oracle.encode_batch(oracle_tables[table], 0xFF, data, offs, 4 * len(data) + 64)
-                total = int(enc["out_offsets"][-1])
-                payload = enc["out"][:total].copy()
-                if shape % 2 and total:  # corrupt some bytes: unknown symbols / truncated codes inside items
-                    hits = rng.integers(0, total, size=max(1, total // 400))
-                    payload[hits] ^= rng.integers(1, 256, size=len(hits)).astype(np.uint8)
-                want = oracle.decode_batch(oracle_tables[table], payload, enc["out_offsets"], 8 * total + 64)
-                got = ctx.decode(payload, enc["out_offsets"], 8 * total + 64)
-                for k in ("out_offsets", "out_lens", "status", "consumed", "leftover_working_bits", "leftover_num_bits"):
-                    assert np.array_equal(got[k], want[k]), (table, shape, k)
-                produced = int(want["out_offsets"][-1])
-                assert np.array_equal(got["out"][:produced], want["out"][:produced]), (table, shape)
-        finally:
-            ctx.close()
-
-
-def test_slots_decoder_matches_the_oracle(pkg, coders, oracle, oracle_tables, monkeypatch):
-    """The opt-in in-place decoder (decode_slots.cuh: stage and rows share one slot per string; recorded A/B partner of
-    decode_batch_kernel) against the oracle, same shapes as the rows decoder's test plus a batch whose first and
-    last strings touch the ends of the input buffer at every 16-byte phase."""
-    monkeypatch.setenv("AWS_HUFFMAN_BATCH_SLOTS_DECODE", "1")
+def test_batch_decoder_matches_the_oracle(pkg, coders, oracle, oracle_tables):
+    """The batch decoder of the host entry point (decode_batch_kernel) against the oracle: ragged lengths incl. empty,
+    very short and long strings, corrupted bytes (unknown symbols, bad padding), both tables, every per-item output
+    array."""
     rng = np.random.default_rng(777)
     for table in ("hpack", "test"):
         ctx = pkg.BatchContext(coders.coder(table), eos_padding=0xFF, device=0)
@@ -233,15 +199,12 @@ def test_slots_decoder_matches_the_oracle(pkg, coders, oracle, oracle_tables, mo
             ctx.close()
 
 
-def test_pipelined_host_path_into_pinned_output(pkg, coders, oracle, oracle_tables, monkeypatch):
-    """The host entry points with a PINNED output buffer and AWS_HUFFMAN_BATCH_CHAIN=1 (opt-in: measured slower than the
-    copy engines, kept as the record) take the chained route of the pipelined host path: the
-    sub-batches' payloads are written into the caller's buffer by a kernel that learns their size and position on
-    the device (no host round trip per sub-batch). Same bytes, offsets and per-item arrays as the oracle — with an
-    odd base address of the buffer, all optional arrays, both directions, and the call-level SHORT_BUFFER (offsets
-    complete, payload of the sub-batches that fit still in place)."""
+def test_pipelined_host_path_into_pinned_output(pkg, coders, oracle, oracle_tables):
+    """The host entry points with a PINNED output buffer take the pipelined host path (the batch is over 40 MB): the
+    sub-batches' payloads are copied into the caller's buffer one after the other. Same bytes, offsets and per-item
+    arrays as the oracle — with an odd base address of the buffer, all optional arrays, both directions, and the
+    call-level SHORT_BUFFER (offsets complete, payload of the sub-batches that fit still in place)."""
     import torch
-    monkeypatch.setenv("AWS_HUFFMAN_BATCH_CHAIN", "1")
     rng = np.random.default_rng(31337)
     ctx = pkg.BatchContext(coders.coder("hpack"), eos_padding=0xFF, device=0)
     try:
