@@ -98,7 +98,7 @@ class LiteralOracle:
         if not huff:
             return OK, payload
         dec = self.h.new_decoder(self.table)
-        out = np.zeros(len(payload) * 2 + 8, dtype=np.uint8)
+        out = np.zeros(len(payload) * 8 + 8, dtype=np.uint8)  # (a code of 1 bit: eight symbols per octet)
         rc, _, olen = self.h.decode_call(dec, np.frombuffer(payload, dtype=np.uint8), out, 0, len(out))
         if rc != OK:
             return rc, b""
