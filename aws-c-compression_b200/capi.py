@@ -17,7 +17,7 @@ AWS_ERROR_COMPRESSION_INVALID_PADDING = 3075
 HPACK_HUFFMAN_SMALLEST, HPACK_HUFFMAN_NEVER, HPACK_HUFFMAN_ALWAYS = 0, 1, 2
 # enum aws_hpack_field_kind
 (HPACK_FIELD_INDEXED, HPACK_FIELD_LITERAL_INCREMENTAL, HPACK_FIELD_LITERAL_WITHOUT_INDEXING,
- HPACK_FIELD_LITERAL_NEVER_INDEXED, HPACK_FIELD_TABLE_SIZE_UPDATE) = range(5)
+ HPACK_FIELD_LITERAL_NEVER_INDEXED, HPACK_FIELD_TABLE_SIZE_UPDATE, HPACK_FIELD_AUTO) = range(6)
 
 
 class CodecError(RuntimeError):
@@ -147,6 +147,7 @@ EXPORTED_SYMBOLS = [
     "aws_huffman_batch_plan_shards", "aws_huffman_batch_concat_offsets",
     "aws_hpack_header_block_decode_batch", "aws_hpack_header_block_encode_batch",
     "aws_hpack_header_block_decode_batch_device", "aws_hpack_header_block_encode_batch_device",
+    "aws_hpack_header_block_encode_records_batch", "aws_hpack_header_block_encode_records_batch_device",
 ]
 
 
@@ -246,8 +247,14 @@ class Library:
         L.aws_hpack_header_block_encode_batch_device.argtypes = [C.c_void_p, P(aws_hpack_header_lists), C.c_uint64,
                                                                  C.c_uint64, C.c_int, C.c_void_p, C.c_uint64, C.c_void_p,
                                                                  C.c_void_p]
+        L.aws_hpack_header_block_encode_records_batch.argtypes = [C.c_void_p, P(aws_hpack_header_lists), C.c_int,
+                                                                  C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]
+        L.aws_hpack_header_block_encode_records_batch_device.argtypes = [
+            C.c_void_p, P(aws_hpack_header_lists), C.c_uint64, C.c_uint64, C.c_int, C.c_void_p, C.c_uint64, C.c_void_p,
+            C.c_void_p, C.c_void_p]
         for name in ("aws_hpack_header_block_decode_batch", "aws_hpack_header_block_encode_batch",
-                     "aws_hpack_header_block_decode_batch_device", "aws_hpack_header_block_encode_batch_device"):
+                     "aws_hpack_header_block_decode_batch_device", "aws_hpack_header_block_encode_batch_device",
+                     "aws_hpack_header_block_encode_records_batch", "aws_hpack_header_block_encode_records_batch_device"):
             getattr(L, name).restype = C.c_int
 
     def last_error(self):
@@ -598,6 +605,30 @@ class BatchContext:
             raise
         return res
 
+    def hpack_encode_records(self, field_offsets, field_kind, field_index, strings, string_offsets, out_capacity,
+                             mode=HPACK_HUFFMAN_SMALLEST, never_indexed=None):
+        """Host buffers: field records (the decoder's, or the caller's own) in, header blocks out ({"out",
+        "out_offsets", "status"}). On failure the CodecError carries them as `result`."""
+        field_offsets = np.ascontiguousarray(field_offsets, dtype=np.uint64)
+        field_kind = np.ascontiguousarray(field_kind, dtype=np.uint8)
+        field_index = np.ascontiguousarray(field_index, dtype=np.uint64)
+        strings = np.ascontiguousarray(strings, dtype=np.uint8)
+        string_offsets = np.ascontiguousarray(string_offsets, dtype=np.uint64)
+        if never_indexed is not None:
+            never_indexed = np.ascontiguousarray(never_indexed, dtype=np.uint8)
+        n = len(field_offsets) - 1
+        res = {"out": np.zeros(max(int(out_capacity), 1), dtype=np.uint8), "out_offsets": np.zeros(n + 1, dtype=np.uint64),
+               "status": np.full(n, -1, dtype=np.int32)}
+        lists = aws_hpack_header_lists(n, _ptr(field_offsets), 0, _ptr(field_kind), _ptr(field_index), _ptr(never_indexed),
+                                       _ptr(strings), 0, _ptr(string_offsets))
+        try:
+            self._blocks_call("aws_hpack_header_block_encode_records_batch", C.byref(lists), mode, _ptr(res["out"]),
+                              int(out_capacity), _ptr(res["out_offsets"]), _ptr(res["status"]))
+        except CodecError as err:
+            err.result = res
+            raise
+        return res
+
     def hpack_decode_blocks_device(self, n, in_, in_offsets, in_size, field_offsets, field_kind, field_index, strings,
                                    string_offsets, status=None, stream=None):
         """Torch CUDA tensors; capacities are the tensors' sizes (string_offsets: 2 * field_capacity + 1)."""
@@ -613,6 +644,16 @@ class BatchContext:
                                        _ptr(string_offsets))
         self._blocks_call("aws_hpack_header_block_encode_batch_device", C.byref(lists), int(num_fields),
                           int(strings_size), mode, _ptr(out), out.numel(), _ptr(out_offsets), stream or 0)
+
+    def hpack_encode_records_device(self, n, field_offsets, num_fields, field_kind, field_index, strings, string_offsets,
+                                    strings_size, out, out_offsets, status=None, mode=HPACK_HUFFMAN_SMALLEST,
+                                    never_indexed=None, out_capacity=None, stream=None):
+        """Torch CUDA tensors; out_capacity defaults to out.numel()."""
+        lists = aws_hpack_header_lists(n, _ptr(field_offsets), 0, _ptr(field_kind), _ptr(field_index), _ptr(never_indexed),
+                                       _ptr(strings), 0, _ptr(string_offsets))
+        self._blocks_call("aws_hpack_header_block_encode_records_batch_device", C.byref(lists), int(num_fields),
+                          int(strings_size), mode, _ptr(out), out.numel() if out_capacity is None else int(out_capacity),
+                          _ptr(out_offsets), _ptr(status), stream or 0)
 
     def encode(self, data, in_offsets, out_capacity, **kw):
         return self._host(True, data, in_offsets, out_capacity, **kw)

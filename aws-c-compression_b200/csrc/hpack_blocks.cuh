@@ -12,9 +12,9 @@
 // and the literal spans. The literals are gathered into a packed batch and decoded by the literal path
 // (hpack_decode_on_device, either route); then a per-block pass picks the final status and per-field passes write
 // the records and the strings, each from the static table below or from the decoded literals.
-// Encode: one thread per field matches the field against the static table and picks its representation; every
-// name and value is framed by the literal path; a warp per 32 fields writes the prefix integers and copies the
-// framed literals the representation uses.
+// Encode: one thread per field picks its representation (the caller's record, or a match against the static table);
+// every name and value is framed by the literal path; for records, one thread per block applies the block rules;
+// a warp per 32 fields writes the prefix integers and copies the framed literals the representation uses.
 #pragma once
 
 #include "hpack_literals.cuh"
@@ -328,43 +328,92 @@ __device__ __forceinline__ bool hpack_bytes_equal(const uint8_t *a, const uint8_
     return true;
 }
 
-// Plan byte of a field: representation in bits 0..2, "name literal" in bit 3, "value literal" in bit 4; the index
-// (0..61) in plan_index.
-enum : uint8_t { kPlanNameLit = 8, kPlanValueLit = 16 };
+// Plan byte of a field: representation in bits 0..2, "name literal" in bit 3, "value literal" in bit 4, "emit
+// nothing" in bit 5 (the field is invalid, or its block is); the index or size in plan_index.
+enum : uint8_t { kPlanNameLit = 8, kPlanValueLit = 16, kPlanSkip = 32 };
+// A record's kind on the encode side: the five representations, or the stateless rules (kFieldAuto).
+constexpr uint8_t kFieldAuto = 5;
 
-// Thread per field: representation (the rules of aws_hpack_header_block_encode_batch), and the field's size on
-// the wire from the framed literals (framed_offsets: name of field f is framed item 2f, its value 2f + 1).
+// Prefix bits and first-octet flags of each representation (RFC 7541 6.1 - 6.3).
+__device__ __forceinline__ uint32_t hpack_prefix_bits(uint32_t kind) { return 0x54467u >> (4 * kind) & 15; }  // 7 6 4 4 5
+__device__ __forceinline__ uint8_t hpack_prefix_flags(uint32_t kind) {
+    return (uint8_t)(0x2010004080ull >> (8 * kind));  // 0x80 0x40 0x00 0x10 0x20
+}
+
+// Thread per field: representation and the field's size on the wire from the framed literals (framed_offsets: name
+// of field f is framed item 2f, its value 2f + 1). field_kind == NULL: every field is kFieldAuto (the rules of
+// aws_hpack_header_block_encode_batch); else the caller's kind and field_index[f] are used as given. A field whose
+// kind is unknown, an INDEXED index 0, or an integer that hpack_read_int refuses (more than 9 continuation octets)
+// gets kPlanSkip and length 0.
 __global__ void hpack_field_plan_kernel(
     uint64_t num_fields, const uint8_t *strings, const uint64_t *string_offsets, const uint8_t *never_indexed,
-    const uint64_t *framed_offsets, uint8_t *plan, uint8_t *plan_index, uint64_t *field_lens) {
+    const uint8_t *field_kind, const uint64_t *field_index, const uint64_t *framed_offsets, uint8_t *plan,
+    uint64_t *plan_index, uint64_t *field_lens) {
     const uint64_t f = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (f >= num_fields) return;
-    const uint64_t n0 = string_offsets[2 * f], v0 = string_offsets[2 * f + 1], v1 = string_offsets[2 * f + 2];
-    const uint8_t *name = strings + n0, *value = strings + v0;
-    const uint64_t name_len = v0 - n0, value_len = v1 - v0;
-    uint32_t name_match = 0, exact = 0;
-    for (uint32_t e = 1; e <= kStaticEntries && !exact; ++e) {
-        const uint32_t s0 = kStaticOff[2 * e - 2], s1 = kStaticOff[2 * e - 1], s2 = kStaticOff[2 * e];
-        if (s1 - s0 != name_len || !hpack_bytes_equal(name, kStaticBlob + s0, name_len)) continue;
-        if (!name_match) name_match = e;
-        if (s2 - s1 == value_len && hpack_bytes_equal(value, kStaticBlob + s1, value_len)) exact = e;
-    }
-    const bool never = never_indexed && never_indexed[f];
+    const uint8_t kind = field_kind ? field_kind[f] : kFieldAuto;
     uint8_t p;
-    uint32_t index;
-    if (!never && exact) {
-        p = kFieldIndexed;
-        index = exact;
+    uint64_t index;
+    if (kind == kFieldAuto) {
+        const uint64_t n0 = string_offsets[2 * f], v0 = string_offsets[2 * f + 1], v1 = string_offsets[2 * f + 2];
+        const uint8_t *name = strings + n0, *value = strings + v0;
+        const uint64_t name_len = v0 - n0, value_len = v1 - v0;
+        uint32_t name_match = 0, exact = 0;
+        for (uint32_t e = 1; e <= kStaticEntries && !exact; ++e) {
+            const uint32_t s0 = kStaticOff[2 * e - 2], s1 = kStaticOff[2 * e - 1], s2 = kStaticOff[2 * e];
+            if (s1 - s0 != name_len || !hpack_bytes_equal(name, kStaticBlob + s0, name_len)) continue;
+            if (!name_match) name_match = e;
+            if (s2 - s1 == value_len && hpack_bytes_equal(value, kStaticBlob + s1, value_len)) exact = e;
+        }
+        const bool never = never_indexed && never_indexed[f];
+        if (!never && exact) {
+            p = kFieldIndexed;
+            index = exact;
+        } else {
+            p = (never ? kFieldNever : kFieldWithout) | kPlanValueLit | (name_match ? 0 : kPlanNameLit);
+            index = name_match;
+        }
+    } else if (kind < kFieldAuto) {
+        index = field_index[f];
+        p = kind;
+        if (kind != kFieldIndexed && kind != kFieldSizeUpdate) p |= kPlanValueLit | (index ? 0 : kPlanNameLit);
+        if (kind == kFieldIndexed && index == 0) p |= kPlanSkip;
     } else {
-        p = (never ? kFieldNever : kFieldWithout) | kPlanValueLit | (name_match ? 0 : kPlanNameLit);
-        index = name_match;
+        p = kPlanSkip;
+        index = 0;
     }
-    uint64_t len = hpack_int_bytes(index, p == kFieldIndexed ? 7 : 4);
-    if (p & kPlanNameLit) len += framed_offsets[2 * f + 1] - framed_offsets[2 * f];
-    if (p & kPlanValueLit) len += framed_offsets[2 * f + 2] - framed_offsets[2 * f + 1];
+    uint64_t len = 0;
+    if (!(p & kPlanSkip)) {
+        len = hpack_int_bytes(index, hpack_prefix_bits(p & 7));
+        if (len > 10) p |= kPlanSkip;
+        if (p & kPlanNameLit) len += framed_offsets[2 * f + 1] - framed_offsets[2 * f];
+        if (p & kPlanValueLit) len += framed_offsets[2 * f + 2] - framed_offsets[2 * f + 1];
+    }
     plan[f] = p;
-    plan_index[f] = (uint8_t)index;
-    field_lens[f] = len;
+    plan_index[f] = index;
+    field_lens[f] = p & kPlanSkip ? 0 : len;
+}
+
+// Thread per block, after the plan and before the scan of field lengths (records only): a block is invalid when a
+// field of it is marked kPlanSkip, or when a size update follows a field that is not one (the decoder's rule). An
+// invalid block gets INVALID_ARGUMENT and every field of it kPlanSkip and length 0: it encodes to zero octets.
+__global__ void hpack_block_check_kernel(uint64_t n, const uint64_t *field_offsets, uint8_t *plan, uint64_t *field_lens,
+                                         int32_t *status) {
+    const uint64_t b = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= n) return;
+    const uint64_t f0 = field_offsets[b], f1 = field_offsets[b + 1];
+    bool ok = true, seen_field = false;
+    for (uint64_t f = f0; f < f1 && ok; ++f) {
+        const uint8_t p = plan[f], kind = p & 7;
+        ok = !(p & kPlanSkip) && !(kind == kFieldSizeUpdate && seen_field);
+        seen_field |= kind != kFieldSizeUpdate;
+    }
+    if (status) status[b] = ok ? kStatusOk : kStatusInvalidArgument;
+    if (ok) return;
+    for (uint64_t f = f0; f < f1; ++f) {
+        plan[f] |= kPlanSkip;
+        field_lens[f] = 0;
+    }
 }
 
 // out_offsets[b] = the wire position of list b's first field.
@@ -375,21 +424,21 @@ __global__ void hpack_block_offsets_kernel(uint64_t n, const uint64_t *field_off
 }
 
 // A warp takes 32 fields: every lane writes its field's prefix integer, then the warp copies the 32 name literals
-// and the 32 value literals (those the plan uses). Never writes at or after out + out_capacity.
+// and the 32 value literals (those the plan uses). Fields marked kPlanSkip write nothing. Never writes at or after
+// out + out_capacity.
 __global__ void __launch_bounds__(256) hpack_field_emit_kernel(
-    uint64_t num_fields, const uint8_t *plan, const uint8_t *plan_index, const uint8_t *framed,
+    uint64_t num_fields, const uint8_t *plan, const uint64_t *plan_index, const uint8_t *framed,
     const uint64_t *framed_offsets, const uint64_t *field_pos, uint8_t *out, uint64_t out_capacity) {
     __shared__ MoveJob s_jobs[8][32];
     const uint32_t lane = lane_id(), warp = threadIdx.x >> 5;
     const uint64_t f = ((uint64_t)blockIdx.x * 8 + warp) * 32 + lane;
     MoveJob name = {nullptr, nullptr, 0}, value = {nullptr, nullptr, 0};
-    if (f < num_fields) {
+    if (f < num_fields && !(plan[f] & kPlanSkip)) {
         const uint8_t p = plan[f], kind = p & 7;
-        const uint32_t index = plan_index[f];
+        const uint64_t index = plan_index[f];
         uint64_t pos = field_pos[f];
-        const uint32_t prefix_bits = kind == kFieldIndexed ? 7 : 4;
-        hpack_put_int(out, pos, out_capacity, index, prefix_bits,
-                      kind == kFieldIndexed ? 0x80 : (kind == kFieldNever ? 0x10 : 0x00));
+        const uint32_t prefix_bits = hpack_prefix_bits(kind);
+        hpack_put_int(out, pos, out_capacity, index, prefix_bits, hpack_prefix_flags(kind));
         pos += hpack_int_bytes(index, prefix_bits);
         for (uint32_t w = 0; w < 2; ++w) {
             if (!(p & (w ? kPlanValueLit : kPlanNameLit))) continue;

@@ -1247,13 +1247,17 @@ int hpack_blocks_decode_on_device(
     return AWS_OP_SUCCESS;
 }
 
+// field_kind == NULL: every field is AUTO (aws_hpack_header_block_encode_batch); else the caller's records, with
+// the per-block status (optional) of aws_hpack_header_block_encode_records_batch.
 int hpack_blocks_encode_on_device(
     aws_huffman_batch_ctx *ctx, uint64_t n, const uint64_t *field_offsets, uint64_t num_fields, const uint8_t *never_indexed,
-    const uint8_t *strings, const uint64_t *string_offsets, uint64_t strings_size, uint32_t mode, uint8_t *out,
-    uint64_t out_capacity, uint64_t *out_offsets, cudaStream_t st) {
+    const uint8_t *field_kind, const uint64_t *field_index, const uint8_t *strings, const uint64_t *string_offsets,
+    uint64_t strings_size, uint32_t mode, uint8_t *out, uint64_t out_capacity, uint64_t *out_offsets, int32_t *status,
+    cudaStream_t st) {
     hb_host::BlockBufs &B = ctx->blk;
     if (n == 0 || num_fields == 0) {
         HB_CUDA_TRY(cudaMemsetAsync(out_offsets, 0, (n + 1) * sizeof(uint64_t), st));
+        if (status && n) HB_CUDA_TRY(cudaMemsetAsync(status, 0, n * sizeof(int32_t), st));
         return AWS_OP_SUCCESS;
     }
     const uint64_t F = num_fields;
@@ -1263,26 +1267,31 @@ int hpack_blocks_encode_on_device(
     HB_CUDA_TRY(B.framed.reserve(framed_cap + 64));
     HB_CUDA_TRY(B.framed_offsets.reserve((2 * F + 1) * sizeof(uint64_t)));
     HB_CUDA_TRY(B.plan.reserve(F));
-    HB_CUDA_TRY(B.plan_index.reserve(F));
+    HB_CUDA_TRY(B.plan_index.reserve(F * sizeof(uint64_t)));
     HB_CUDA_TRY(B.field_lens.reserve(F * sizeof(uint64_t)));
     HB_CUDA_TRY(B.field_pos.reserve((F + 1) * sizeof(uint64_t)));
     const uint64_t *framed_offsets = B.framed_offsets.as<uint64_t>();
     uint64_t *field_pos = B.field_pos.as<uint64_t>();
 
     // 1. every name and value framed (indexed names too: simpler than a compacted batch); 2. representation and size
-    // per field; 3. wire positions of fields and blocks; 4. prefixes and literals
+    // per field, and for records the block rules; 3. wire positions of fields and blocks; 4. prefixes and literals
     if (hpack_encode_on_device(ctx, 2 * F, strings, string_offsets, strings_size, mode, B.framed.as<uint8_t>(), framed_cap,
                                B.framed_offsets.as<uint64_t>(), st))
         return AWS_OP_ERR;
     hb::hpack_field_plan_kernel<<<grid_of(F, 256), 256, 0, st>>>(
-        F, strings, string_offsets, never_indexed, framed_offsets, B.plan.as<uint8_t>(), B.plan_index.as<uint8_t>(),
-        B.field_lens.as<uint64_t>());
+        F, strings, string_offsets, never_indexed, field_kind, field_index, framed_offsets, B.plan.as<uint8_t>(),
+        B.plan_index.as<uint64_t>(), B.field_lens.as<uint64_t>());
     ++ctx->launches;
+    if (field_kind) {
+        hb::hpack_block_check_kernel<<<grid_of(n, 256), 256, 0, st>>>(
+            n, field_offsets, B.plan.as<uint8_t>(), B.field_lens.as<uint64_t>(), status);
+        ++ctx->launches;
+    }
     if (launch_scan(ctx, ctx->scratch, B.field_lens.as<uint64_t>(), field_pos, F, st)) return AWS_OP_ERR;
     hb::hpack_block_offsets_kernel<<<grid_of(n + 1, 256), 256, 0, st>>>(n, field_offsets, field_pos, out_offsets);
     ++ctx->launches;
     hb::hpack_field_emit_kernel<<<grid_of(F, 256), 256, 0, st>>>(
-        F, B.plan.as<uint8_t>(), B.plan_index.as<uint8_t>(), B.framed.as<uint8_t>(), framed_offsets, field_pos, out,
+        F, B.plan.as<uint8_t>(), B.plan_index.as<uint64_t>(), B.framed.as<uint8_t>(), framed_offsets, field_pos, out,
         out_capacity);
     ++ctx->launches;
     HB_CUDA_TRY(cudaGetLastError());
@@ -1355,10 +1364,13 @@ int hpack_blocks_decode_host(
     return AWS_OP_SUCCESS;
 }
 
+// records: field_kind and field_index are read (aws_hpack_header_block_encode_records_batch), status is optional.
 int hpack_blocks_encode_host(
-    aws_huffman_batch_ctx *ctx, const aws_hpack_header_lists *in, uint32_t mode, uint8_t *out, uint64_t out_capacity,
-    uint64_t *out_off) {
-    if (!ctx || check_block_lists(in, false) || !out_off || (out_capacity && !out)) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    aws_huffman_batch_ctx *ctx, const aws_hpack_header_lists *in, bool records, uint32_t mode, uint8_t *out,
+    uint64_t out_capacity, uint64_t *out_off, int32_t *status) {
+    if (!ctx || check_block_lists(in, false) || !out_off || (out_capacity && !out) ||
+        (records && (!in->field_kind || !in->field_index)))
+        return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
     const uint64_t n = in->n;
     if (n == 0) {
         out_off[0] = 0;
@@ -1388,11 +1400,26 @@ int hpack_blocks_encode_host(
         HB_CUDA_TRY(cudaMemcpyAsync(B.s_never.ptr, in->never_indexed, F, cudaMemcpyHostToDevice, st));
         never = B.s_never.as<uint8_t>();
     }
-    if (hpack_blocks_encode_on_device(ctx, n, B.s_field_offsets.as<uint64_t>(), F, never, ctx->s_in.as<uint8_t>(),
+    const uint8_t *kind = nullptr;
+    const uint64_t *index = nullptr;
+    if (records) {
+        HB_CUDA_TRY(B.s_kind.reserve(F + 1));
+        HB_CUDA_TRY(B.s_index.reserve((F + 1) * sizeof(uint64_t)));
+        HB_CUDA_TRY(ctx->s_status.reserve(n * sizeof(int32_t)));
+        if (F) {
+            HB_CUDA_TRY(cudaMemcpyAsync(B.s_kind.ptr, in->field_kind, F, cudaMemcpyHostToDevice, st));
+            HB_CUDA_TRY(cudaMemcpyAsync(B.s_index.ptr, in->field_index, F * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
+        }
+        kind = B.s_kind.as<uint8_t>();
+        index = B.s_index.as<uint64_t>();
+    }
+    int32_t *d_status = records ? ctx->s_status.as<int32_t>() : nullptr;
+    if (hpack_blocks_encode_on_device(ctx, n, B.s_field_offsets.as<uint64_t>(), F, never, kind, index, ctx->s_in.as<uint8_t>(),
                                       ctx->s_in_off.as<uint64_t>(), S, mode, ctx->s_out.as<uint8_t>(), out_capacity,
-                                      ctx->s_out_off.as<uint64_t>(), st))
+                                      ctx->s_out_off.as<uint64_t>(), d_status, st))
         return AWS_OP_ERR;
     HB_CUDA_TRY(cudaMemcpyAsync(out_off, ctx->s_out_off.ptr, (n + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    if (status && d_status) HB_CUDA_TRY(cudaMemcpyAsync(status, d_status, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     HB_CUDA_TRY(cudaStreamSynchronize(st));
     const uint64_t total = out_off[n];
     if (total > out_capacity) return aws_raise_error(AWS_ERROR_SHORT_BUFFER);
@@ -1843,7 +1870,14 @@ int aws_hpack_header_block_encode_batch(
     struct aws_huffman_batch_ctx *ctx, const struct aws_hpack_header_lists *in, enum aws_hpack_huffman_mode mode,
     uint8_t *out, uint64_t out_capacity, uint64_t *out_offsets) {
     if ((unsigned)mode > (unsigned)AWS_HPACK_HUFFMAN_ALWAYS) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
-    return hpack_blocks_encode_host(ctx, in, (uint32_t)mode, out, out_capacity, out_offsets);
+    return hpack_blocks_encode_host(ctx, in, false, (uint32_t)mode, out, out_capacity, out_offsets, nullptr);
+}
+
+int aws_hpack_header_block_encode_records_batch(
+    struct aws_huffman_batch_ctx *ctx, const struct aws_hpack_header_lists *in, enum aws_hpack_huffman_mode mode,
+    uint8_t *out, uint64_t out_capacity, uint64_t *out_offsets, int32_t *status) {
+    if ((unsigned)mode > (unsigned)AWS_HPACK_HUFFMAN_ALWAYS) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    return hpack_blocks_encode_host(ctx, in, true, (uint32_t)mode, out, out_capacity, out_offsets, status);
 }
 
 int aws_hpack_header_block_decode_batch_device(
@@ -1866,9 +1900,25 @@ int aws_hpack_header_block_encode_batch_device(
     cudaStream_t st;
     if (device_call_begin(ctx, cuda_stream, &st)) return AWS_OP_ERR;
     return device_call_end(ctx, st,
-                           hpack_blocks_encode_on_device(ctx, in->n, in->field_offsets, num_fields, in->never_indexed, in->strings,
-                                                         in->string_offsets, strings_size, (uint32_t)mode, out, out_capacity,
-                                                         out_offsets, st));
+                           hpack_blocks_encode_on_device(ctx, in->n, in->field_offsets, num_fields, in->never_indexed, nullptr,
+                                                         nullptr, in->strings, in->string_offsets, strings_size, (uint32_t)mode,
+                                                         out, out_capacity, out_offsets, nullptr, st));
+}
+
+int aws_hpack_header_block_encode_records_batch_device(
+    struct aws_huffman_batch_ctx *ctx, const struct aws_hpack_header_lists *in, uint64_t num_fields,
+    uint64_t strings_size, enum aws_hpack_huffman_mode mode, uint8_t *out, uint64_t out_capacity, uint64_t *out_offsets,
+    int32_t *status, void *cuda_stream) {
+    if (!ctx || check_block_lists(in, false) || !in->field_kind || !in->field_index || !out_offsets ||
+        (out_capacity && !out) || (strings_size && !in->strings) || (unsigned)mode > (unsigned)AWS_HPACK_HUFFMAN_ALWAYS)
+        return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    cudaStream_t st;
+    if (device_call_begin(ctx, cuda_stream, &st)) return AWS_OP_ERR;
+    return device_call_end(ctx, st,
+                           hpack_blocks_encode_on_device(ctx, in->n, in->field_offsets, num_fields, in->never_indexed,
+                                                         in->field_kind, in->field_index, in->strings, in->string_offsets,
+                                                         strings_size, (uint32_t)mode, out, out_capacity, out_offsets, status,
+                                                         st));
 }
 
 int aws_huffman_get_encoded_length_batch(

@@ -8,7 +8,8 @@
  *
  * The wire layer of a header block is stateless: where each representation starts, its kind, its integers, its
  * literals and the static table (indices 1..61) are all read here. Only the meaning of an index >= 62 depends on
- * the connection's dynamic table, which stays the caller's: such references are reported, not resolved.
+ * the connection's dynamic table, which stays the caller's: such references are reported, not resolved, and the
+ * records encoder writes the references and insertions the caller chose.
  */
 #include <aws/compression/hpack_string_batch.h>
 
@@ -21,6 +22,7 @@ enum aws_hpack_field_kind {
     AWS_HPACK_FIELD_LITERAL_WITHOUT_INDEXING = 2, /* 6.2.2 0000xxxx: name index (4-bit prefix)                  */
     AWS_HPACK_FIELD_LITERAL_NEVER_INDEXED = 3,    /* 6.2.3 0001xxxx: name index (4-bit prefix)                  */
     AWS_HPACK_FIELD_TABLE_SIZE_UPDATE = 4,        /* 6.3   001xxxxx: new maximum size (5-bit prefix)            */
+    AWS_HPACK_FIELD_AUTO = 5,                     /* encode records only: the stateless rules choose (no decode) */
 };
 
 /*
@@ -34,8 +36,8 @@ struct aws_hpack_header_lists {
     uint64_t *field_offsets;   /* n + 1 */
     uint64_t field_capacity;   /* decode: entries available in field_kind, field_index (and 2 * this + 1 in
                                   string_offsets) */
-    uint8_t *field_kind;       /* decode: written (enum aws_hpack_field_kind); encode: ignored */
-    uint64_t *field_index;     /* decode: written; encode: ignored */
+    uint8_t *field_kind;       /* decode: written (enum aws_hpack_field_kind); encode records: read; encode: ignored */
+    uint64_t *field_index;     /* decode: written; encode records: read; encode: ignored */
     uint8_t *never_indexed;    /* encode: optional (NULL = none), one flag per field: sensitive fields (7.1.3) */
     uint8_t *strings;
     uint64_t strings_capacity; /* decode: bytes available in strings; encode: ignored */
@@ -102,14 +104,48 @@ int aws_hpack_header_block_encode_batch(
     uint64_t *out_offsets);
 
 /*
+ * The encoder for a caller that keeps its own dynamic table: field f is written as the record (field_kind[f],
+ * field_index[f]) says, the records aws_hpack_header_block_decode_batch writes (in->field_kind and in->field_index
+ * must not be NULL). Per field_kind[f]:
+ *     INDEXED                    6.1   1xxxxxxx  field_index (static or dynamic; 0 is invalid)
+ *     LITERAL_INCREMENTAL        6.2.1 01xxxxxx  name index field_index (0: the name follows as a literal), value
+ *     LITERAL_WITHOUT_INDEXING   6.2.2 0000xxxx  as above
+ *     LITERAL_NEVER_INDEXED      6.2.3 0001xxxx  as above
+ *     TABLE_SIZE_UPDATE          6.3   001xxxxx  field_index is the new maximum size
+ *     AUTO                       the rules of aws_hpack_header_block_encode_batch, never_indexed[f] included;
+ *                                field_index is ignored
+ * Indices are written as given: there is no static lookup for an explicit kind, so encoding the records a decode
+ * returned gives back the decoded block (with the same Huffman choices). The caller decides which fields enter its
+ * table (INCREMENTAL) and when its size changes; the device does the octets. Literals are framed by `mode`. The
+ * strings a representation does not send are ignored (the name and value of INDEXED and TABLE_SIZE_UPDATE, the name
+ * behind a non-zero name index): empty strings, or Appendix A strings as a decode writes them, are both fine.
+ *
+ * status (optional, n) per block: 0, or AWS_ERROR_INVALID_ARGUMENT when the block holds a kind above AUTO, INDEXED
+ * with index 0, a TABLE_SIZE_UPDATE after a field that is not one, or an integer a decoder refuses (over 9
+ * continuation octets, i.e. at or above 2^63 plus the prefix's maximum). An invalid block encodes to zero octets
+ * (out_offsets[i + 1] == out_offsets[i]); the other blocks are not affected. Offsets, capacity and
+ * AWS_ERROR_SHORT_BUFFER are as in aws_hpack_header_block_encode_batch; status is complete in every case the
+ * offsets are.
+ */
+AWS_COMPRESSION_API
+int aws_hpack_header_block_encode_records_batch(
+    struct aws_huffman_batch_ctx *ctx,
+    const struct aws_hpack_header_lists *in,
+    enum aws_hpack_huffman_mode mode,
+    uint8_t *out,
+    uint64_t out_capacity,
+    uint64_t *out_offsets,
+    int32_t *status);
+
+/*
  * The same with device pointers (every array of `out` / `in` and `in`, `in_offsets`, `status`, `out`, `out_offsets`
  * live on the device); work is enqueued on cuda_stream (NULL = the context's stream). The caller reads the offsets
  * to learn the sizes and checks them against its capacities; nothing is written past a capacity.
  *
  * decode: in_size == in_offsets[n]. The call waits once, after the structural pass, for three totals (fields,
  * literals, literal octets): the literal decoder's launch is sized from them.
- * encode: num_fields == in->field_offsets[in->n], strings_size == in->string_offsets[2 * num_fields]; it does
- * not wait.
+ * encode, encode records: num_fields == in->field_offsets[in->n], strings_size == in->string_offsets[2 *
+ * num_fields]; they do not wait and read nothing back.
  */
 AWS_COMPRESSION_API
 int aws_hpack_header_block_decode_batch_device(
@@ -132,6 +168,19 @@ int aws_hpack_header_block_encode_batch_device(
     uint8_t *out,
     uint64_t out_capacity,
     uint64_t *out_offsets,
+    void *cuda_stream);
+
+AWS_COMPRESSION_API
+int aws_hpack_header_block_encode_records_batch_device(
+    struct aws_huffman_batch_ctx *ctx,
+    const struct aws_hpack_header_lists *in,
+    uint64_t num_fields,
+    uint64_t strings_size,
+    enum aws_hpack_huffman_mode mode,
+    uint8_t *out,
+    uint64_t out_capacity,
+    uint64_t *out_offsets,
+    int32_t *status,
     void *cuda_stream);
 
 AWS_EXTERN_C_END

@@ -2,6 +2,9 @@
 """HPACK header blocks, device pointers: a seeded request mix of 256K header lists of 8-24 fields through
 aws_hpack_header_block_encode_batch_device and _decode_batch_device, beside the string-literal calls on the same
 names and values, so that the cost of the block layer is visible. One JSON line (profiles/r3_header_blocks.json).
+With --records: the same lists through aws_hpack_header_block_encode_records_batch_device instead, with records from
+an encoder-side dynamic table (EncoderTable of tests/hpack_records_oracle.py, 4096 octets) per connection of 64 consecutive lists, built on the
+host and not timed; the blocks decode back to exactly those records (profiles/r3_header_block_records.json).
 
 Mix per field: 25 % an exact Appendix A entry (indexed), 45 % an Appendix A name with a value, 30 % one of 32
 custom names with a value; values of 8-256 octets of Zipf-sampled HPACK symbols (tests/refcodec.py); 5 % of the
@@ -19,6 +22,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 import __graft_entry__ as graft  # noqa: E402
+import hpack_records_oracle as _rec  # noqa: E402
 import refcodec  # noqa: E402
 
 _spec = importlib.util.spec_from_file_location(
@@ -126,6 +130,60 @@ def round_trip(ctx, lists, dev, reps=1, stream=None):
     return r
 
 
+def policy_records(lists, per_connection=64, max_size=4096):
+    """Host arrays (field_offsets, field_kind, field_index, strings, string_offsets) of the records an encoder with its
+    own dynamic table writes for the lists: a fresh EncoderTable every `per_connection` lists."""
+    fo, strings, so, never = [t.cpu().numpy() for t in lists]
+    fo, so, never, raw = fo.tolist(), so.tolist(), never.tolist(), strings.tobytes()
+    blocks = []
+    for b in range(len(fo) - 1):
+        if b % per_connection == 0:
+            table = _rec.EncoderTable(max_size)
+        f0, f1 = fo[b], fo[b + 1]
+        headers = [(raw[so[2 * f]:so[2 * f + 1]], raw[so[2 * f + 1]:so[2 * f + 2]]) for f in range(f0, f1)]
+        blocks.append(table.records(headers, never[f0:f1]))
+    return _rec.records_batch(blocks)
+
+
+def records_leg(ctx, records, dev, reps=8, stream=None):
+    """records through encode_records_batch_device (timed: CUDA events, first two repetitions are warm-up), then
+    decoded back; returns the decoded arrays, the block size and the times."""
+    fo, kind, index, strings, so = [torch.from_numpy(np.require(a, requirements="W").view(np.int64) if a.dtype == np.uint64
+                                                     else np.require(a, requirements="W")).to(dev) for a in records]
+    n, F, S = fo.numel() - 1, kind.numel(), strings.numel()
+    stream = stream or torch.cuda.Stream(dev)
+    out = torch.empty(S + 12 * F + 64, dtype=torch.uint8, device=dev)
+    out_off = torch.zeros(n + 1, dtype=torch.int64, device=dev)
+    status = torch.ones(n, dtype=torch.int32, device=dev)
+    r = {"field_offsets": torch.zeros(n + 1, dtype=torch.int64, device=dev),
+         "field_kind": torch.empty(F, dtype=torch.uint8, device=dev),
+         "field_index": torch.empty(F, dtype=torch.int64, device=dev),
+         "strings": torch.empty(S + 64, dtype=torch.uint8, device=dev),
+         "string_offsets": torch.zeros(2 * F + 1, dtype=torch.int64, device=dev),
+         "status": torch.ones(n, dtype=torch.int32, device=dev)}
+    times = []
+    cs = stream.cuda_stream
+    with torch.cuda.stream(stream):
+        for rep in range(reps):
+            ev = [torch.cuda.Event(enable_timing=True) for _ in range(2)]
+            ev[0].record(stream)
+            ctx.hpack_encode_records_device(n, fo, F, kind, index, strings, so, S, out, out_off, status, mode=0,
+                                            stream=cs)
+            ev[1].record(stream)
+            torch.cuda.synchronize(dev)
+            if rep >= 2:
+                times.append(ev[0].elapsed_time(ev[1]))
+        in_size = int(out_off[-1].item())
+        ctx.hpack_decode_blocks_device(n, out, out_off, in_size, r["field_offsets"], r["field_kind"], r["field_index"],
+                                       r["strings"], r["string_offsets"], status=r["status"], stream=cs)
+        torch.cuda.synchronize(dev)
+    assert int(status.abs().sum().item()) == 0 and int(r["status"].abs().sum().item()) == 0
+    assert torch.equal(r["field_offsets"], fo) and torch.equal(r["field_kind"], kind)
+    assert torch.equal(r["field_index"], index) and torch.equal(r["string_offsets"], so)
+    assert torch.equal(r["strings"][:S], strings)
+    return {"block_bytes": in_size, "times": times, "fields": F}
+
+
 def card():
     name = torch.cuda.get_device_name(0)
     try:
@@ -137,6 +195,7 @@ def card():
 
 
 def main():
+    records_mode = "--records" in sys.argv
     pkg = graft.load_package()
     dev = torch.device("cuda", 0)
     torch.cuda.set_device(dev)
@@ -145,12 +204,32 @@ def main():
     fo, strings, so, never = lists
     F, S = (so.numel() - 1) // 2, strings.numel()
     ctx = pkg.BatchContext(pkg.coders_library().coder("hpack"), eos_padding=0xFF, device=0)
+    if records_mode:
+        records = policy_records(lists)
     r = round_trip(ctx, lists, dev, reps=8)
     assert int(r["status"].abs().sum().item()) == 0 and torch.equal(r["field_offsets"], fo)
     assert torch.equal(r["string_offsets"], so) and torch.equal(r["strings"][:S], strings)
     t = {k: float(np.median(v)) for k, v in r["times"].items()}
     moved = r["block_bytes"] + S
     name, power = card()
+    if records_mode:
+        k = records_leg(ctx, records, dev)
+        kinds = np.bincount(records[1], minlength=5)
+        print(json.dumps({
+            "workload": "hpack header blocks from records (RFC 7541 2.3, 4, 6): the lists of r3_header_blocks.json, "
+                        "records of an encoder-side dynamic table of 4096 octets per connection of 64 lists (built on "
+                        "the host, not timed), SMALLEST mode, device pointers",
+            "header_lists": n, "connections": (n + 63) // 64, "fields": F, "string_bytes": S,
+            "records": {"indexed_static": int(((records[1] == 0) & (records[2] <= 61)).sum()),
+                        "indexed_dynamic": int(((records[1] == 0) & (records[2] > 61)).sum()),
+                        "incremental": int(kinds[1]), "never_indexed": int(kinds[3])},
+            "block_bytes": k["block_bytes"], "stateless_block_bytes": r["block_bytes"],
+            "encode_records_ms": float(np.median(k["times"])), "stateless_encode_ms": t["encode"],
+            "round_trip": "decoded records identical to the encoded ones",
+            "repetitions": len(k["times"]), "statistic": "median after 2 warm-up repetitions",
+            "gpu": name, "power_limit": power}))
+        ctx.close()
+        return
     print(json.dumps({
         "workload": "hpack header blocks (RFC 7541 6), %d header lists of 8-24 fields (25%% exact static, 45%% static "
                     "name, 30%% custom name; values 8-256 B Zipf), SMALLEST mode, device pointers" % n,
