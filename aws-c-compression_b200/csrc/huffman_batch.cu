@@ -49,11 +49,17 @@ void hb_note_cuda_error(cudaError_t err, const char *what, int line) {
 }  // namespace
 
 namespace hb_host {
-// Device buffer that only ever grows.
+// Device buffer that only ever grows; freed with its owner.
 struct GrowBuf {
     void *ptr = nullptr;
     size_t bytes = 0;
 
+    GrowBuf() = default;
+    GrowBuf(const GrowBuf &) = delete;
+    GrowBuf &operator=(const GrowBuf &) = delete;
+    ~GrowBuf() {
+        if (ptr) cudaFree(ptr);
+    }
     cudaError_t reserve(size_t want) {
         if (want <= bytes) return cudaSuccess;
         size_t grown = std::max(want, bytes + bytes / 2);
@@ -66,11 +72,6 @@ struct GrowBuf {
         bytes = grown;
         return cudaSuccess;
     }
-    void release() {
-        if (ptr) cudaFree(ptr);
-        ptr = nullptr;
-        bytes = 0;
-    }
     template <typename T>
     T *as() const {
         return static_cast<T *>(ptr);
@@ -80,11 +81,6 @@ struct GrowBuf {
 struct Scratch {
     GrowBuf lens, tile_state, tile_first, chunks, chunk_lens, chunk_offsets, fused, slot_base, deferred, str_ctl, str_state,
         str_tiles, str_bits, str_bits_first;
-    void release() {
-        GrowBuf *all[] = {&lens,     &tile_state, &tile_first, &chunks,  &chunk_lens, &chunk_offsets, &fused,
-                          &slot_base, &deferred,  &str_ctl,    &str_state, &str_tiles, &str_bits,     &str_bits_first};
-        for (GrowBuf *g : all) g->release();
-    }
 };
 
 // lanes of the pipelined host path (round 2, 12 MiB sub-batches: retired one issue later with 4 lanes 60.9,
@@ -97,17 +93,11 @@ struct Lane {
     uint64_t *h_total = nullptr;  // pinned: the sub-batch's output size
     Scratch scratch;
     GrowBuf in, in_off, out, out_off, lens, status, consumed, aux32, aux8, aux64;
-    void release() {
-        GrowBuf *all[] = {&in, &in_off, &out, &out_off, &lens, &status, &consumed, &aux32, &aux8, &aux64};
-        for (GrowBuf *g : all) g->release();
-        scratch.release();
+    ~Lane() {
         if (h_total) cudaFreeHost(h_total);
         if (kernels_done) cudaEventDestroy(kernels_done);
         if (retired) cudaEventDestroy(retired);
         if (stream) cudaStreamDestroy(stream);
-        h_total = nullptr;
-        kernels_done = retired = nullptr;
-        stream = nullptr;
     }
 };
 // HPACK header blocks (hpack_blocks.cuh): per-block counts and bases, parsed fields, literal spans and the decoded
@@ -118,17 +108,19 @@ struct BlockBufs {
         plan_index, field_lens, field_pos, framed, framed_offsets, s_field_offsets, s_never, s_kind, s_index,
         s_string_offsets;
     uint64_t *h_totals = nullptr;  // pinned: fields, literals, literal octets
-    void release() {
-        GrowBuf *all[] = {&num_fields, &num_lits,      &lit_bytes,  &struct_status, &out_fields,      &status,
-                          &field_base, &lit_base,      &lit_byte_base, &f_kind,     &f_index,         &f_block,
-                          &f_lits,     &lit_src,       &lit_offsets, &lits,         &dec,             &dec_offsets,
-                          &lit_status, &str_lens,      &plan,       &plan_index,    &field_lens,      &field_pos,
-                          &framed,     &framed_offsets, &s_field_offsets, &s_never, &s_kind,          &s_index,
-                          &s_string_offsets};
-        for (GrowBuf *g : all) g->release();
+    ~BlockBufs() {
         if (h_totals) cudaFreeHost(h_totals);
-        h_totals = nullptr;
     }
+};
+// Shared-memory layout of decode_batch_kernel<framed> (decode_batch_fast): [LUT2][team 0: stage, rows][team 1: ...].
+struct DecLayout {
+    size_t stage_bytes = 0, rows_bytes = 0, smem = 0;
+};
+// Shared memory of the single-stream kernels (decode_stream_fast), and whether the fused kernel runs.
+struct StreamLayout {
+    uint32_t row_words = 0;
+    size_t smem = 0, smem_staged = 0, fused_smem = 0;
+    bool fused = false;
 };
 }  // namespace hb_host
 using hb_host::GrowBuf;
@@ -151,10 +143,13 @@ struct aws_huffman_batch_ctx {
     // pipelined host path: independent lanes (stream + scratch + staging) so that the H2D copy of one
     // sub-batch, the kernels of the next and the D2H copy of the previous one overlap
     hb_host::Lane lanes[hb_host::kLanes];
+    // launch configuration, fixed at creation (configure_kernels): resident blocks per SM, decode layouts
     int sm_count = 148;
-    int enc_blocks_per_sm[2] = {0, 0};  // resident blocks per SM of encode_tiled_kernel<seg>
+    int enc_blocks_per_sm[2] = {0, 0};  // encode_tiled_kernel<seg>
     int enc_slots_blocks_per_sm = 0;
-    int str_blocks_per_sm[3] = {0, 0, 0};  // str_bits_kernel, str_pack_kernel, str_scan_kernel
+    int str_blocks_per_sm[2] = {0, 0};  // str_bits_kernel, str_pack_kernel
+    hb_host::DecLayout dec_layout[2];   // decode_batch_kernel<framed>
+    hb_host::StreamLayout stream_layout;
     // staging for the host entry points
     GrowBuf s_in, s_in_off, s_out, s_out_off, s_caps, s_status, s_consumed, s_ovf_pattern, s_ovf_bits, s_left_bits,
         s_left_num;
@@ -163,28 +158,36 @@ struct aws_huffman_batch_ctx {
         hp_left_num, hp_status;
     hb_host::BlockBufs blk;
     uint64_t *h_scalar = nullptr;  // pinned
-    // The *_device entry points enqueue on the caller's stream but share ctx->scratch (tile descriptors, ...).
-    // `scratch_free` is recorded after every such call; a call on ANOTHER stream waits for it first, so two calls
-    // in flight on different streams never touch the scratch at the same time.
+    // Calls enqueue on the caller's stream (device pointers) or on ctx->stream (host pointers) but share
+    // ctx->scratch, the staging and the HPACK buffers. `scratch_free` is recorded after every such call; a call on
+    // ANOTHER stream waits for it first, so two calls in flight on different streams never touch them at the same time.
     cudaEvent_t scratch_free = nullptr;
     cudaStream_t scratch_stream = nullptr;
     bool scratch_busy = false;
     // switches, read once at context creation (DESIGN.md 6b)
     bool force_generic = false, no_slots = false, no_strings = false, no_fused_stream = false;
-    size_t dec_static_smem[2] = {0, 0};
+
+    ~aws_huffman_batch_ctx() {
+        if (h_scalar) cudaFreeHost(h_scalar);
+        if (scratch_free) cudaEventDestroy(scratch_free);
+        if (stream) cudaStreamDestroy(stream);
+        if (d_enc) cudaFree(d_enc);
+        if (d_lut) cudaFree(d_lut);
+        if (d_lut2) cudaFree(d_lut2);
+    }
 };
 
 namespace {
 
-// Stream of a *_device call: the caller's, or the context's own; ordered behind the previous device call when
-// that one ran on a different stream (they share ctx->scratch).
-int device_call_begin(aws_huffman_batch_ctx *ctx, void *cuda_stream, cudaStream_t *st) {
+// Stream of a call on the context's shared buffers: the caller's, or the context's own (cuda_stream NULL, and every
+// host-pointer call); ordered behind the previous call when that one ran on a different stream.
+int call_begin(aws_huffman_batch_ctx *ctx, void *cuda_stream, cudaStream_t *st) {
     HB_CUDA_TRY(cudaSetDevice(ctx->device));
     *st = cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : ctx->stream;
     if (ctx->scratch_busy && ctx->scratch_stream != *st) HB_CUDA_TRY(cudaStreamWaitEvent(*st, ctx->scratch_free, 0));
     return AWS_OP_SUCCESS;
 }
-int device_call_end(aws_huffman_batch_ctx *ctx, cudaStream_t st, int rc) {
+int call_end(aws_huffman_batch_ctx *ctx, cudaStream_t st, int rc) {
     if (ctx->scratch_free && cudaEventRecord(ctx->scratch_free, st) == cudaSuccess) {
         ctx->scratch_stream = st;
         ctx->scratch_busy = true;
@@ -192,31 +195,6 @@ int device_call_end(aws_huffman_batch_ctx *ctx, cudaStream_t st, int rc) {
         (void)cudaGetLastError();
     }
     return rc;
-}
-
-// The dynamic shared-memory limit belongs to a kernel ON A DEVICE, not to a context; tables differ in size. It is
-// raised when a launch needs more than was ever asked for on that device (not on every call: the host path issues
-// one call per 8 MiB sub-batch).
-template <typename K>
-int ensure_dynamic_smem(K kernel, int device, size_t bytes) {
-    struct Seen {
-        const void *kernel;
-        size_t bytes[16];
-    };
-    static Seen seen[16] = {};  // (a handful of kernels ask; keyed by the kernel's address, then by device)
-    const void *key = reinterpret_cast<const void *>(kernel);
-    for (Seen &e : seen) {
-        if (e.kernel != key && e.kernel != nullptr) continue;
-        e.kernel = key;
-        size_t &cur = e.bytes[device & 15];
-        if (bytes > cur) {
-            HB_CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-            cur = bytes;
-        }
-        return AWS_OP_SUCCESS;
-    }
-    HB_CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-    return AWS_OP_SUCCESS;
 }
 
 #ifndef HB_LUT_ROOT_BITS
@@ -296,30 +274,16 @@ int encode_slots_on_device(
     a.ticket = reinterpret_cast<uint32_t *>(a.tile_state + num_tiles_ub);
     a.num_tiles_ub = (uint32_t)num_tiles_ub;
     a.eos_padding = ctx->tables.eos_padding;
-    if (!ctx->enc_slots_blocks_per_sm) {
-        int per_sm = 0;
-        HB_CUDA_TRY(cudaFuncSetAttribute(
-            encode_slots_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kEncSlotSmemBytes));
-        HB_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, encode_slots_kernel, kEncBlock, kEncSlotSmemBytes));
-        ctx->enc_slots_blocks_per_sm = std::max(1, per_sm);
-    }
     const unsigned grid = (unsigned)std::min<uint64_t>(num_tiles_ub, (uint64_t)ctx->sm_count * ctx->enc_slots_blocks_per_sm);
     encode_slots_kernel<<<grid, kEncBlock, kEncSlotSmemBytes, stream>>>(ctx->tables.enc, a);
     ++ctx->launches;
     HB_CUDA_TRY(cudaGetLastError());
-    if (v.out_lens || v.status || v.consumed || v.overflow_pattern || v.overflow_num_bits) {
-        fill_packed_meta_kernel<<<(unsigned)((v.n + 255) / 256), 256, 0, stream>>>(
-            v.n, v.in_offsets, v.out_offsets, v.out_lens, v.status, v.consumed, v.overflow_pattern,
-            v.overflow_num_bits);
-        ++ctx->launches;
-        HB_CUDA_TRY(cudaGetLastError());
-    }
     return AWS_OP_SUCCESS;
 }
 
 int encode_tiled_on_device(
     aws_huffman_batch_ctx *ctx, Scratch &sc, const hb::BatchView &v, uint64_t total_in, cudaStream_t stream,
-    const uint32_t *gate);
+    const uint32_t *gate = nullptr);
 
 // Packed layout, many short strings, every symbol has a code: one thread per string (encode_strings.cuh).
 int encode_strings_on_device(
@@ -368,14 +332,6 @@ int encode_strings_on_device(
     m.bits = p.bits;
     m.control = a.control;
     m.num_bits_tiles = (uint32_t)bits_tiles;
-    if (!ctx->str_blocks_per_sm[0]) {
-        int per_sm = 0;
-        HB_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, str_bits_kernel, kBitsThreads, 0));
-        ctx->str_blocks_per_sm[0] = std::max(1, per_sm);
-        HB_CUDA_TRY(cudaFuncSetAttribute(str_pack_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kStrPackSmemBytes));
-        HB_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, str_pack_kernel, kStrThreads, kStrPackSmemBytes));
-        ctx->str_blocks_per_sm[1] = std::max(1, per_sm);
-    }
     const unsigned grid_prep = (unsigned)std::min<uint64_t>((v.n + 256) / 256, (uint64_t)ctx->sm_count * 16);
     str_prep_kernel<<<grid_prep, 256, 0, stream>>>(p);
     const unsigned grid_b = (unsigned)std::min<uint64_t>(std::max<uint64_t>(1, bits_tiles), (uint64_t)ctx->sm_count * ctx->str_blocks_per_sm[0]);
@@ -387,21 +343,13 @@ int encode_strings_on_device(
     ctx->launches += 4;
     HB_CUDA_TRY(cudaGetLastError());
     // strings this path does not take (very long ones): the tiled kernel redoes the batch, on the device's own flag
-    if (encode_tiled_on_device(ctx, sc, v, total_in, stream, a.control + kStrCtlFallback)) return AWS_OP_ERR;
-    if (v.out_lens || v.status || v.consumed || v.overflow_pattern || v.overflow_num_bits) {
-        fill_packed_meta_kernel<<<(unsigned)((v.n + 255) / 256), 256, 0, stream>>>(
-            v.n, v.in_offsets, v.out_offsets, v.out_lens, v.status, v.consumed, v.overflow_pattern,
-            v.overflow_num_bits);
-        ++ctx->launches;
-        HB_CUDA_TRY(cudaGetLastError());
-    }
-    return AWS_OP_SUCCESS;
+    return encode_tiled_on_device(ctx, sc, v, total_in, stream, a.control + kStrCtlFallback);
 }
 
 // Packed layout, every symbol has a code: the tiled symbol-parallel kernel.
 int encode_tiled_on_device(
     aws_huffman_batch_ctx *ctx, Scratch &sc, const hb::BatchView &v, uint64_t total_in, cudaStream_t stream,
-    const uint32_t *gate = nullptr) {
+    const uint32_t *gate) {
     const uint64_t num_tiles = (total_in + kEncTile - 1) / kEncTile;
     const bool seg = v.n > 1;
     const size_t state_bytes = num_tiles * sizeof(uint64_t) + 256;
@@ -427,35 +375,12 @@ int encode_tiled_on_device(
             v.in_offsets, v.n, total_in, num_tiles, sc.tile_first.as<uint32_t>(), gate);
         ++ctx->launches;
     }
-    if (!ctx->enc_blocks_per_sm[seg]) {
-        int per_sm = 0;
-        if (seg) {
-            HB_CUDA_TRY(cudaFuncSetAttribute(
-                encode_tiled_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kEncSmemBytes));
-            HB_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(
-                &per_sm, encode_tiled_kernel<true>, kEncBlock, kEncSmemBytes));
-        } else {
-            HB_CUDA_TRY(cudaFuncSetAttribute(
-                encode_tiled_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kEncSmemBytes));
-            HB_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(
-                &per_sm, encode_tiled_kernel<false>, kEncBlock, kEncSmemBytes));
-        }
-        ctx->enc_blocks_per_sm[seg] = std::max(1, per_sm);
-    }
     const unsigned grid =
         (unsigned)std::min<uint64_t>(num_tiles, (uint64_t)ctx->sm_count * ctx->enc_blocks_per_sm[seg]);
     if (seg) encode_tiled_kernel<true><<<grid, kEncBlock, kEncSmemBytes, stream>>>(ctx->tables.enc, a);
     else encode_tiled_kernel<false><<<grid, kEncBlock, kEncSmemBytes, stream>>>(ctx->tables.enc, a);
     ++ctx->launches;
     HB_CUDA_TRY(cudaGetLastError());
-    if (gate) return AWS_OP_SUCCESS;  // (the caller fills the per-item arrays once)
-    if (v.out_lens || v.status || v.consumed || v.overflow_pattern || v.overflow_num_bits) {
-        fill_packed_meta_kernel<<<(unsigned)((v.n + 255) / 256), 256, 0, stream>>>(
-            v.n, v.in_offsets, v.out_offsets, v.out_lens, v.status, v.consumed, v.overflow_pattern,
-            v.overflow_num_bits);
-        ++ctx->launches;
-        HB_CUDA_TRY(cudaGetLastError());
-    }
     return AWS_OP_SUCCESS;
 }
 
@@ -466,15 +391,25 @@ int encode_on_device(
     // (the tiled kernel's multiply-add accumulator needs 1 << len to fit a word: codes of up to 31 bits)
     if (!v.resume && !v.out_caps && !ctx->tables.has_unknown && ctx->tables.max_len <= 31 && total_in > 0 && v.n < 0xffffffffull &&
         (total_in + kEncTile - 1) / kEncTile < 0xffffffffull && !force_generic) {
+        int rc;
         // many short strings: one thread per string
         if (v.n > 1 && total_in / v.n <= 2048 && (reinterpret_cast<uintptr_t>(v.in) & 15) == 0 &&
             (4 * total_in + v.n) / kStrTileBytes < 0xfffffff0ull && !ctx->no_strings)
-            return encode_strings_on_device(ctx, sc, v, total_in, stream);
+            rc = encode_strings_on_device(ctx, sc, v, total_in, stream);
         // many items of some length: thread ranges aligned to the items
-        if (v.n > 1 && total_in / v.n >= 24 && total_in < (1ull << 31) && (reinterpret_cast<uintptr_t>(v.in) & 15) == 0 &&
-            !ctx->no_slots)
-            return encode_slots_on_device(ctx, sc, v, total_in, stream);
-        return encode_tiled_on_device(ctx, sc, v, total_in, stream);
+        else if (v.n > 1 && total_in / v.n >= 24 && total_in < (1ull << 31) && (reinterpret_cast<uintptr_t>(v.in) & 15) == 0 &&
+                 !ctx->no_slots)
+            rc = encode_slots_on_device(ctx, sc, v, total_in, stream);
+        else
+            rc = encode_tiled_on_device(ctx, sc, v, total_in, stream);
+        if (rc) return AWS_OP_ERR;
+        if (v.out_lens || v.status || v.consumed || v.overflow_pattern || v.overflow_num_bits) {
+            fill_packed_meta_kernel<<<(unsigned)((v.n + 255) / 256), 256, 0, stream>>>(
+                v.n, v.in_offsets, v.out_offsets, v.out_lens, v.status, v.consumed, v.overflow_pattern, v.overflow_num_bits);
+            ++ctx->launches;
+            HB_CUDA_TRY(cudaGetLastError());
+        }
+        return AWS_OP_SUCCESS;
     }
     if (!v.out_lens) {
         HB_CUDA_TRY(sc.lens.reserve(v.n * sizeof(uint64_t)));
@@ -505,25 +440,9 @@ int decode_batch_fast(
     a.lut2_trap = ctx->lut2_trap;
     a.root_bits = ctx->tables.lut_root_bits;
     a.min_len = std::max<uint32_t>(1, ctx->tables.min_len);
-    // Shared memory of one block (two blocks per SM): [LUT][stage][rows]. A string of L bytes decodes to at
-    // most 8 L / min_len symbols, so the row area is that much larger than the stage; and the dense output
-    // image (which reuses the stage and the front of the rows) must end before row offset `front`
-    // (decode_batch_kernel step 4): rows <= stage + front - 32.
-    const size_t lut_bytes = (size_t)a.lut2_count * 8;
-    // one block per SM: [LUT2][team 0: stage, rows][team 1: stage, rows] + the teams' static arrays (what the kernel
-    // declares is asked from the runtime: every KB of the SM's 227 is a string more per tile)
-    if (!ctx->dec_static_smem[framed]) {
-        cudaFuncAttributes attr{};
-        HB_CUDA_TRY(framed ? cudaFuncGetAttributes(&attr, decode_batch_kernel<true>) : cudaFuncGetAttributes(&attr, decode_batch_kernel<false>));
-        ctx->dec_static_smem[framed] = attr.sharedSizeBytes;
-    }
-    const size_t budget = (((size_t)227 * 1024 - ctx->dec_static_smem[framed] - lut_bytes) / kDecTeams - 128) & ~size_t(15);
+    const hb_host::DecLayout &L = ctx->dec_layout[framed];
+    const size_t stage_bytes = L.stage_bytes, rows_bytes = L.rows_bytes;
     const double expand = 8.0 / a.min_len;
-    size_t stage_bytes = (size_t)((double)budget / (1.0 + expand)) & ~size_t(15);
-    stage_bytes = std::max<size_t>(stage_bytes, 2 * kDecMaxRow);
-    size_t rows_bytes = budget - stage_bytes;
-    const size_t front = (stage_bytes - kDecMaxRow - 32) & ~size_t(3);
-    rows_bytes = std::min(rows_bytes, stage_bytes + front - 64) & ~size_t(15);
     a.stage_words = (uint32_t)(stage_bytes / 4 - 2);
     a.rows_bytes = (uint32_t)rows_bytes;
     // strings per tile: as many as fit the stage and the row area at the batch's average length, with room to spare
@@ -547,13 +466,9 @@ int decode_batch_fast(
     a.tile_state = sc.tile_state.as<uint64_t>();
     a.ticket = reinterpret_cast<uint32_t *>(a.tile_state + num_tiles);
     a.num_tiles = (uint32_t)num_tiles;
-    const size_t team_bytes = ((stage_bytes + 15) & ~size_t(15)) + rows_bytes + 64;
-    const size_t smem = lut_bytes + kDecTeams * team_bytes;
-    if (framed ? ensure_dynamic_smem(decode_batch_kernel<true>, ctx->device, smem) : ensure_dynamic_smem(decode_batch_kernel<false>, ctx->device, smem))
-        return AWS_OP_ERR;
     const unsigned blocks = (unsigned)std::min<uint64_t>((num_tiles + kDecTeams - 1) / kDecTeams, (uint64_t)ctx->sm_count);
-    if (framed) decode_batch_kernel<true><<<blocks, kDecTeams * kDecBlock, smem, stream>>>(a);
-    else decode_batch_kernel<false><<<blocks, kDecTeams * kDecBlock, smem, stream>>>(a);
+    if (framed) decode_batch_kernel<true><<<blocks, kDecTeams * kDecBlock, L.smem, stream>>>(a);
+    else decode_batch_kernel<false><<<blocks, kDecTeams * kDecBlock, L.smem, stream>>>(a);
     ++ctx->launches;
     HB_CUDA_TRY(cudaGetLastError());
     return AWS_OP_SUCCESS;
@@ -582,26 +497,16 @@ int decode_stream_fast(
     a.lut = ctx->tables.lut;
     a.lut_count = ctx->tables.lut_count;
     a.root_bits = ctx->tables.lut_root_bits;
-    const size_t smem = ctx->tables.lut_count * sizeof(uint32_t);
-    const size_t smem_staged = smem + kStreamStageWords * sizeof(uint32_t);
+    const hb_host::StreamLayout &L = ctx->stream_layout;
 
     // ---- fused single pass ------------------------------------------------------------------------------------
-    const uint32_t min_len = std::max<uint32_t>(1, ctx->tables.min_len);
-    const uint32_t row_words = (((kChunkBits + 31) / min_len + 4 + 3) / 4) | 1u;
-    const size_t lut_bytes = (size_t)ctx->lut2_count * 8;
-    const size_t stage_bytes = (kStreamStageWords * 4 + 15) & ~size_t(15);
-    const size_t team_bytes = (stage_bytes + (size_t)kStreamThreads * row_words * 4 + 16 + 15) & ~size_t(15);
-    const size_t fused_smem = lut_bytes + kStreamTeams * team_bytes;  // one block per SM, two teams, one table
-    // (the dense output image reuses the stage and the front of the rows: stream_fused_kernel step 5)
-    const bool fused = (size_t)kStreamThreads * row_words * 4 + 16 <= 2 * stage_bytes - row_words * 4 - 32 &&
-                       fused_smem <= 220 * 1024 && !ctx->no_fused_stream;
-    if (fused) {
+    if (L.fused) {
         StreamFusedArgs f{};
         f.s = a;
         f.s.num_chunks = std::max<uint64_t>(1, (end_bit > 31 ? end_bit - 31 + kChunkBits - 1 : 0) / kChunkBits);
         f.b = v;
         f.num_tiles = (uint32_t)((f.s.num_chunks + kStreamThreads - 1) / kStreamThreads);
-        f.row_words = row_words;
+        f.row_words = L.row_words;
         f.lut2 = ctx->d_lut2;
         f.lut2_count = ctx->lut2_count;
         f.lut2_trap = ctx->lut2_trap;
@@ -614,9 +519,8 @@ int decode_stream_fast(
         f.ticket = reinterpret_cast<uint32_t *>(f.tile_rec + f.num_tiles);
         f.fail = f.ticket + 2;
         a.gate = f.fail;
-        if (ensure_dynamic_smem(stream_fused_kernel, ctx->device, fused_smem)) return AWS_OP_ERR;
         const unsigned blocks = (unsigned)std::min<uint64_t>((f.num_tiles + kStreamTeams - 1) / kStreamTeams, (uint64_t)ctx->sm_count);
-        stream_fused_kernel<<<blocks, kStreamTeams * kStreamTeamThreads, fused_smem, stream>>>(f);
+        stream_fused_kernel<<<blocks, kStreamTeams * kStreamTeamThreads, L.fused_smem, stream>>>(f);
         stream_fused_verify_kernel<<<(unsigned)std::min<uint64_t>((f.num_tiles + 255) / 256, 1024), 256, 0, stream>>>(f);
         ctx->launches += 2;
         HB_CUDA_TRY(cudaGetLastError());
@@ -624,22 +528,20 @@ int decode_stream_fast(
 
     // ---- multi-kernel path (alone, or gated behind the fused kernel's fail flag) ----------------------------------
     HB_CUDA_TRY(cudaMemsetAsync(a.control, 0xff, 2 * sizeof(uint64_t), stream));
-    if (ensure_dynamic_smem(stream_sync_kernel, ctx->device, smem_staged) || ensure_dynamic_smem(stream_write_kernel, ctx->device, smem_staged))
-        return AWS_OP_ERR;
     // a gated launch that finds the flag clear costs a few microseconds: keep those grids small
-    const uint64_t cap_wide = fused ? (uint64_t)ctx->sm_count * 4 : (uint64_t)ctx->sm_count * 12;
-    const uint64_t cap_flat = fused ? (uint64_t)ctx->sm_count * 4 : (uint64_t)ctx->sm_count * 8;
+    const uint64_t cap_wide = L.fused ? (uint64_t)ctx->sm_count * 4 : (uint64_t)ctx->sm_count * 12;
+    const uint64_t cap_flat = L.fused ? (uint64_t)ctx->sm_count * 4 : (uint64_t)ctx->sm_count * 8;
     const unsigned wide = (unsigned)std::min<uint64_t>((num_chunks + kStreamThreads - 1) / kStreamThreads, cap_wide);
     const unsigned flat = (unsigned)std::min<uint64_t>((num_chunks + 255) / 256, cap_flat);
-    stream_sync_kernel<<<wide, kStreamThreads, smem_staged, stream>>>(a);
-    for (int round = 0; round < 2; ++round) stream_fix_kernel<<<wide, kStreamThreads, smem, stream>>>(a);
+    stream_sync_kernel<<<wide, kStreamThreads, L.smem_staged, stream>>>(a);
+    for (int round = 0; round < 2; ++round) stream_fix_kernel<<<wide, kStreamThreads, L.smem, stream>>>(a);
     stream_verify_kernel<<<flat, 256, 0, stream>>>(a);
-    stream_repair_kernel<<<1, 32, smem, stream>>>(a);
+    stream_repair_kernel<<<1, 32, L.smem, stream>>>(a);
     stream_counts_kernel<<<flat, 256, 0, stream>>>(a, sc.chunk_lens.as<uint64_t>());
     ctx->launches += 6;
     HB_CUDA_TRY(cudaGetLastError());
     if (launch_scan(ctx, sc, sc.chunk_lens.as<uint64_t>(), a.chunk_offsets, num_chunks, stream, a.gate)) return AWS_OP_ERR;
-    stream_write_kernel<<<wide, kStreamThreads, smem_staged, stream>>>(a, v);
+    stream_write_kernel<<<wide, kStreamThreads, L.smem_staged, stream>>>(a, v);
     ++ctx->launches;
     HB_CUDA_TRY(cudaGetLastError());
     return AWS_OP_SUCCESS;
@@ -725,12 +627,38 @@ int copy_item_arrays_to_host(const aws_huffman_batch *b, const hb::BatchView &v,
     return AWS_OP_SUCCESS;
 }
 
+// Host-pointer staging: grows `buf` to `room` bytes, uploads `count` elements of `src` to it on `st` and sets `*dev`
+// to the device copy (count 0: only the room, for an array the call writes).
+template <typename T, typename D>
+int stage_in(GrowBuf &buf, size_t room, const T *src, size_t count, cudaStream_t st, D **dev) {
+    HB_CUDA_TRY(buf.reserve(room));
+    if (count) HB_CUDA_TRY(cudaMemcpyAsync(buf.ptr, src, count * sizeof(T), cudaMemcpyHostToDevice, st));
+    *dev = static_cast<D *>(buf.ptr);
+    return AWS_OP_SUCCESS;
+}
+
+// The end of a host-pointer call with a packed result: offsets[0..count] (and status[0..count) when the caller asked
+// for it) come down; then AWS_ERROR_SHORT_BUFFER when offsets[count] > capacity, else the payload of offsets[count]
+// bytes is enqueued (d_out == NULL: there is none). The caller synchronises `st` after its last copy.
+int finish_packed(cudaStream_t st, size_t count, const uint64_t *d_offsets, uint64_t *offsets, const void *d_out,
+                  void *out, uint64_t capacity, const int32_t *d_status = nullptr, int32_t *status = nullptr) {
+    HB_CUDA_TRY(cudaMemcpyAsync(offsets, d_offsets, (count + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    if (status && d_status) HB_CUDA_TRY(cudaMemcpyAsync(status, d_status, count * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    HB_CUDA_TRY(cudaStreamSynchronize(st));
+    const uint64_t total = offsets[count];
+    if (total > capacity) return aws_raise_error(AWS_ERROR_SHORT_BUFFER);
+    if (d_out && total) HB_CUDA_TRY(cudaMemcpyAsync(out, d_out, total, cudaMemcpyDeviceToHost, st));
+    return AWS_OP_SUCCESS;
+}
+
 // Packed layout with many items: the batch is cut into sub-batches (contiguous item ranges balanced by
 // bytes) that flow through kLanes lanes, so the host->device copy of one sub-batch, the kernels of the
 // next and the device->host copy of the previous one run at the same time. Sub-batches are ordinary
 // independent batches on the device; their packed offsets are rebased on the host at the end
-// (the same concatenation step as multi-GPU sharding).
+// (the same concatenation step as multi-GPU sharding). Only the lanes' own buffers are used, none of the
+// context's shared ones, so this path needs no call_begin / call_end.
 int run_host_batch_pipelined(aws_huffman_batch_ctx *ctx, const aws_huffman_batch *b, bool encode) {
+    HB_CUDA_TRY(cudaSetDevice(ctx->device));
     const size_t n = b->n;
     const uint64_t total_in = b->in_offsets[n];
     size_t shards = (size_t)std::min<uint64_t>(256, std::max<uint64_t>(2, total_in / kPipelineShardBytes));
@@ -854,7 +782,6 @@ int run_host_batch_pipelined(aws_huffman_batch_ctx *ctx, const aws_huffman_batch
     return AWS_OP_SUCCESS;
 }
 
-// Host-pointer entry point shared by encode and decode: stage in, run, stage out.
 int check_resume(const aws_huffman_batch *b, bool encode) {
     // the state arrays are inputs as well as outputs
     if (b && b->n &&
@@ -863,6 +790,53 @@ int check_resume(const aws_huffman_batch *b, bool encode) {
     return AWS_OP_SUCCESS;
 }
 
+// One host-pointer call through the context's staging: stage in, run, stage out.
+int run_host_batch_staged(aws_huffman_batch_ctx *ctx, const aws_huffman_batch *b, bool encode, bool resume, cudaStream_t st) {
+    const size_t n = b->n;
+    const uint64_t total_in = b->in_offsets[n];
+    const bool slotted = b->out_caps != nullptr;
+    const size_t up = resume ? n : 0;  // (the resume state goes up; otherwise those arrays are outputs only)
+    hb::BatchView v{};
+    v.resume = resume;
+    v.n = n;
+    v.out_capacity = b->out_capacity;
+    // (slotted: bytes the codec does not touch must come back unchanged, so the output goes up too)
+    if (stage_in(ctx->s_in, total_in + 16, b->in, total_in, st, &v.in) ||
+        stage_in(ctx->s_in_off, (n + 1) * sizeof(uint64_t), b->in_offsets, n + 1, st, &v.in_offsets) ||
+        stage_in(ctx->s_out, b->out_capacity + 16, b->out, slotted ? b->out_capacity : 0, st, &v.out) ||
+        stage_in(ctx->s_out_off, (n + 1) * sizeof(uint64_t), b->out_offsets, slotted ? n : 0, st, &v.out_offsets) ||
+        (slotted && stage_in(ctx->s_caps, n * sizeof(uint64_t), b->out_caps, n, st, &v.out_caps)) ||
+        (b->status && stage_in(ctx->s_status, n * sizeof(int32_t), b->status, 0, st, &v.status)) ||
+        (b->consumed && stage_in(ctx->s_consumed, n * sizeof(uint64_t), b->consumed, 0, st, &v.consumed)))
+        return AWS_OP_ERR;
+    if (encode) {
+        if ((b->overflow_pattern &&
+             stage_in(ctx->s_ovf_pattern, n * sizeof(uint32_t), b->overflow_pattern, up, st, &v.overflow_pattern)) ||
+            (b->overflow_num_bits && stage_in(ctx->s_ovf_bits, n, b->overflow_num_bits, up, st, &v.overflow_num_bits)))
+            return AWS_OP_ERR;
+    } else if ((b->leftover_working_bits && stage_in(ctx->s_left_bits, n * sizeof(uint64_t), b->leftover_working_bits, up,
+                                                     st, &v.leftover_working_bits)) ||
+               (b->leftover_num_bits && stage_in(ctx->s_left_num, n, b->leftover_num_bits, up, st, &v.leftover_num_bits))) {
+        return AWS_OP_ERR;
+    }
+    HB_CUDA_TRY(ctx->scratch.lens.reserve(n * sizeof(uint64_t)));
+    v.out_lens = b->out_lens ? ctx->scratch.lens.as<uint64_t>() : nullptr;
+
+    if ((encode ? encode_on_device(ctx, ctx->scratch, v, total_in, st)
+                : decode_on_device(ctx, ctx->scratch, v, total_in, st)) != AWS_OP_SUCCESS)
+        return AWS_OP_ERR;
+
+    if (copy_item_arrays_to_host(b, v, 0, n, st)) return AWS_OP_ERR;
+    if (slotted) {
+        if (b->out_capacity) HB_CUDA_TRY(cudaMemcpyAsync(b->out, v.out, b->out_capacity, cudaMemcpyDeviceToHost, st));
+    } else if (finish_packed(st, n, v.out_offsets, b->out_offsets, v.out, b->out, b->out_capacity)) {
+        return AWS_OP_ERR;
+    }
+    HB_CUDA_TRY(cudaStreamSynchronize(st));
+    return AWS_OP_SUCCESS;
+}
+
+// Host-pointer entry point shared by encode and decode.
 int run_host_batch(aws_huffman_batch_ctx *ctx, const aws_huffman_batch *b, bool encode, bool resume = false) {
     if (!ctx) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
     if (check_batch(b)) return AWS_OP_ERR;
@@ -872,92 +846,26 @@ int run_host_batch(aws_huffman_batch_ctx *ctx, const aws_huffman_batch *b, bool 
         if (!b->out_caps && b->out_offsets) b->out_offsets[0] = 0;
         return AWS_OP_SUCCESS;
     }
-    HB_CUDA_TRY(cudaSetDevice(ctx->device));
-    cudaStream_t st = ctx->stream;
     const uint64_t total_in = b->in_offsets[n];
-    const bool slotted = b->out_caps != nullptr;
     if ((total_in && !b->in) || (b->out_capacity && !b->out)) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
     // (payloads are always staged through device memory, pinned caller buffers too: kernels that read and write pinned
     // host memory over PCIe measured slower end to end than the copy engines, DESIGN.md 6)
-    if (!resume && !slotted && n >= 2 && total_in >= kPipelineMinBytes) return run_host_batch_pipelined(ctx, b, encode);
+    if (!resume && !b->out_caps && n >= 2 && total_in >= kPipelineMinBytes) return run_host_batch_pipelined(ctx, b, encode);
+    cudaStream_t st;
+    if (call_begin(ctx, nullptr, &st)) return AWS_OP_ERR;
+    return call_end(ctx, st, run_host_batch_staged(ctx, b, encode, resume, st));
+}
 
-    HB_CUDA_TRY(ctx->s_in.reserve(total_in + 16));
-    HB_CUDA_TRY(ctx->s_in_off.reserve((n + 1) * sizeof(uint64_t)));
-    HB_CUDA_TRY(ctx->s_out.reserve(b->out_capacity + 16));
-    HB_CUDA_TRY(ctx->s_out_off.reserve((n + 1) * sizeof(uint64_t)));
-    HB_CUDA_TRY(ctx->scratch.lens.reserve(n * sizeof(uint64_t)));
-    if (slotted) HB_CUDA_TRY(ctx->s_caps.reserve(n * sizeof(uint64_t)));
-    if (b->status) HB_CUDA_TRY(ctx->s_status.reserve(n * sizeof(int32_t)));
-    if (b->consumed) HB_CUDA_TRY(ctx->s_consumed.reserve(n * sizeof(uint64_t)));
-    if (encode && b->overflow_pattern) HB_CUDA_TRY(ctx->s_ovf_pattern.reserve(n * sizeof(uint32_t)));
-    if (encode && b->overflow_num_bits) HB_CUDA_TRY(ctx->s_ovf_bits.reserve(n));
-    if (!encode && b->leftover_working_bits) HB_CUDA_TRY(ctx->s_left_bits.reserve(n * sizeof(uint64_t)));
-    if (!encode && b->leftover_num_bits) HB_CUDA_TRY(ctx->s_left_num.reserve(n));
-
-    if (total_in) HB_CUDA_TRY(cudaMemcpyAsync(ctx->s_in.ptr, b->in, total_in, cudaMemcpyHostToDevice, st));
-    HB_CUDA_TRY(cudaMemcpyAsync(ctx->s_in_off.ptr, b->in_offsets, (n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
-    if (slotted) {
-        HB_CUDA_TRY(cudaMemcpyAsync(ctx->s_out_off.ptr, b->out_offsets, n * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
-        HB_CUDA_TRY(cudaMemcpyAsync(ctx->s_caps.ptr, b->out_caps, n * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
-        // bytes the codec does not touch must come back unchanged
-        if (b->out_capacity)
-            HB_CUDA_TRY(cudaMemcpyAsync(ctx->s_out.ptr, b->out, b->out_capacity, cudaMemcpyHostToDevice, st));
-    }
-
-    if (resume) {
-        if (encode) {
-            HB_CUDA_TRY(cudaMemcpyAsync(ctx->s_ovf_pattern.ptr, b->overflow_pattern, n * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
-            HB_CUDA_TRY(cudaMemcpyAsync(ctx->s_ovf_bits.ptr, b->overflow_num_bits, n, cudaMemcpyHostToDevice, st));
-        } else {
-            HB_CUDA_TRY(cudaMemcpyAsync(ctx->s_left_bits.ptr, b->leftover_working_bits, n * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
-            HB_CUDA_TRY(cudaMemcpyAsync(ctx->s_left_num.ptr, b->leftover_num_bits, n, cudaMemcpyHostToDevice, st));
-        }
-    }
-
-    hb::BatchView v{};
+// Device-pointer entry point shared by encode and decode.
+int run_device_batch(aws_huffman_batch_ctx *ctx, const aws_huffman_batch *b, void *cuda_stream, bool encode, bool resume) {
+    if (!ctx) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    if (check_batch(b) || (resume && check_resume(b, encode))) return AWS_OP_ERR;
+    cudaStream_t st;
+    if (call_begin(ctx, cuda_stream, &st)) return AWS_OP_ERR;
+    hb::BatchView v = make_view(b);
     v.resume = resume;
-    v.n = n;
-    v.in = ctx->s_in.as<uint8_t>();
-    v.in_offsets = ctx->s_in_off.as<uint64_t>();
-    v.out = ctx->s_out.as<uint8_t>();
-    v.out_capacity = b->out_capacity;
-    v.out_offsets = ctx->s_out_off.as<uint64_t>();
-    v.out_caps = slotted ? ctx->s_caps.as<uint64_t>() : nullptr;
-    v.out_lens = ctx->scratch.lens.as<uint64_t>();
-    v.status = b->status ? ctx->s_status.as<int32_t>() : nullptr;
-    v.consumed = b->consumed ? ctx->s_consumed.as<uint64_t>() : nullptr;
-    if (encode) {
-        v.overflow_pattern = b->overflow_pattern ? ctx->s_ovf_pattern.as<uint32_t>() : nullptr;
-        v.overflow_num_bits = b->overflow_num_bits ? ctx->s_ovf_bits.as<uint8_t>() : nullptr;
-    } else {
-        v.leftover_working_bits = b->leftover_working_bits ? ctx->s_left_bits.as<uint64_t>() : nullptr;
-        v.leftover_num_bits = b->leftover_num_bits ? ctx->s_left_num.as<uint8_t>() : nullptr;
-    }
-
-    v.out_lens = b->out_lens ? ctx->scratch.lens.as<uint64_t>() : nullptr;
-    if ((encode ? encode_on_device(ctx, ctx->scratch, v, total_in, st)
-                : decode_on_device(ctx, ctx->scratch, v, total_in, st)) != AWS_OP_SUCCESS)
-        return AWS_OP_ERR;
-
-    if (copy_item_arrays_to_host(b, v, 0, n, st)) return AWS_OP_ERR;
-
-    if (slotted) {
-        if (b->out_capacity)
-            HB_CUDA_TRY(cudaMemcpyAsync(b->out, v.out, b->out_capacity, cudaMemcpyDeviceToHost, st));
-        HB_CUDA_TRY(cudaStreamSynchronize(st));
-        return AWS_OP_SUCCESS;
-    }
-
-    HB_CUDA_TRY(
-        cudaMemcpyAsync(b->out_offsets, v.out_offsets, (n + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-    HB_CUDA_TRY(cudaStreamSynchronize(st));
-    const uint64_t total_out = b->out_offsets[n];
-    if (total_out > b->out_capacity) return aws_raise_error(AWS_ERROR_SHORT_BUFFER);
-    if (total_out) {
-        HB_CUDA_TRY(cudaMemcpyAsync(b->out, v.out, total_out, cudaMemcpyDeviceToHost, st));
-        HB_CUDA_TRY(cudaStreamSynchronize(st));
-    }
-    return AWS_OP_SUCCESS;
+    return call_end(ctx, st, encode ? encode_on_device(ctx, ctx->scratch, v, b->in_size, st)
+                                    : decode_on_device(ctx, ctx->scratch, v, b->in_size, st));
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1002,7 +910,8 @@ int hpack_decode_on_device(
     if (n == 0) return AWS_OP_SUCCESS;
     // (the one-kernel route copies raw literals into rows sized 8 len / min_len: a table whose shortest code is longer
     // than a byte — not HPACK's — takes the multi-pass route)
-    if (n > 1 && ctx->tables.lut_count <= kDecLutMaxSmem && ctx->tables.min_len <= 8 && !getenv("AWS_HUFFMAN_BATCH_FORCE_GENERIC") &&
+    // (AWS_HUFFMAN_HPACK_PASSES is read per call, DESIGN.md 6b)
+    if (n > 1 && ctx->tables.lut_count <= kDecLutMaxSmem && ctx->tables.min_len <= 8 && !ctx->force_generic &&
         !getenv("AWS_HUFFMAN_HPACK_PASSES")) {
         // one kernel: the batch decoder parses the literals in its string table, copies raw payloads, applies
         // the padding rule to what it leaves over and writes strings, offsets and status itself
@@ -1082,6 +991,30 @@ int hpack_decode_on_device(
 }
 
 // Host pointers: stage in, run, stage out.
+int hpack_run_staged(
+    aws_huffman_batch_ctx *ctx, bool encode, size_t n, const uint8_t *in, const uint64_t *in_off, uint32_t mode, uint8_t *out,
+    uint64_t out_capacity, uint64_t *out_off, int32_t *status, cudaStream_t st) {
+    const uint64_t total_in = in_off[n];
+    const uint8_t *d_in = nullptr;
+    const uint64_t *d_in_off = nullptr;
+    if (stage_in(ctx->s_in, total_in + 16, in, total_in, st, &d_in) ||
+        stage_in(ctx->s_in_off, (n + 1) * sizeof(uint64_t), in_off, n + 1, st, &d_in_off))
+        return AWS_OP_ERR;
+    HB_CUDA_TRY(ctx->s_out.reserve(out_capacity + 16));
+    HB_CUDA_TRY(ctx->s_out_off.reserve((n + 1) * sizeof(uint64_t)));
+    HB_CUDA_TRY(ctx->s_status.reserve(n * sizeof(int32_t)));
+    uint8_t *d_out = ctx->s_out.as<uint8_t>();
+    uint64_t *d_out_off = ctx->s_out_off.as<uint64_t>();
+    int32_t *d_status = ctx->s_status.as<int32_t>();
+    if (encode ? hpack_encode_on_device(ctx, n, d_in, d_in_off, total_in, mode, d_out, out_capacity, d_out_off, st)
+               : hpack_decode_on_device(ctx, n, d_in, d_in_off, total_in, d_out, out_capacity, d_out_off, d_status, st))
+        return AWS_OP_ERR;
+    if (finish_packed(st, n, d_out_off, out_off, d_out, out, out_capacity, encode ? nullptr : d_status, status))
+        return AWS_OP_ERR;
+    HB_CUDA_TRY(cudaStreamSynchronize(st));
+    return AWS_OP_SUCCESS;
+}
+
 int hpack_run_host(
     aws_huffman_batch_ctx *ctx, bool encode, size_t n, const uint8_t *in, const uint64_t *in_off, uint32_t mode, uint8_t *out,
     uint64_t out_capacity, uint64_t *out_off, int32_t *status) {
@@ -1090,33 +1023,10 @@ int hpack_run_host(
         if (out_off) out_off[0] = 0;
         return AWS_OP_SUCCESS;
     }
-    const uint64_t total_in = in_off[n];
-    if ((total_in && !in) || (out_capacity && !out)) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
-    HB_CUDA_TRY(cudaSetDevice(ctx->device));
-    cudaStream_t st = ctx->stream;
-    HB_CUDA_TRY(ctx->s_in.reserve(total_in + 16));
-    HB_CUDA_TRY(ctx->s_in_off.reserve((n + 1) * sizeof(uint64_t)));
-    HB_CUDA_TRY(ctx->s_out.reserve(out_capacity + 16));
-    HB_CUDA_TRY(ctx->s_out_off.reserve((n + 1) * sizeof(uint64_t)));
-    HB_CUDA_TRY(ctx->s_status.reserve(n * sizeof(int32_t)));
-    if (total_in) HB_CUDA_TRY(cudaMemcpyAsync(ctx->s_in.ptr, in, total_in, cudaMemcpyHostToDevice, st));
-    HB_CUDA_TRY(cudaMemcpyAsync(ctx->s_in_off.ptr, in_off, (n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
-    const int rc = encode ? hpack_encode_on_device(ctx, n, ctx->s_in.as<uint8_t>(), ctx->s_in_off.as<uint64_t>(), total_in, mode,
-                                                   ctx->s_out.as<uint8_t>(), out_capacity, ctx->s_out_off.as<uint64_t>(), st)
-                          : hpack_decode_on_device(ctx, n, ctx->s_in.as<uint8_t>(), ctx->s_in_off.as<uint64_t>(), total_in,
-                                                   ctx->s_out.as<uint8_t>(), out_capacity, ctx->s_out_off.as<uint64_t>(),
-                                                   ctx->s_status.as<int32_t>(), st);
-    if (rc) return AWS_OP_ERR;
-    HB_CUDA_TRY(cudaMemcpyAsync(out_off, ctx->s_out_off.ptr, (n + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-    if (!encode && status) HB_CUDA_TRY(cudaMemcpyAsync(status, ctx->s_status.ptr, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    HB_CUDA_TRY(cudaStreamSynchronize(st));
-    const uint64_t total_out = out_off[n];
-    if (total_out > out_capacity) return aws_raise_error(AWS_ERROR_SHORT_BUFFER);
-    if (total_out) {
-        HB_CUDA_TRY(cudaMemcpyAsync(out, ctx->s_out.ptr, total_out, cudaMemcpyDeviceToHost, st));
-        HB_CUDA_TRY(cudaStreamSynchronize(st));
-    }
-    return AWS_OP_SUCCESS;
+    if ((in_off[n] && !in) || (out_capacity && !out)) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    cudaStream_t st;
+    if (call_begin(ctx, nullptr, &st)) return AWS_OP_ERR;
+    return call_end(ctx, st, hpack_run_staged(ctx, encode, n, in, in_off, mode, out, out_capacity, out_off, status, st));
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1320,6 +1230,36 @@ BlockLists block_lists(const aws_hpack_header_lists *l) {
 }
 
 // Host pointers: stage in, run, stage out (the way hpack_run_host does).
+int hpack_blocks_decode_staged(
+    aws_huffman_batch_ctx *ctx, size_t n, const uint8_t *in, const uint64_t *in_off, aws_hpack_header_lists *out,
+    int32_t *status, cudaStream_t st) {
+    hb_host::BlockBufs &B = ctx->blk;
+    const uint64_t total_in = in_off[n];
+    const uint8_t *d_in = nullptr;
+    const uint64_t *d_in_off = nullptr;
+    BlockLists o = block_lists(out);
+    if (stage_in(ctx->s_in, total_in + 16, in, total_in, st, &d_in) ||
+        stage_in(ctx->s_in_off, (n + 1) * sizeof(uint64_t), in_off, n + 1, st, &d_in_off) ||
+        stage_in(B.s_field_offsets, (n + 1) * sizeof(uint64_t), out->field_offsets, 0, st, &o.field_offsets))
+        return AWS_OP_ERR;
+    HB_CUDA_TRY(ctx->s_status.reserve(n * sizeof(int32_t)));
+    if (hpack_blocks_decode_on_device(ctx, n, d_in, d_in_off, o, ctx->s_status.as<int32_t>(), true, st)) return AWS_OP_ERR;
+    // field records (no payload of their own here), then the strings behind them
+    if (finish_packed(st, n, o.field_offsets, out->field_offsets, nullptr, nullptr, out->field_capacity,
+                      ctx->s_status.as<int32_t>(), status))
+        return AWS_OP_ERR;
+    const uint64_t fields = out->field_offsets[n];
+    if (finish_packed(st, 2 * fields, B.s_string_offsets.as<uint64_t>(), out->string_offsets, ctx->s_out.ptr, out->strings,
+                      out->strings_capacity))
+        return AWS_OP_ERR;
+    if (fields) {
+        HB_CUDA_TRY(cudaMemcpyAsync(out->field_kind, B.s_kind.ptr, fields, cudaMemcpyDeviceToHost, st));
+        HB_CUDA_TRY(cudaMemcpyAsync(out->field_index, B.s_index.ptr, fields * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    }
+    HB_CUDA_TRY(cudaStreamSynchronize(st));
+    return AWS_OP_SUCCESS;
+}
+
 int hpack_blocks_decode_host(
     aws_huffman_batch_ctx *ctx, size_t n, const uint8_t *in, const uint64_t *in_off, aws_hpack_header_lists *out,
     int32_t *status) {
@@ -1329,42 +1269,40 @@ int hpack_blocks_decode_host(
         out->string_offsets[0] = 0;
         return AWS_OP_SUCCESS;
     }
-    const uint64_t total_in = in_off[n];
-    if ((total_in && !in) || !offsets_sorted(in_off, n + 1)) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
-    HB_CUDA_TRY(cudaSetDevice(ctx->device));
-    cudaStream_t st = ctx->stream;
+    if ((in_off[n] && !in) || !offsets_sorted(in_off, n + 1)) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    cudaStream_t st;
+    if (call_begin(ctx, nullptr, &st)) return AWS_OP_ERR;
+    return call_end(ctx, st, hpack_blocks_decode_staged(ctx, n, in, in_off, out, status, st));
+}
+
+// records: field_kind and field_index are read (aws_hpack_header_block_encode_records_batch), status is optional.
+int hpack_blocks_encode_staged(
+    aws_huffman_batch_ctx *ctx, const aws_hpack_header_lists *in, bool records, uint32_t mode, uint8_t *out,
+    uint64_t out_capacity, uint64_t *out_off, int32_t *status, cudaStream_t st) {
     hb_host::BlockBufs &B = ctx->blk;
-    HB_CUDA_TRY(ctx->s_in.reserve(total_in + 16));
-    HB_CUDA_TRY(ctx->s_in_off.reserve((n + 1) * sizeof(uint64_t)));
-    HB_CUDA_TRY(ctx->s_status.reserve(n * sizeof(int32_t)));
-    HB_CUDA_TRY(B.s_field_offsets.reserve((n + 1) * sizeof(uint64_t)));
-    if (total_in) HB_CUDA_TRY(cudaMemcpyAsync(ctx->s_in.ptr, in, total_in, cudaMemcpyHostToDevice, st));
-    HB_CUDA_TRY(cudaMemcpyAsync(ctx->s_in_off.ptr, in_off, (n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
-    BlockLists o = block_lists(out);
-    o.field_offsets = B.s_field_offsets.as<uint64_t>();
-    if (hpack_blocks_decode_on_device(ctx, n, ctx->s_in.as<uint8_t>(), ctx->s_in_off.as<uint64_t>(), o,
-                                      ctx->s_status.as<int32_t>(), true, st))
+    const uint64_t n = in->n, F = in->field_offsets[n], S = in->string_offsets[2 * F];
+    const uint64_t *d_field_offsets = nullptr, *d_string_offsets = nullptr;
+    const uint8_t *d_strings = nullptr, *never = nullptr, *kind = nullptr;
+    const uint64_t *index = nullptr;
+    int32_t *d_status = nullptr;
+    if (stage_in(B.s_field_offsets, (n + 1) * sizeof(uint64_t), in->field_offsets, n + 1, st, &d_field_offsets) ||
+        stage_in(ctx->s_in, S + 16, in->strings, S, st, &d_strings) ||
+        stage_in(ctx->s_in_off, (2 * F + 1) * sizeof(uint64_t), in->string_offsets, 2 * F + 1, st, &d_string_offsets) ||
+        (in->never_indexed && F && stage_in(B.s_never, F, in->never_indexed, F, st, &never)) ||
+        (records && (stage_in(B.s_kind, F + 1, in->field_kind, F, st, &kind) ||
+                     stage_in(B.s_index, (F + 1) * sizeof(uint64_t), in->field_index, F, st, &index) ||
+                     stage_in(ctx->s_status, n * sizeof(int32_t), status, 0, st, &d_status))))
         return AWS_OP_ERR;
-    HB_CUDA_TRY(cudaMemcpyAsync(out->field_offsets, o.field_offsets, (n + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-    if (status) HB_CUDA_TRY(cudaMemcpyAsync(status, ctx->s_status.ptr, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    HB_CUDA_TRY(cudaStreamSynchronize(st));
-    const uint64_t fields = out->field_offsets[n];
-    if (fields > out->field_capacity) return aws_raise_error(AWS_ERROR_SHORT_BUFFER);
-    HB_CUDA_TRY(cudaMemcpyAsync(out->string_offsets, B.s_string_offsets.ptr, (2 * fields + 1) * sizeof(uint64_t),
-                                cudaMemcpyDeviceToHost, st));
-    HB_CUDA_TRY(cudaStreamSynchronize(st));
-    const uint64_t total = out->string_offsets[2 * fields];
-    if (total > out->strings_capacity) return aws_raise_error(AWS_ERROR_SHORT_BUFFER);
-    if (fields) {
-        HB_CUDA_TRY(cudaMemcpyAsync(out->field_kind, B.s_kind.ptr, fields, cudaMemcpyDeviceToHost, st));
-        HB_CUDA_TRY(cudaMemcpyAsync(out->field_index, B.s_index.ptr, fields * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-    }
-    if (total) HB_CUDA_TRY(cudaMemcpyAsync(out->strings, ctx->s_out.ptr, total, cudaMemcpyDeviceToHost, st));
+    HB_CUDA_TRY(ctx->s_out.reserve(out_capacity + 16));
+    HB_CUDA_TRY(ctx->s_out_off.reserve((n + 1) * sizeof(uint64_t)));
+    if (hpack_blocks_encode_on_device(ctx, n, d_field_offsets, F, never, kind, index, d_strings, d_string_offsets, S, mode,
+                                      ctx->s_out.as<uint8_t>(), out_capacity, ctx->s_out_off.as<uint64_t>(), d_status, st) ||
+        finish_packed(st, n, ctx->s_out_off.as<uint64_t>(), out_off, ctx->s_out.ptr, out, out_capacity, d_status, status))
+        return AWS_OP_ERR;
     HB_CUDA_TRY(cudaStreamSynchronize(st));
     return AWS_OP_SUCCESS;
 }
 
-// records: field_kind and field_index are read (aws_hpack_header_block_encode_records_batch), status is optional.
 int hpack_blocks_encode_host(
     aws_huffman_batch_ctx *ctx, const aws_hpack_header_lists *in, bool records, uint32_t mode, uint8_t *out,
     uint64_t out_capacity, uint64_t *out_off, int32_t *status) {
@@ -1381,53 +1319,10 @@ int hpack_blocks_encode_host(
     const uint64_t F = in->field_offsets[n];
     if (in->string_offsets[0] != 0 || !offsets_sorted(in->string_offsets, 2 * F + 1))
         return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
-    const uint64_t S = in->string_offsets[2 * F];
-    if (S && !in->strings) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
-    HB_CUDA_TRY(cudaSetDevice(ctx->device));
-    cudaStream_t st = ctx->stream;
-    hb_host::BlockBufs &B = ctx->blk;
-    HB_CUDA_TRY(B.s_field_offsets.reserve((n + 1) * sizeof(uint64_t)));
-    HB_CUDA_TRY(ctx->s_in.reserve(S + 16));
-    HB_CUDA_TRY(ctx->s_in_off.reserve((2 * F + 1) * sizeof(uint64_t)));
-    HB_CUDA_TRY(ctx->s_out.reserve(out_capacity + 16));
-    HB_CUDA_TRY(ctx->s_out_off.reserve((n + 1) * sizeof(uint64_t)));
-    HB_CUDA_TRY(cudaMemcpyAsync(B.s_field_offsets.ptr, in->field_offsets, (n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
-    if (S) HB_CUDA_TRY(cudaMemcpyAsync(ctx->s_in.ptr, in->strings, S, cudaMemcpyHostToDevice, st));
-    HB_CUDA_TRY(cudaMemcpyAsync(ctx->s_in_off.ptr, in->string_offsets, (2 * F + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
-    const uint8_t *never = nullptr;
-    if (in->never_indexed && F) {
-        HB_CUDA_TRY(B.s_never.reserve(F));
-        HB_CUDA_TRY(cudaMemcpyAsync(B.s_never.ptr, in->never_indexed, F, cudaMemcpyHostToDevice, st));
-        never = B.s_never.as<uint8_t>();
-    }
-    const uint8_t *kind = nullptr;
-    const uint64_t *index = nullptr;
-    if (records) {
-        HB_CUDA_TRY(B.s_kind.reserve(F + 1));
-        HB_CUDA_TRY(B.s_index.reserve((F + 1) * sizeof(uint64_t)));
-        HB_CUDA_TRY(ctx->s_status.reserve(n * sizeof(int32_t)));
-        if (F) {
-            HB_CUDA_TRY(cudaMemcpyAsync(B.s_kind.ptr, in->field_kind, F, cudaMemcpyHostToDevice, st));
-            HB_CUDA_TRY(cudaMemcpyAsync(B.s_index.ptr, in->field_index, F * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
-        }
-        kind = B.s_kind.as<uint8_t>();
-        index = B.s_index.as<uint64_t>();
-    }
-    int32_t *d_status = records ? ctx->s_status.as<int32_t>() : nullptr;
-    if (hpack_blocks_encode_on_device(ctx, n, B.s_field_offsets.as<uint64_t>(), F, never, kind, index, ctx->s_in.as<uint8_t>(),
-                                      ctx->s_in_off.as<uint64_t>(), S, mode, ctx->s_out.as<uint8_t>(), out_capacity,
-                                      ctx->s_out_off.as<uint64_t>(), d_status, st))
-        return AWS_OP_ERR;
-    HB_CUDA_TRY(cudaMemcpyAsync(out_off, ctx->s_out_off.ptr, (n + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-    if (status && d_status) HB_CUDA_TRY(cudaMemcpyAsync(status, d_status, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    HB_CUDA_TRY(cudaStreamSynchronize(st));
-    const uint64_t total = out_off[n];
-    if (total > out_capacity) return aws_raise_error(AWS_ERROR_SHORT_BUFFER);
-    if (total) {
-        HB_CUDA_TRY(cudaMemcpyAsync(out, ctx->s_out.ptr, total, cudaMemcpyDeviceToHost, st));
-        HB_CUDA_TRY(cudaStreamSynchronize(st));
-    }
-    return AWS_OP_SUCCESS;
+    if (in->string_offsets[2 * F] && !in->strings) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    cudaStream_t st;
+    if (call_begin(ctx, nullptr, &st)) return AWS_OP_ERR;
+    return call_end(ctx, st, hpack_blocks_encode_staged(ctx, in, records, mode, out, out_capacity, out_off, status, st));
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1502,6 +1397,100 @@ __global__ void encoded_length_kernel(hb::DeviceTables t, const uint8_t *in, con
 #pragma unroll
     for (int d = 16; d > 0; d >>= 1) bits += __shfl_xor_sync(0xffffffffu, bits, d);
     if (hb::lane_id() == 0) lens[item] = (bits + 7) >> 3;
+}
+
+int encoded_lengths_on_device(
+    aws_huffman_batch_ctx *ctx, const uint8_t *in, const uint64_t *in_offsets, size_t n, uint64_t *lens, cudaStream_t st) {
+    const unsigned blocks = (unsigned)((n + kWarpsPerBlock - 1) / kWarpsPerBlock);
+    encoded_length_kernel<<<blocks, kWarpsPerBlock * 32, 0, st>>>(ctx->tables, in, in_offsets, n, lens);
+    ++ctx->launches;
+    HB_CUDA_TRY(cudaGetLastError());
+    return AWS_OP_SUCCESS;
+}
+
+int encoded_lengths_staged(
+    aws_huffman_batch_ctx *ctx, const uint8_t *in, const uint64_t *in_offsets, size_t n, uint64_t *lens, cudaStream_t st) {
+    const uint64_t total_in = in_offsets[n];
+    const uint8_t *d_in = nullptr;
+    const uint64_t *d_in_off = nullptr;
+    uint64_t *d_lens = nullptr;
+    if (stage_in(ctx->s_in, total_in + 16, in, total_in, st, &d_in) ||
+        stage_in(ctx->s_in_off, (n + 1) * sizeof(uint64_t), in_offsets, n + 1, st, &d_in_off) ||
+        stage_in(ctx->scratch.lens, n * sizeof(uint64_t), lens, 0, st, &d_lens) ||
+        encoded_lengths_on_device(ctx, d_in, d_in_off, n, d_lens, st))
+        return AWS_OP_ERR;
+    HB_CUDA_TRY(cudaMemcpyAsync(lens, d_lens, n * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    HB_CUDA_TRY(cudaStreamSynchronize(st));
+    return AWS_OP_SUCCESS;
+}
+
+// What the launches need that depends only on the device and the code table, worked out once per context. The
+// dynamic shared-memory limits are the same for every context on a device (the encoders' compile-time sizes; the
+// decoders get all the device allows beside what they declare), so no context can lower another one's.
+int configure_kernels(aws_huffman_batch_ctx *ctx) {
+    constexpr cudaFuncAttribute kLimit = cudaFuncAttributeMaxDynamicSharedMemorySize;
+    int sms = 0, optin = 0;
+    if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ctx->device) == cudaSuccess && sms > 0)
+        ctx->sm_count = sms;
+    HB_CUDA_TRY(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, ctx->device));
+
+    HB_CUDA_TRY(cudaFuncSetAttribute(encode_tiled_kernel<false>, kLimit, (int)kEncSmemBytes));
+    HB_CUDA_TRY(cudaFuncSetAttribute(encode_tiled_kernel<true>, kLimit, (int)kEncSmemBytes));
+    HB_CUDA_TRY(cudaFuncSetAttribute(encode_slots_kernel, kLimit, (int)kEncSlotSmemBytes));
+    HB_CUDA_TRY(cudaFuncSetAttribute(str_pack_kernel, kLimit, (int)kStrPackSmemBytes));
+    HB_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->enc_blocks_per_sm[0], encode_tiled_kernel<false>, kEncBlock, kEncSmemBytes));
+    HB_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->enc_blocks_per_sm[1], encode_tiled_kernel<true>, kEncBlock, kEncSmemBytes));
+    HB_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->enc_slots_blocks_per_sm, encode_slots_kernel, kEncBlock, kEncSlotSmemBytes));
+    HB_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->str_blocks_per_sm[0], str_bits_kernel, kBitsThreads, 0));
+    HB_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->str_blocks_per_sm[1], str_pack_kernel, kStrThreads, kStrPackSmemBytes));
+    for (int *per_sm : {&ctx->enc_blocks_per_sm[0], &ctx->enc_blocks_per_sm[1], &ctx->enc_slots_blocks_per_sm,
+                        &ctx->str_blocks_per_sm[0], &ctx->str_blocks_per_sm[1]})
+        *per_sm = std::max(1, *per_sm);
+
+    size_t declared[2] = {0, 0};  // static shared memory of decode_batch_kernel<framed>
+    auto open_up = [&](auto kernel, size_t *static_smem) -> int {
+        cudaFuncAttributes attr{};
+        HB_CUDA_TRY(cudaFuncGetAttributes(&attr, kernel));
+        if (static_smem) *static_smem = attr.sharedSizeBytes;
+        HB_CUDA_TRY(cudaFuncSetAttribute(kernel, kLimit, optin - (int)attr.sharedSizeBytes));
+        return AWS_OP_SUCCESS;
+    };
+    if (open_up(decode_batch_kernel<false>, &declared[0]) || open_up(decode_batch_kernel<true>, &declared[1]) ||
+        open_up(stream_fused_kernel, nullptr) || open_up(stream_sync_kernel, nullptr) || open_up(stream_write_kernel, nullptr))
+        return AWS_OP_ERR;
+
+    // decode_batch_fast. Shared memory of one block (two blocks per SM): [LUT][stage][rows]. A string of L bytes
+    // decodes to at most 8 L / min_len symbols, so the row area is that much larger than the stage; and the dense
+    // output image (which reuses the stage and the front of the rows) must end before row offset `front`
+    // (decode_batch_kernel step 4): rows <= stage + front - 32.
+    const uint32_t min_len = std::max<uint32_t>(1, ctx->tables.min_len);
+    const size_t lut_bytes = (size_t)ctx->lut2_count * 8;
+    for (int framed = 0; framed < 2; ++framed) {
+        // one block per SM: [LUT2][team 0: stage, rows][team 1: stage, rows] + the teams' static arrays (what the
+        // kernel declares is asked from the runtime: every KB of the SM's 227 is a string more per tile)
+        const size_t budget = (((size_t)227 * 1024 - declared[framed] - lut_bytes) / kDecTeams - 128) & ~size_t(15);
+        const double expand = 8.0 / min_len;
+        size_t stage_bytes = (size_t)((double)budget / (1.0 + expand)) & ~size_t(15);
+        stage_bytes = std::max<size_t>(stage_bytes, 2 * kDecMaxRow);
+        size_t rows_bytes = budget - stage_bytes;
+        const size_t front = (stage_bytes - kDecMaxRow - 32) & ~size_t(3);
+        rows_bytes = std::min(rows_bytes, stage_bytes + front - 64) & ~size_t(15);
+        const size_t team_bytes = ((stage_bytes + 15) & ~size_t(15)) + rows_bytes + 64;
+        ctx->dec_layout[framed] = {stage_bytes, rows_bytes, lut_bytes + kDecTeams * team_bytes};
+    }
+
+    // decode_stream_fast
+    hb_host::StreamLayout &S = ctx->stream_layout;
+    S.smem = ctx->tables.lut_count * sizeof(uint32_t);
+    S.smem_staged = S.smem + kStreamStageWords * sizeof(uint32_t);
+    S.row_words = (((kChunkBits + 31) / min_len + 4 + 3) / 4) | 1u;
+    const size_t stage_bytes = (kStreamStageWords * 4 + 15) & ~size_t(15);
+    const size_t team_bytes = (stage_bytes + (size_t)kStreamThreads * S.row_words * 4 + 16 + 15) & ~size_t(15);
+    S.fused_smem = lut_bytes + kStreamTeams * team_bytes;  // one block per SM, two teams, one table
+    // (the dense output image reuses the stage and the front of the rows: stream_fused_kernel step 5)
+    S.fused = (size_t)kStreamThreads * S.row_words * 4 + 16 <= 2 * stage_bytes - S.row_words * 4 - 32 &&
+              S.fused_smem <= 220 * 1024 && !ctx->no_fused_stream;
+    return AWS_OP_SUCCESS;
 }
 
 }  // namespace
@@ -1681,11 +1670,6 @@ static int hb_ctx_from_codes(
         HB_CTX_TRY(cudaMalloc(&ctx->d_lut2, lut2.size() * sizeof(uint2)));
         HB_CTX_TRY(cudaMemcpy(ctx->d_lut2, lut2.data(), lut2.size() * sizeof(uint2), cudaMemcpyHostToDevice));
     }
-    {
-        int sms = 0;
-        if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device_id) == cudaSuccess && sms > 0)
-            ctx->sm_count = sms;
-    }
 #undef HB_CTX_TRY
 
     ctx->tables.enc = ctx->d_enc;
@@ -1699,6 +1683,10 @@ static int hb_ctx_from_codes(
     ctx->lut_smem_entries = std::min<uint32_t>(lut.count, kLutMaxSmemEntries);
     if (ctx->lut_smem_entries < (1u << lut.root_bits)) ctx->lut_smem_entries = 1u << lut.root_bits;
     huffman_lut_clean_up(&lut);
+    if (configure_kernels(ctx)) {
+        aws_huffman_batch_ctx_destroy(ctx);
+        return AWS_OP_ERR;
+    }
 
     *out_ctx = ctx;
     return AWS_OP_SUCCESS;
@@ -1707,27 +1695,9 @@ static int hb_ctx_from_codes(
 void aws_huffman_batch_ctx_destroy(struct aws_huffman_batch_ctx *ctx) {
     if (!ctx) return;
     cudaSetDevice(ctx->device);
-    if (ctx->stream) {
-        cudaStreamSynchronize(ctx->stream);
-        cudaStreamDestroy(ctx->stream);
-        if (ctx->scratch_free) cudaEventDestroy(ctx->scratch_free);
-    }
-    if (ctx->d_enc) cudaFree(ctx->d_enc);
-    if (ctx->d_lut) cudaFree(ctx->d_lut);
-    if (ctx->d_lut2) cudaFree(ctx->d_lut2);
-    GrowBuf *bufs[] = {&ctx->s_in,       &ctx->s_in_off,      &ctx->s_out,      &ctx->s_out_off,
-                       &ctx->s_caps,     &ctx->s_status,      &ctx->s_consumed, &ctx->s_ovf_pattern,
-                       &ctx->s_ovf_bits, &ctx->s_left_bits,   &ctx->s_left_num, &ctx->hp_pay,
-                       &ctx->hp_pay_off, &ctx->hp_dec,        &ctx->hp_dec_off, &ctx->hp_huff,
-                       &ctx->hp_prefix,  &ctx->hp_lens,       &ctx->hp_pay_lens, &ctx->hp_dec_status,
-                       &ctx->hp_left_bits, &ctx->hp_left_num, &ctx->hp_status};
-    for (GrowBuf *g : bufs) g->release();
-    if (ctx->h_scalar) cudaFreeHost(ctx->h_scalar);
-    ctx->blk.release();
-    ctx->scratch.release();
-    for (Lane &lane : ctx->lanes) lane.release();
-    (void)cudaGetLastError();
+    if (ctx->stream) cudaStreamSynchronize(ctx->stream);
     delete ctx;
+    (void)cudaGetLastError();
 }
 
 int aws_huffman_encode_batch(struct aws_huffman_batch_ctx *ctx, const struct aws_huffman_batch *batch) {
@@ -1750,48 +1720,28 @@ int aws_huffman_encode_batch_resume_device(
     struct aws_huffman_batch_ctx *ctx,
     const struct aws_huffman_batch *batch,
     void *cuda_stream) {
-    if (!ctx) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
-    if (check_batch(batch) || check_resume(batch, true)) return AWS_OP_ERR;
-    cudaStream_t st;
-    if (device_call_begin(ctx, cuda_stream, &st)) return AWS_OP_ERR;
-    hb::BatchView v = make_view(batch);
-    v.resume = true;
-    return device_call_end(ctx, st, encode_on_device(ctx, ctx->scratch, v, batch->in_size, st));
+    return run_device_batch(ctx, batch, cuda_stream, true, true);
 }
 
 int aws_huffman_decode_batch_resume_device(
     struct aws_huffman_batch_ctx *ctx,
     const struct aws_huffman_batch *batch,
     void *cuda_stream) {
-    if (!ctx) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
-    if (check_batch(batch) || check_resume(batch, false)) return AWS_OP_ERR;
-    cudaStream_t st;
-    if (device_call_begin(ctx, cuda_stream, &st)) return AWS_OP_ERR;
-    hb::BatchView v = make_view(batch);
-    v.resume = true;
-    return device_call_end(ctx, st, decode_on_device(ctx, ctx->scratch, v, batch->in_size, st));
+    return run_device_batch(ctx, batch, cuda_stream, false, true);
 }
 
 int aws_huffman_encode_batch_device(
     struct aws_huffman_batch_ctx *ctx,
     const struct aws_huffman_batch *batch,
     void *cuda_stream) {
-    if (!ctx) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
-    if (check_batch(batch)) return AWS_OP_ERR;
-    cudaStream_t st;
-    if (device_call_begin(ctx, cuda_stream, &st)) return AWS_OP_ERR;
-    return device_call_end(ctx, st, encode_on_device(ctx, ctx->scratch, make_view(batch), batch->in_size, st));
+    return run_device_batch(ctx, batch, cuda_stream, true, false);
 }
 
 int aws_huffman_decode_batch_device(
     struct aws_huffman_batch_ctx *ctx,
     const struct aws_huffman_batch *batch,
     void *cuda_stream) {
-    if (!ctx) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
-    if (check_batch(batch)) return AWS_OP_ERR;
-    cudaStream_t st;
-    if (device_call_begin(ctx, cuda_stream, &st)) return AWS_OP_ERR;
-    return device_call_end(ctx, st, decode_on_device(ctx, ctx->scratch, make_view(batch), batch->in_size, st));
+    return run_device_batch(ctx, batch, cuda_stream, false, false);
 }
 
 int aws_huffman_histogram_device(const uint8_t *in, uint64_t size, uint64_t *counts, void *cuda_stream) {
@@ -1845,8 +1795,8 @@ int aws_hpack_string_encode_batch_device(
     if (!ctx || (n && (!in_offsets || !out_offsets)) || (unsigned)mode > (unsigned)AWS_HPACK_HUFFMAN_ALWAYS)
         return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
     cudaStream_t st;
-    if (device_call_begin(ctx, cuda_stream, &st)) return AWS_OP_ERR;
-    return device_call_end(
+    if (call_begin(ctx, cuda_stream, &st)) return AWS_OP_ERR;
+    return call_end(
         ctx, st, hpack_encode_on_device(ctx, n, in, in_offsets, in_size, (uint32_t)mode, out, out_capacity, out_offsets, st));
 }
 
@@ -1855,8 +1805,8 @@ int aws_hpack_string_decode_batch_device(
     uint8_t *out, uint64_t out_capacity, uint64_t *out_offsets, int32_t *status, void *cuda_stream) {
     if (!ctx || (n && (!in_offsets || !out_offsets))) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
     cudaStream_t st;
-    if (device_call_begin(ctx, cuda_stream, &st)) return AWS_OP_ERR;
-    return device_call_end(
+    if (call_begin(ctx, cuda_stream, &st)) return AWS_OP_ERR;
+    return call_end(
         ctx, st, hpack_decode_on_device(ctx, n, in, in_offsets, in_size, out, out_capacity, out_offsets, status, st));
 }
 
@@ -1886,8 +1836,8 @@ int aws_hpack_header_block_decode_batch_device(
     if (!ctx || (n && !in_offsets) || (in_size && !in) || check_block_lists(out, true) || out->n != n)
         return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
     cudaStream_t st;
-    if (device_call_begin(ctx, cuda_stream, &st)) return AWS_OP_ERR;
-    return device_call_end(ctx, st, hpack_blocks_decode_on_device(ctx, n, in, in_offsets, block_lists(out), status, false, st));
+    if (call_begin(ctx, cuda_stream, &st)) return AWS_OP_ERR;
+    return call_end(ctx, st, hpack_blocks_decode_on_device(ctx, n, in, in_offsets, block_lists(out), status, false, st));
 }
 
 int aws_hpack_header_block_encode_batch_device(
@@ -1898,8 +1848,8 @@ int aws_hpack_header_block_encode_batch_device(
         (unsigned)mode > (unsigned)AWS_HPACK_HUFFMAN_ALWAYS)
         return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
     cudaStream_t st;
-    if (device_call_begin(ctx, cuda_stream, &st)) return AWS_OP_ERR;
-    return device_call_end(ctx, st,
+    if (call_begin(ctx, cuda_stream, &st)) return AWS_OP_ERR;
+    return call_end(ctx, st,
                            hpack_blocks_encode_on_device(ctx, in->n, in->field_offsets, num_fields, in->never_indexed, nullptr,
                                                          nullptr, in->strings, in->string_offsets, strings_size, (uint32_t)mode,
                                                          out, out_capacity, out_offsets, nullptr, st));
@@ -1913,8 +1863,8 @@ int aws_hpack_header_block_encode_records_batch_device(
         (out_capacity && !out) || (strings_size && !in->strings) || (unsigned)mode > (unsigned)AWS_HPACK_HUFFMAN_ALWAYS)
         return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
     cudaStream_t st;
-    if (device_call_begin(ctx, cuda_stream, &st)) return AWS_OP_ERR;
-    return device_call_end(ctx, st,
+    if (call_begin(ctx, cuda_stream, &st)) return AWS_OP_ERR;
+    return call_end(ctx, st,
                            hpack_blocks_encode_on_device(ctx, in->n, in->field_offsets, num_fields, in->never_indexed,
                                                          in->field_kind, in->field_index, in->strings, in->string_offsets,
                                                          strings_size, (uint32_t)mode, out, out_capacity, out_offsets, status,
@@ -1929,23 +1879,10 @@ int aws_huffman_get_encoded_length_batch(
     uint64_t *lens) {
     if (!ctx || (n && (!in_offsets || !lens))) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
     if (n == 0) return AWS_OP_SUCCESS;
-    HB_CUDA_TRY(cudaSetDevice(ctx->device));
-    cudaStream_t st = ctx->stream;
-    const uint64_t total_in = in_offsets[n];
-    if (total_in && !in) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
-    HB_CUDA_TRY(ctx->s_in.reserve(total_in + 16));
-    HB_CUDA_TRY(ctx->s_in_off.reserve((n + 1) * sizeof(uint64_t)));
-    HB_CUDA_TRY(ctx->scratch.lens.reserve(n * sizeof(uint64_t)));
-    if (total_in) HB_CUDA_TRY(cudaMemcpyAsync(ctx->s_in.ptr, in, total_in, cudaMemcpyHostToDevice, st));
-    HB_CUDA_TRY(cudaMemcpyAsync(ctx->s_in_off.ptr, in_offsets, (n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
-    const unsigned blocks = (unsigned)((n + kWarpsPerBlock - 1) / kWarpsPerBlock);
-    encoded_length_kernel<<<blocks, kWarpsPerBlock * 32, 0, st>>>(
-        ctx->tables, ctx->s_in.as<uint8_t>(), ctx->s_in_off.as<uint64_t>(), n, ctx->scratch.lens.as<uint64_t>());
-    ++ctx->launches;
-    HB_CUDA_TRY(cudaGetLastError());
-    HB_CUDA_TRY(cudaMemcpyAsync(lens, ctx->scratch.lens.ptr, n * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
-    HB_CUDA_TRY(cudaStreamSynchronize(st));
-    return AWS_OP_SUCCESS;
+    if (in_offsets[n] && !in) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    cudaStream_t st;
+    if (call_begin(ctx, nullptr, &st)) return AWS_OP_ERR;
+    return call_end(ctx, st, encoded_lengths_staged(ctx, in, in_offsets, n, lens, st));
 }
 
 int aws_huffman_batch_ctx_synchronize(struct aws_huffman_batch_ctx *ctx) {
@@ -2095,12 +2032,8 @@ int aws_huffman_get_encoded_length_batch_device(
     if (!ctx || (n && (!in_offsets || !lens))) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
     if (n == 0) return AWS_OP_SUCCESS;
     cudaStream_t st;
-    if (device_call_begin(ctx, cuda_stream, &st)) return AWS_OP_ERR;
-    const unsigned blocks = (unsigned)((n + kWarpsPerBlock - 1) / kWarpsPerBlock);
-    encoded_length_kernel<<<blocks, kWarpsPerBlock * 32, 0, st>>>(ctx->tables, in, in_offsets, n, lens);
-    ++ctx->launches;
-    HB_CUDA_TRY(cudaGetLastError());
-    return device_call_end(ctx, st, AWS_OP_SUCCESS);
+    if (call_begin(ctx, cuda_stream, &st)) return AWS_OP_ERR;
+    return call_end(ctx, st, encoded_lengths_on_device(ctx, in, in_offsets, n, lens, st));
 }
 
 }  // extern "C"

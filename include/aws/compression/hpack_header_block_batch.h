@@ -4,7 +4,8 @@
  * Batched HPACK header blocks (RFC 7541 section 6 representations, Appendix A static table) on the device: the
  * layer above the string literals of hpack_string_batch.h. Same context, same conventions: CSR batches with 64-bit
  * offsets, packed output, AWS_ERROR_SHORT_BUFFER meaning "offsets are complete: size and retry", host and _device
- * entry points, no CPU fallback (AWS_ERROR_COMPRESSION_DEVICE_FAILURE without a device).
+ * entry points, no CPU fallback (AWS_ERROR_COMPRESSION_DEVICE_FAILURE without a device). A host-pointer call first
+ * waits for the context's device calls still in flight on other streams.
  *
  * The wire layer of a header block is stateless: where each representation starts, its kind, its integers, its
  * literals and the static table (indices 1..61) are all read here. Only the meaning of an index >= 62 depends on

@@ -30,7 +30,8 @@ enum aws_hpack_huffman_mode {
 
 AWS_EXTERN_C_BEGIN
 
-/* n strings in, n string literals out (H bit, length, payload). Host pointers. */
+/* n strings in, n string literals out (H bit, length, payload). Host pointers. A host-pointer call first waits for
+ * the context's device calls still in flight on other streams. */
 AWS_COMPRESSION_API
 int aws_hpack_string_encode_batch(
     struct aws_huffman_batch_ctx *ctx,

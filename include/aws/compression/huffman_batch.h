@@ -99,7 +99,8 @@ int aws_huffman_batch_ctx_new_from_code_table(
 AWS_COMPRESSION_API
 void aws_huffman_batch_ctx_destroy(struct aws_huffman_batch_ctx *ctx);
 
-/* Host buffers in, host buffers out (copies staged through the context's stream). */
+/* Host buffers in, host buffers out (copies staged through the context's stream). A host-pointer call first waits
+ * for the context's device calls still in flight on other streams. */
 AWS_COMPRESSION_API
 int aws_huffman_encode_batch(struct aws_huffman_batch_ctx *ctx, const struct aws_huffman_batch *batch);
 
