@@ -856,12 +856,19 @@ int run_host_batch(aws_huffman_batch_ctx *ctx, const aws_huffman_batch *b, bool 
     return call_end(ctx, st, run_host_batch_staged(ctx, b, encode, resume, st));
 }
 
+// An empty packed batch on the device: its whole result is out_offsets[0] = 0 (NULL: nothing to write).
+int write_empty_packed(uint64_t *out_offsets, cudaStream_t st) {
+    if (out_offsets) HB_CUDA_TRY(cudaMemsetAsync(out_offsets, 0, sizeof(uint64_t), st));
+    return AWS_OP_SUCCESS;
+}
+
 // Device-pointer entry point shared by encode and decode.
 int run_device_batch(aws_huffman_batch_ctx *ctx, const aws_huffman_batch *b, void *cuda_stream, bool encode, bool resume) {
     if (!ctx) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
     if (check_batch(b) || (resume && check_resume(b, encode))) return AWS_OP_ERR;
     cudaStream_t st;
     if (call_begin(ctx, cuda_stream, &st)) return AWS_OP_ERR;
+    if (b->n == 0) return call_end(ctx, st, b->out_caps ? AWS_OP_SUCCESS : write_empty_packed(b->out_offsets, st));
     hb::BatchView v = make_view(b);
     v.resume = resume;
     return call_end(ctx, st, encode ? encode_on_device(ctx, ctx->scratch, v, b->in_size, st)
@@ -1796,6 +1803,7 @@ int aws_hpack_string_encode_batch_device(
         return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
     cudaStream_t st;
     if (call_begin(ctx, cuda_stream, &st)) return AWS_OP_ERR;
+    if (n == 0) return call_end(ctx, st, write_empty_packed(out_offsets, st));
     return call_end(
         ctx, st, hpack_encode_on_device(ctx, n, in, in_offsets, in_size, (uint32_t)mode, out, out_capacity, out_offsets, st));
 }
@@ -1806,6 +1814,7 @@ int aws_hpack_string_decode_batch_device(
     if (!ctx || (n && (!in_offsets || !out_offsets))) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
     cudaStream_t st;
     if (call_begin(ctx, cuda_stream, &st)) return AWS_OP_ERR;
+    if (n == 0) return call_end(ctx, st, write_empty_packed(out_offsets, st));
     return call_end(
         ctx, st, hpack_decode_on_device(ctx, n, in, in_offsets, in_size, out, out_capacity, out_offsets, status, st));
 }
