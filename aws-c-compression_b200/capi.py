@@ -148,6 +148,9 @@ EXPORTED_SYMBOLS = [
     "aws_hpack_header_block_decode_batch", "aws_hpack_header_block_encode_batch",
     "aws_hpack_header_block_decode_batch_device", "aws_hpack_header_block_encode_batch_device",
     "aws_hpack_header_block_encode_records_batch", "aws_hpack_header_block_encode_records_batch_device",
+    "aws_hpack_string_encode_batch_multi", "aws_hpack_string_decode_batch_multi",
+    "aws_hpack_header_block_decode_batch_multi", "aws_hpack_header_block_encode_batch_multi",
+    "aws_hpack_header_block_encode_records_batch_multi",
 ]
 
 
@@ -238,24 +241,34 @@ class Library:
         L.aws_huffman_batch_plan_shards.restype = C.c_int
         L.aws_huffman_batch_concat_offsets.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]
         L.aws_huffman_batch_concat_offsets.restype = C.c_int
-        L.aws_hpack_header_block_decode_batch.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p,
-                                                          P(aws_hpack_header_lists), C.c_void_p]
-        L.aws_hpack_header_block_encode_batch.argtypes = [C.c_void_p, P(aws_hpack_header_lists), C.c_int, C.c_void_p,
-                                                          C.c_uint64, C.c_void_p]
         L.aws_hpack_header_block_decode_batch_device.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_uint64,
                                                                  P(aws_hpack_header_lists), C.c_void_p, C.c_void_p]
         L.aws_hpack_header_block_encode_batch_device.argtypes = [C.c_void_p, P(aws_hpack_header_lists), C.c_uint64,
                                                                  C.c_uint64, C.c_int, C.c_void_p, C.c_uint64, C.c_void_p,
                                                                  C.c_void_p]
-        L.aws_hpack_header_block_encode_records_batch.argtypes = [C.c_void_p, P(aws_hpack_header_lists), C.c_int,
-                                                                  C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]
         L.aws_hpack_header_block_encode_records_batch_device.argtypes = [
             C.c_void_p, P(aws_hpack_header_lists), C.c_uint64, C.c_uint64, C.c_int, C.c_void_p, C.c_uint64, C.c_void_p,
             C.c_void_p, C.c_void_p]
-        for name in ("aws_hpack_header_block_decode_batch", "aws_hpack_header_block_encode_batch",
-                     "aws_hpack_header_block_decode_batch_device", "aws_hpack_header_block_encode_batch_device",
-                     "aws_hpack_header_block_encode_records_batch", "aws_hpack_header_block_encode_records_batch_device"):
+        for name in ("aws_hpack_header_block_decode_batch_device", "aws_hpack_header_block_encode_batch_device",
+                     "aws_hpack_header_block_encode_records_batch_device"):
             getattr(L, name).restype = C.c_int
+        # the HPACK host-pointer calls and their _multi forms (ctxs, n_ctx ahead of the same arguments)
+        hpack_host = {
+            "aws_hpack_string_encode_batch": [C.c_size_t, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_uint64,
+                                              C.c_void_p],
+            "aws_hpack_string_decode_batch": [C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p,
+                                              C.c_void_p],
+            "aws_hpack_header_block_decode_batch": [C.c_size_t, C.c_void_p, C.c_void_p, P(aws_hpack_header_lists),
+                                                    C.c_void_p],
+            "aws_hpack_header_block_encode_batch": [P(aws_hpack_header_lists), C.c_int, C.c_void_p, C.c_uint64,
+                                                    C.c_void_p],
+            "aws_hpack_header_block_encode_records_batch": [P(aws_hpack_header_lists), C.c_int, C.c_void_p, C.c_uint64,
+                                                            C.c_void_p, C.c_void_p],
+        }
+        for name, args in hpack_host.items():
+            getattr(L, name).argtypes = [C.c_void_p] + args
+            getattr(L, name + "_multi").argtypes = [C.c_void_p, C.c_size_t] + args
+            getattr(L, name).restype = getattr(L, name + "_multi").restype = C.c_int
 
     def last_error(self):
         return self.lib.aws_last_error()
@@ -712,3 +725,18 @@ def run_multi(contexts, encode, data, in_offsets, out_capacity):
     if rc != 0:
         raise CodecError(lib.last_error(), "aws_huffman_%s_batch_multi" % ("encode" if encode else "decode"))
     return res
+
+
+def hpack_host_call(target, name, *args, n_ctx=None, library=None):
+    """One HPACK host-pointer entry point, `name` as the single-context call is named (e.g.
+    "aws_hpack_header_block_decode_batch"), with the raw arguments that follow the context: on one BatchContext, or its
+    _multi form when `target` is a list of BatchContexts (None entries are NULL contexts; target None is a NULL array,
+    of n_ctx entries). Returns 0, or the error code the call raised."""
+    lib = library or (target.library if isinstance(target, BatchContext) else product_library())
+    if isinstance(target, BatchContext):
+        rc = getattr(lib.lib, name)(target.handle, *args)
+    else:
+        handles = None if target is None else (C.c_void_p * max(len(target), 1))(
+            *[c.handle if c is not None else None for c in target])
+        rc = getattr(lib.lib, name + "_multi")(handles, len(target) if n_ctx is None else n_ctx, *args)
+    return 0 if rc == 0 else lib.last_error()

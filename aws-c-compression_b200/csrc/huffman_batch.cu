@@ -20,8 +20,11 @@
 #include "decode_fast.cuh"
 
 #include <algorithm>
+#include <array>
+#include <condition_variable>
 #include <cstdio>
 #include <cstring>
+#include <mutex>
 #include <new>
 #include <thread>
 #include <vector>
@@ -586,6 +589,15 @@ __global__ void add_base_kernel(uint64_t *offsets, uint64_t count, uint64_t base
     if (i < count) offsets[i] += base;
 }
 
+// offsets[0..count) += base on the device (0 - b subtracts b: the sum wraps).
+int add_base(aws_huffman_batch_ctx *ctx, uint64_t *offsets, uint64_t count, uint64_t base, cudaStream_t st) {
+    if (base == 0 || count == 0) return AWS_OP_SUCCESS;
+    add_base_kernel<<<(unsigned)((count + 255) / 256), 256, 0, st>>>(offsets, count, base);
+    ++ctx->launches;
+    HB_CUDA_TRY(cudaGetLastError());
+    return AWS_OP_SUCCESS;
+}
+
 int lane_prepare(Lane &lane) {
     if (lane.stream) return AWS_OP_SUCCESS;
     HB_CUDA_TRY(cudaStreamCreateWithFlags(&lane.stream, cudaStreamNonBlocking));
@@ -648,6 +660,35 @@ int finish_packed(cudaStream_t st, size_t count, const uint64_t *d_offsets, uint
     const uint64_t total = offsets[count];
     if (total > capacity) return aws_raise_error(AWS_ERROR_SHORT_BUFFER);
     if (d_out && total) HB_CUDA_TRY(cudaMemcpyAsync(out, d_out, total, cudaMemcpyDeviceToHost, st));
+    return AWS_OP_SUCCESS;
+}
+
+// One value the host needs before it can go on (an output size): copied down and waited for.
+int read_back(const uint64_t *d_value, uint64_t *value, cudaStream_t st) {
+    HB_CUDA_TRY(cudaMemcpyAsync(value, d_value, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    HB_CUDA_TRY(cudaStreamSynchronize(st));
+    return AWS_OP_SUCCESS;
+}
+
+// The end of a host-pointer call for one slice of its items (all of them, or one shard of a multi call) whose packed
+// output starts at `base` in the caller's arrays: the slice's `count` offsets, and the closing one when the slice is
+// the last, are rebased on the device and come down to `offsets`, with status when the caller asked for it. Then
+// AWS_ERROR_SHORT_BUFFER when the whole call's output `total` is over `capacity` (offsets and status are complete),
+// else the slice's `size` payload octets go to out + base (d_out == NULL: there is none). The caller synchronises
+// `st` after its last copy.
+int finish_slice(aws_huffman_batch_ctx *ctx, cudaStream_t st, size_t count, bool last, uint64_t *d_offsets, uint64_t *offsets,
+                 uint64_t base, const void *d_out, void *out, uint64_t size, uint64_t total, uint64_t capacity,
+                 const int32_t *d_status = nullptr, int32_t *status = nullptr) {
+    const size_t entries = count + (last ? 1 : 0);
+    if (add_base(ctx, d_offsets, entries, base, st)) return AWS_OP_ERR;
+    if (entries) HB_CUDA_TRY(cudaMemcpyAsync(offsets, d_offsets, entries * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    if (status && d_status && count)
+        HB_CUDA_TRY(cudaMemcpyAsync(status, d_status, count * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    if (total > capacity) {
+        HB_CUDA_TRY(cudaStreamSynchronize(st));
+        return aws_raise_error(AWS_ERROR_SHORT_BUFFER);
+    }
+    if (d_out && size) HB_CUDA_TRY(cudaMemcpyAsync(static_cast<uint8_t *>(out) + base, d_out, size, cudaMemcpyDeviceToHost, st));
     return AWS_OP_SUCCESS;
 }
 
@@ -997,15 +1038,18 @@ int hpack_decode_on_device(
     return AWS_OP_SUCCESS;
 }
 
-// Host pointers: stage in, run, stage out.
-int hpack_run_staged(
-    aws_huffman_batch_ctx *ctx, bool encode, size_t n, const uint8_t *in, const uint64_t *in_off, uint32_t mode, uint8_t *out,
-    uint64_t out_capacity, uint64_t *out_off, int32_t *status, cudaStream_t st) {
-    const uint64_t total_in = in_off[n];
+// Host pointers, run on the device: the n items of in_off[0..n] (offsets into the caller's `in`) are staged from
+// octet in_base on, their offsets rebased to it, and framed or decoded into the context's staging, out_capacity
+// octets at most; *size receives the output size. hpack_run_finish then writes them into the caller's arrays.
+int hpack_run_slice(
+    aws_huffman_batch_ctx *ctx, bool encode, size_t n, const uint8_t *in, const uint64_t *in_off, uint64_t in_base,
+    uint32_t mode, uint64_t out_capacity, uint64_t *size, cudaStream_t st) {
+    const uint64_t total_in = in_off[n] - in_base;
     const uint8_t *d_in = nullptr;
-    const uint64_t *d_in_off = nullptr;
-    if (stage_in(ctx->s_in, total_in + 16, in, total_in, st, &d_in) ||
-        stage_in(ctx->s_in_off, (n + 1) * sizeof(uint64_t), in_off, n + 1, st, &d_in_off))
+    uint64_t *d_in_off = nullptr;
+    if (stage_in(ctx->s_in, total_in + 16, in + in_base, total_in, st, &d_in) ||
+        stage_in(ctx->s_in_off, (n + 1) * sizeof(uint64_t), in_off, n + 1, st, &d_in_off) ||
+        add_base(ctx, d_in_off, n + 1, 0 - in_base, st))
         return AWS_OP_ERR;
     HB_CUDA_TRY(ctx->s_out.reserve(out_capacity + 16));
     HB_CUDA_TRY(ctx->s_out_off.reserve((n + 1) * sizeof(uint64_t)));
@@ -1016,21 +1060,51 @@ int hpack_run_staged(
     if (encode ? hpack_encode_on_device(ctx, n, d_in, d_in_off, total_in, mode, d_out, out_capacity, d_out_off, st)
                : hpack_decode_on_device(ctx, n, d_in, d_in_off, total_in, d_out, out_capacity, d_out_off, d_status, st))
         return AWS_OP_ERR;
-    if (finish_packed(st, n, d_out_off, out_off, d_out, out, out_capacity, encode ? nullptr : d_status, status))
+    return read_back(d_out_off + n, size, st);
+}
+
+// Host pointers, finish into place: the items hpack_run_slice ran are the caller's from out_off / status on (the
+// closing offset too when `last`), their `size` octets go to out + base; `total`, the output size of the whole call,
+// decides AWS_ERROR_SHORT_BUFFER.
+int hpack_run_finish(
+    aws_huffman_batch_ctx *ctx, bool encode, size_t n, bool last, uint64_t base, uint64_t size, uint64_t total, uint8_t *out,
+    uint64_t out_capacity, uint64_t *out_off, int32_t *status, cudaStream_t st) {
+    if (finish_slice(ctx, st, n, last, ctx->s_out_off.as<uint64_t>(), out_off, base, ctx->s_out.ptr, out, size, total,
+                     out_capacity, encode ? nullptr : ctx->s_status.as<int32_t>(), status))
         return AWS_OP_ERR;
     HB_CUDA_TRY(cudaStreamSynchronize(st));
+    return AWS_OP_SUCCESS;
+}
+
+// Host pointers: run on the device, then finish at base 0.
+int hpack_run_staged(
+    aws_huffman_batch_ctx *ctx, bool encode, size_t n, const uint8_t *in, const uint64_t *in_off, uint32_t mode, uint8_t *out,
+    uint64_t out_capacity, uint64_t *out_off, int32_t *status, cudaStream_t st) {
+    uint64_t size = 0;
+    if (hpack_run_slice(ctx, encode, n, in, in_off, 0, mode, out_capacity, &size, st)) return AWS_OP_ERR;
+    return hpack_run_finish(ctx, encode, n, true, 0, size, size, out, out_capacity, out_off, status, st);
+}
+
+// Arguments of the host-pointer literal calls; a call with no items is answered here (*done).
+int hpack_host_args(size_t n, const uint8_t *in, const uint64_t *in_off, const uint8_t *out, uint64_t out_capacity,
+                    uint64_t *out_off, bool *done) {
+    *done = false;
+    if (n && (!in_off || !out_off)) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    if (n == 0) {
+        if (out_off) out_off[0] = 0;
+        *done = true;
+        return AWS_OP_SUCCESS;
+    }
+    if ((in_off[n] && !in) || (out_capacity && !out)) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
     return AWS_OP_SUCCESS;
 }
 
 int hpack_run_host(
     aws_huffman_batch_ctx *ctx, bool encode, size_t n, const uint8_t *in, const uint64_t *in_off, uint32_t mode, uint8_t *out,
     uint64_t out_capacity, uint64_t *out_off, int32_t *status) {
-    if (!ctx || (n && (!in_off || !out_off))) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
-    if (n == 0) {
-        if (out_off) out_off[0] = 0;
-        return AWS_OP_SUCCESS;
-    }
-    if ((in_off[n] && !in) || (out_capacity && !out)) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    bool done;
+    if (!ctx) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    if (hpack_host_args(n, in, in_off, out, out_capacity, out_off, &done) || done) return done ? AWS_OP_SUCCESS : AWS_OP_ERR;
     cudaStream_t st;
     if (call_begin(ctx, nullptr, &st)) return AWS_OP_ERR;
     return call_end(ctx, st, hpack_run_staged(ctx, encode, n, in, in_off, mode, out, out_capacity, out_off, status, st));
@@ -1236,89 +1310,156 @@ BlockLists block_lists(const aws_hpack_header_lists *l) {
                       l->string_offsets};
 }
 
-// Host pointers: stage in, run, stage out (the way hpack_run_host does).
+// Host pointers, run on the device (the way hpack_run_slice does): the n blocks of in_off[0..n] are staged from octet
+// in_base on and decoded into the context's staging, within the capacities given; size[0] receives their fields and,
+// when those fit field_capacity, size[1] their string octets.
+int hpack_blocks_decode_slice(
+    aws_huffman_batch_ctx *ctx, size_t n, const uint8_t *in, const uint64_t *in_off, uint64_t in_base,
+    uint64_t field_capacity, uint64_t strings_capacity, uint64_t size[2], cudaStream_t st) {
+    hb_host::BlockBufs &B = ctx->blk;
+    const uint64_t total_in = in_off[n] - in_base;
+    const uint8_t *d_in = nullptr;
+    uint64_t *d_in_off = nullptr;
+    BlockLists o{nullptr, field_capacity, nullptr, nullptr, nullptr, strings_capacity, nullptr};
+    if (stage_in(ctx->s_in, total_in + 16, in + in_base, total_in, st, &d_in) ||
+        stage_in(ctx->s_in_off, (n + 1) * sizeof(uint64_t), in_off, n + 1, st, &d_in_off) ||
+        add_base(ctx, d_in_off, n + 1, 0 - in_base, st))
+        return AWS_OP_ERR;
+    HB_CUDA_TRY(B.s_field_offsets.reserve((n + 1) * sizeof(uint64_t)));
+    HB_CUDA_TRY(ctx->s_status.reserve(n * sizeof(int32_t)));
+    o.field_offsets = B.s_field_offsets.as<uint64_t>();
+    if (hpack_blocks_decode_on_device(ctx, n, d_in, d_in_off, o, ctx->s_status.as<int32_t>(), true, st) ||
+        read_back(o.field_offsets + n, &size[0], st))
+        return AWS_OP_ERR;
+    size[1] = 0;  // (string offsets exist for the fields that fit)
+    return size[0] <= field_capacity ? read_back(B.s_string_offsets.as<uint64_t>() + 2 * size[0], &size[1], st) : AWS_OP_SUCCESS;
+}
+
+// Host pointers, finish into place: the blocks hpack_blocks_decode_slice ran are the caller's from block `first` on,
+// their fields from field base[0] on and their string octets from base[1] on; `total` (fields, string octets) of the
+// whole call decides AWS_ERROR_SHORT_BUFFER.
+int hpack_blocks_decode_finish(
+    aws_huffman_batch_ctx *ctx, size_t first, size_t n, bool last, const uint64_t base[2], const uint64_t size[2],
+    const uint64_t total[2], aws_hpack_header_lists *out, int32_t *status, cudaStream_t st) {
+    hb_host::BlockBufs &B = ctx->blk;
+    const uint64_t fields = size[0];
+    // field records (no payload of their own here), then the strings behind them
+    if (finish_slice(ctx, st, n, last, B.s_field_offsets.as<uint64_t>(), out->field_offsets + first, base[0], nullptr, nullptr,
+                     0, total[0], out->field_capacity, ctx->s_status.as<int32_t>(), status ? status + first : nullptr) ||
+        finish_slice(ctx, st, 2 * fields, last, B.s_string_offsets.as<uint64_t>(), out->string_offsets + 2 * base[0], base[1],
+                     ctx->s_out.ptr, out->strings, size[1], total[1], out->strings_capacity))
+        return AWS_OP_ERR;
+    if (fields) {
+        HB_CUDA_TRY(cudaMemcpyAsync(out->field_kind + base[0], B.s_kind.ptr, fields, cudaMemcpyDeviceToHost, st));
+        HB_CUDA_TRY(cudaMemcpyAsync(out->field_index + base[0], B.s_index.ptr, fields * sizeof(uint64_t),
+                                    cudaMemcpyDeviceToHost, st));
+    }
+    HB_CUDA_TRY(cudaStreamSynchronize(st));
+    return AWS_OP_SUCCESS;
+}
+
+// Host pointers: run on the device, then finish at base 0.
 int hpack_blocks_decode_staged(
     aws_huffman_batch_ctx *ctx, size_t n, const uint8_t *in, const uint64_t *in_off, aws_hpack_header_lists *out,
     int32_t *status, cudaStream_t st) {
-    hb_host::BlockBufs &B = ctx->blk;
-    const uint64_t total_in = in_off[n];
-    const uint8_t *d_in = nullptr;
-    const uint64_t *d_in_off = nullptr;
-    BlockLists o = block_lists(out);
-    if (stage_in(ctx->s_in, total_in + 16, in, total_in, st, &d_in) ||
-        stage_in(ctx->s_in_off, (n + 1) * sizeof(uint64_t), in_off, n + 1, st, &d_in_off) ||
-        stage_in(B.s_field_offsets, (n + 1) * sizeof(uint64_t), out->field_offsets, 0, st, &o.field_offsets))
+    const uint64_t base[2] = {0, 0};
+    uint64_t size[2];
+    if (hpack_blocks_decode_slice(ctx, n, in, in_off, 0, out->field_capacity, out->strings_capacity, size, st))
         return AWS_OP_ERR;
-    HB_CUDA_TRY(ctx->s_status.reserve(n * sizeof(int32_t)));
-    if (hpack_blocks_decode_on_device(ctx, n, d_in, d_in_off, o, ctx->s_status.as<int32_t>(), true, st)) return AWS_OP_ERR;
-    // field records (no payload of their own here), then the strings behind them
-    if (finish_packed(st, n, o.field_offsets, out->field_offsets, nullptr, nullptr, out->field_capacity,
-                      ctx->s_status.as<int32_t>(), status))
-        return AWS_OP_ERR;
-    const uint64_t fields = out->field_offsets[n];
-    if (finish_packed(st, 2 * fields, B.s_string_offsets.as<uint64_t>(), out->string_offsets, ctx->s_out.ptr, out->strings,
-                      out->strings_capacity))
-        return AWS_OP_ERR;
-    if (fields) {
-        HB_CUDA_TRY(cudaMemcpyAsync(out->field_kind, B.s_kind.ptr, fields, cudaMemcpyDeviceToHost, st));
-        HB_CUDA_TRY(cudaMemcpyAsync(out->field_index, B.s_index.ptr, fields * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    return hpack_blocks_decode_finish(ctx, 0, n, true, base, size, size, out, status, st);
+}
+
+// Arguments of the host-pointer decode calls; a call with no blocks is answered here (*done).
+int hpack_blocks_decode_args(size_t n, const uint8_t *in, const uint64_t *in_off, aws_hpack_header_lists *out, bool *done) {
+    *done = false;
+    if ((n && !in_off) || check_block_lists(out, true) || out->n != n) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    if (n == 0) {
+        out->field_offsets[0] = 0;
+        out->string_offsets[0] = 0;
+        *done = true;
+        return AWS_OP_SUCCESS;
     }
-    HB_CUDA_TRY(cudaStreamSynchronize(st));
+    if ((in_off[n] && !in) || !offsets_sorted(in_off, n + 1)) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
     return AWS_OP_SUCCESS;
 }
 
 int hpack_blocks_decode_host(
     aws_huffman_batch_ctx *ctx, size_t n, const uint8_t *in, const uint64_t *in_off, aws_hpack_header_lists *out,
     int32_t *status) {
-    if (!ctx || (n && !in_off) || check_block_lists(out, true) || out->n != n) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
-    if (n == 0) {
-        out->field_offsets[0] = 0;
-        out->string_offsets[0] = 0;
-        return AWS_OP_SUCCESS;
-    }
-    if ((in_off[n] && !in) || !offsets_sorted(in_off, n + 1)) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    bool done;
+    if (!ctx) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    if (hpack_blocks_decode_args(n, in, in_off, out, &done) || done) return done ? AWS_OP_SUCCESS : AWS_OP_ERR;
     cudaStream_t st;
     if (call_begin(ctx, nullptr, &st)) return AWS_OP_ERR;
     return call_end(ctx, st, hpack_blocks_decode_staged(ctx, n, in, in_off, out, status, st));
 }
 
-// records: field_kind and field_index are read (aws_hpack_header_block_encode_records_batch), status is optional.
-int hpack_blocks_encode_staged(
-    aws_huffman_batch_ctx *ctx, const aws_hpack_header_lists *in, bool records, uint32_t mode, uint8_t *out,
-    uint64_t out_capacity, uint64_t *out_off, int32_t *status, cudaStream_t st) {
+// Host pointers, run on the device: lists [first, first + n) of `in` are staged, their field and string offsets
+// rebased to their first field and first string octet, and encoded into the context's staging, out_capacity octets at
+// most; *size receives the output size. records: field_kind and field_index are read
+// (aws_hpack_header_block_encode_records_batch) and a status per list is written to the staging.
+int hpack_blocks_encode_slice(
+    aws_huffman_batch_ctx *ctx, const aws_hpack_header_lists *in, size_t first, size_t n, bool records, uint32_t mode,
+    uint64_t out_capacity, uint64_t *size, cudaStream_t st) {
     hb_host::BlockBufs &B = ctx->blk;
-    const uint64_t n = in->n, F = in->field_offsets[n], S = in->string_offsets[2 * F];
-    const uint64_t *d_field_offsets = nullptr, *d_string_offsets = nullptr;
+    const uint64_t f0 = in->field_offsets[first], F = in->field_offsets[first + n] - f0;
+    const uint64_t s0 = in->string_offsets[2 * f0], S = in->string_offsets[2 * (f0 + F)] - s0;
+    uint64_t *d_field_offsets = nullptr, *d_string_offsets = nullptr;
     const uint8_t *d_strings = nullptr, *never = nullptr, *kind = nullptr;
     const uint64_t *index = nullptr;
     int32_t *d_status = nullptr;
-    if (stage_in(B.s_field_offsets, (n + 1) * sizeof(uint64_t), in->field_offsets, n + 1, st, &d_field_offsets) ||
-        stage_in(ctx->s_in, S + 16, in->strings, S, st, &d_strings) ||
-        stage_in(ctx->s_in_off, (2 * F + 1) * sizeof(uint64_t), in->string_offsets, 2 * F + 1, st, &d_string_offsets) ||
-        (in->never_indexed && F && stage_in(B.s_never, F, in->never_indexed, F, st, &never)) ||
-        (records && (stage_in(B.s_kind, F + 1, in->field_kind, F, st, &kind) ||
-                     stage_in(B.s_index, (F + 1) * sizeof(uint64_t), in->field_index, F, st, &index) ||
-                     stage_in(ctx->s_status, n * sizeof(int32_t), status, 0, st, &d_status))))
+    if (records) {
+        HB_CUDA_TRY(ctx->s_status.reserve(n * sizeof(int32_t)));
+        d_status = ctx->s_status.as<int32_t>();
+    }
+    if (stage_in(B.s_field_offsets, (n + 1) * sizeof(uint64_t), in->field_offsets + first, n + 1, st, &d_field_offsets) ||
+        add_base(ctx, d_field_offsets, n + 1, 0 - f0, st) ||
+        stage_in(ctx->s_in, S + 16, in->strings + s0, S, st, &d_strings) ||
+        stage_in(ctx->s_in_off, (2 * F + 1) * sizeof(uint64_t), in->string_offsets + 2 * f0, 2 * F + 1, st, &d_string_offsets) ||
+        add_base(ctx, d_string_offsets, 2 * F + 1, 0 - s0, st) ||
+        (in->never_indexed && F && stage_in(B.s_never, F, in->never_indexed + f0, F, st, &never)) ||
+        (records && (stage_in(B.s_kind, F + 1, in->field_kind + f0, F, st, &kind) ||
+                     stage_in(B.s_index, (F + 1) * sizeof(uint64_t), in->field_index + f0, F, st, &index))))
         return AWS_OP_ERR;
     HB_CUDA_TRY(ctx->s_out.reserve(out_capacity + 16));
     HB_CUDA_TRY(ctx->s_out_off.reserve((n + 1) * sizeof(uint64_t)));
     if (hpack_blocks_encode_on_device(ctx, n, d_field_offsets, F, never, kind, index, d_strings, d_string_offsets, S, mode,
-                                      ctx->s_out.as<uint8_t>(), out_capacity, ctx->s_out_off.as<uint64_t>(), d_status, st) ||
-        finish_packed(st, n, ctx->s_out_off.as<uint64_t>(), out_off, ctx->s_out.ptr, out, out_capacity, d_status, status))
+                                      ctx->s_out.as<uint8_t>(), out_capacity, ctx->s_out_off.as<uint64_t>(), d_status, st))
+        return AWS_OP_ERR;
+    return read_back(ctx->s_out_off.as<uint64_t>() + n, size, st);
+}
+
+// Host pointers, finish into place: the lists hpack_blocks_encode_slice ran are the caller's from list `first` on,
+// their `size` octets go to out + base; `total`, the output size of the whole call, decides AWS_ERROR_SHORT_BUFFER.
+int hpack_blocks_encode_finish(
+    aws_huffman_batch_ctx *ctx, size_t first, size_t n, bool last, bool records, uint64_t base, uint64_t size, uint64_t total,
+    uint8_t *out, uint64_t out_capacity, uint64_t *out_off, int32_t *status, cudaStream_t st) {
+    if (finish_slice(ctx, st, n, last, ctx->s_out_off.as<uint64_t>(), out_off + first, base, ctx->s_out.ptr, out, size, total,
+                     out_capacity, records ? ctx->s_status.as<int32_t>() : nullptr, status ? status + first : nullptr))
         return AWS_OP_ERR;
     HB_CUDA_TRY(cudaStreamSynchronize(st));
     return AWS_OP_SUCCESS;
 }
 
-int hpack_blocks_encode_host(
+// Host pointers: run on the device, then finish at base 0.
+int hpack_blocks_encode_staged(
     aws_huffman_batch_ctx *ctx, const aws_hpack_header_lists *in, bool records, uint32_t mode, uint8_t *out,
-    uint64_t out_capacity, uint64_t *out_off, int32_t *status) {
-    if (!ctx || check_block_lists(in, false) || !out_off || (out_capacity && !out) ||
-        (records && (!in->field_kind || !in->field_index)))
+    uint64_t out_capacity, uint64_t *out_off, int32_t *status, cudaStream_t st) {
+    uint64_t size = 0;
+    if (hpack_blocks_encode_slice(ctx, in, 0, in->n, records, mode, out_capacity, &size, st)) return AWS_OP_ERR;
+    return hpack_blocks_encode_finish(ctx, 0, in->n, true, records, 0, size, size, out, out_capacity, out_off, status, st);
+}
+
+// Arguments of the host-pointer encode calls; a call with no lists is answered here (*done).
+int hpack_blocks_encode_args(const aws_hpack_header_lists *in, bool records, const uint8_t *out, uint64_t out_capacity,
+                             uint64_t *out_off, bool *done) {
+    *done = false;
+    if (check_block_lists(in, false) || !out_off || (out_capacity && !out) || (records && (!in->field_kind || !in->field_index)))
         return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
     const uint64_t n = in->n;
     if (n == 0) {
         out_off[0] = 0;
+        *done = true;
         return AWS_OP_SUCCESS;
     }
     // (fields are numbered from 0 and every one is encoded: lists start at field 0, strings at octet 0)
@@ -1327,6 +1468,16 @@ int hpack_blocks_encode_host(
     if (in->string_offsets[0] != 0 || !offsets_sorted(in->string_offsets, 2 * F + 1))
         return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
     if (in->string_offsets[2 * F] && !in->strings) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    return AWS_OP_SUCCESS;
+}
+
+int hpack_blocks_encode_host(
+    aws_huffman_batch_ctx *ctx, const aws_hpack_header_lists *in, bool records, uint32_t mode, uint8_t *out,
+    uint64_t out_capacity, uint64_t *out_off, int32_t *status) {
+    bool done;
+    if (!ctx) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    if (hpack_blocks_encode_args(in, records, out, out_capacity, out_off, &done) || done)
+        return done ? AWS_OP_SUCCESS : AWS_OP_ERR;
     cudaStream_t st;
     if (call_begin(ctx, nullptr, &st)) return AWS_OP_ERR;
     return call_end(ctx, st, hpack_blocks_encode_staged(ctx, in, records, mode, out, out_capacity, out_off, status, st));
@@ -1498,6 +1649,177 @@ int configure_kernels(aws_huffman_batch_ctx *ctx) {
     S.fused = (size_t)kStreamThreads * S.row_words * 4 + 16 <= 2 * stage_bytes - S.row_words * 4 - 32 &&
               S.fused_smem <= 220 * 1024 && !ctx->no_fused_stream;
     return AWS_OP_SUCCESS;
+}
+
+// ---------------------------------------------------------------------------------------------
+// One host-pointer call over several contexts (the _multi entry points): the items are cut into one contiguous range
+// per context, balanced by bytes (aws_huffman_batch_plan_shards), and each range runs on a host thread of its own.
+// No collective: the shards never talk to each other.
+// ---------------------------------------------------------------------------------------------
+int check_contexts(aws_huffman_batch_ctx *const *ctxs, size_t n_ctx) {
+    if (!ctxs || n_ctx == 0) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    for (size_t d = 0; d < n_ctx; ++d)
+        if (!ctxs[d]) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    return AWS_OP_SUCCESS;
+}
+
+// shard(d) for d in [0, n_ctx), each on a thread of its own. The error slot is per thread, so every shard's error is
+// collected there; the first shard in item order that failed decides the call's error, whichever finished first.
+template <typename Shard>
+int run_shards(size_t n_ctx, const Shard &shard) {
+    std::vector<int> err(n_ctx, 0);
+    std::vector<std::thread> threads;
+    for (size_t d = 0; d < n_ctx; ++d) {
+        threads.emplace_back([&, d]() {
+            if (shard(d) != AWS_OP_SUCCESS) err[d] = aws_last_error() ? aws_last_error() : AWS_ERROR_COMPRESSION_DEVICE_FAILURE;
+        });
+    }
+    for (std::thread &t : threads) t.join();
+    for (int e : err)
+        if (e) return aws_raise_error(e);
+    return AWS_OP_SUCCESS;
+}
+
+// Output totals of one shard: octets out, or fields and string octets.
+using Totals = std::array<uint64_t, 2>;
+
+// Where the shard threads of one call meet after running their shards on the device: every thread publishes its
+// totals, or its failure, exactly once and waits for all the others (an empty shard publishes at once, a failed one
+// too, so no thread waits forever). Each leaves with the same totals, so each finds its own bases and reaches the
+// capacity decision the single-context call reaches.
+class ShardExchange {
+  public:
+    explicit ShardExchange(size_t shards) : totals_(shards), waiting_(shards) {}
+    // false when some shard failed: then no shard writes the caller's arrays
+    bool publish(size_t shard, bool ok, const Totals &totals) {
+        std::unique_lock<std::mutex> lock(mutex_);
+        totals_[shard] = totals;
+        failed_ |= !ok;
+        if (--waiting_ == 0) all_in_.notify_all();
+        else all_in_.wait(lock, [this] { return waiting_ == 0; });
+        return !failed_;
+    }
+    // (after publish) the sum over the shards before `shard`, i.e. its bases, and over all of them
+    Totals before(size_t shard) const {
+        Totals sum{0, 0};
+        for (size_t s = 0; s < shard; ++s)
+            for (size_t k = 0; k < sum.size(); ++k) sum[k] += totals_[s][k];
+        return sum;
+    }
+    Totals all() const { return before(totals_.size()); }
+
+  private:
+    std::vector<Totals> totals_;
+    size_t waiting_;
+    bool failed_ = false;
+    std::mutex mutex_;
+    std::condition_variable all_in_;
+};
+
+// An HPACK host-pointer call over several contexts, its shards planned on `weight` (n + 1 non-decreasing values).
+// Each shard's thread runs its slice on the device straight from the caller's arrays (run: shard totals out), meets
+// the others, and copies its offsets, status, records and payload into the caller's arrays at its bases (finish): no
+// host-side copy or concatenation of the per-item arrays.
+//     run(ctx, first, count, uint64_t *size, st)
+//     finish(ctx, first, count, bool last, const uint64_t *base, const uint64_t *size, const uint64_t *total, st)
+template <typename Run, typename Finish>
+int hpack_multi(aws_huffman_batch_ctx *const *ctxs, size_t n_ctx, size_t n, const uint64_t *weight, const Run &run,
+                const Finish &finish) {
+    std::vector<size_t> begin(n_ctx + 1);
+    if (aws_huffman_batch_plan_shards(weight, n, n_ctx, begin.data())) return AWS_OP_ERR;
+    ShardExchange exchange(n_ctx);
+    return run_shards(n_ctx, [&](size_t d) -> int {
+        aws_huffman_batch_ctx *ctx = ctxs[d];
+        const size_t first = begin[d], count = begin[d + 1] - first;
+        Totals size{0, 0};
+        if (count == 0) {  // no device work
+            exchange.publish(d, true, size);
+            return AWS_OP_SUCCESS;
+        }
+        cudaStream_t st;
+        if (call_begin(ctx, nullptr, &st)) {
+            exchange.publish(d, false, size);
+            return AWS_OP_ERR;
+        }
+        int rc = run(ctx, first, count, size.data(), st);
+        if (exchange.publish(d, rc == AWS_OP_SUCCESS, size)) {
+            const Totals base = exchange.before(d), total = exchange.all();
+            rc = finish(ctx, first, count, first + count == n, base.data(), size.data(), total.data(), st);
+        }
+        return call_end(ctx, st, rc);
+    });
+}
+
+int hpack_literals_multi(
+    aws_huffman_batch_ctx *const *ctxs, size_t n_ctx, bool encode, size_t n, const uint8_t *in, const uint64_t *in_off,
+    uint32_t mode, uint8_t *out, uint64_t out_capacity, uint64_t *out_off, int32_t *status) {
+    bool done;
+    if (check_contexts(ctxs, n_ctx)) return AWS_OP_ERR;
+    if (n_ctx == 1) return hpack_run_host(ctxs[0], encode, n, in, in_off, mode, out, out_capacity, out_off, status);
+    if (hpack_host_args(n, in, in_off, out, out_capacity, out_off, &done) || done) return done ? AWS_OP_SUCCESS : AWS_OP_ERR;
+    auto run = [&](aws_huffman_batch_ctx *ctx, size_t first, size_t count, uint64_t *size, cudaStream_t st) {
+        // the shard's staging holds all its output: framed, a prefix of at most 10 octets and a payload no longer than
+        // the string unless every literal is Huffman-coded; decoded, a raw payload or at most 8 / min_len symbols an octet
+        const uint64_t bytes = in_off[first + count] - in_off[first];
+        const uint64_t expand = mode == hb::kHpackAlways ? (std::max<uint32_t>(1, ctx->tables.max_len) + 7) / 8 : 1;
+        const uint64_t room = encode ? bytes * expand + 10 * (uint64_t)count + 64
+                                     : bytes * 8 / std::min<uint32_t>(8, std::max<uint32_t>(1, ctx->tables.min_len)) + 64;
+        return hpack_run_slice(ctx, encode, count, in, in_off + first, in_off[first], mode, std::min(out_capacity, room), size,
+                               st);
+    };
+    auto finish = [&](aws_huffman_batch_ctx *ctx, size_t first, size_t count, bool last, const uint64_t *base,
+                      const uint64_t *size, const uint64_t *total, cudaStream_t st) {
+        return hpack_run_finish(ctx, encode, count, last, base[0], size[0], total[0], out, out_capacity, out_off + first,
+                                status ? status + first : nullptr, st);
+    };
+    return hpack_multi(ctxs, n_ctx, n, in_off, run, finish);
+}
+
+int hpack_blocks_decode_multi(
+    aws_huffman_batch_ctx *const *ctxs, size_t n_ctx, size_t n, const uint8_t *in, const uint64_t *in_off,
+    aws_hpack_header_lists *out, int32_t *status) {
+    bool done;
+    if (check_contexts(ctxs, n_ctx)) return AWS_OP_ERR;
+    if (n_ctx == 1) return hpack_blocks_decode_host(ctxs[0], n, in, in_off, out, status);
+    if (hpack_blocks_decode_args(n, in, in_off, out, &done) || done) return done ? AWS_OP_SUCCESS : AWS_OP_ERR;
+    auto run = [&](aws_huffman_batch_ctx *ctx, size_t first, size_t count, uint64_t *size, cudaStream_t st) {
+        // (no capacities of the shard's own: its staging is sized from its totals, the caller's decide at the finish)
+        return hpack_blocks_decode_slice(ctx, count, in, in_off + first, in_off[first], ~0ull, ~0ull, size, st);
+    };
+    auto finish = [&](aws_huffman_batch_ctx *ctx, size_t first, size_t count, bool last, const uint64_t *base,
+                      const uint64_t *size, const uint64_t *total, cudaStream_t st) {
+        return hpack_blocks_decode_finish(ctx, first, count, last, base, size, total, out, status, st);
+    };
+    return hpack_multi(ctxs, n_ctx, n, in_off, run, finish);
+}
+
+int hpack_blocks_encode_multi(
+    aws_huffman_batch_ctx *const *ctxs, size_t n_ctx, const aws_hpack_header_lists *in, bool records, uint32_t mode,
+    uint8_t *out, uint64_t out_capacity, uint64_t *out_off, int32_t *status) {
+    bool done;
+    if (check_contexts(ctxs, n_ctx)) return AWS_OP_ERR;
+    if (n_ctx == 1) return hpack_blocks_encode_host(ctxs[0], in, records, mode, out, out_capacity, out_off, status);
+    if (hpack_blocks_encode_args(in, records, out, out_capacity, out_off, &done) || done)
+        return done ? AWS_OP_SUCCESS : AWS_OP_ERR;
+    // shards balanced by string octets: list i's start at string_offsets[2 * field_offsets[i]]
+    const size_t n = in->n;
+    std::vector<uint64_t> weight(n + 1);
+    for (size_t i = 0; i <= n; ++i) weight[i] = in->string_offsets[2 * in->field_offsets[i]];
+    auto run = [&](aws_huffman_batch_ctx *ctx, size_t first, size_t count, uint64_t *size, cudaStream_t st) {
+        // the shard's staging holds all its output: per field a representation of at most 10 octets and two literals
+        // behind prefixes of at most 10 octets each, no longer than the strings unless every literal is Huffman-coded
+        const uint64_t fields = in->field_offsets[first + count] - in->field_offsets[first];
+        const uint64_t octets = weight[first + count] - weight[first];
+        const uint64_t expand = mode == hb::kHpackAlways ? (std::max<uint32_t>(1, ctx->tables.max_len) + 7) / 8 : 1;
+        const uint64_t room = octets * expand + 30 * fields + 64;
+        return hpack_blocks_encode_slice(ctx, in, first, count, records, mode, std::min(out_capacity, room), size, st);
+    };
+    auto finish = [&](aws_huffman_batch_ctx *ctx, size_t first, size_t count, bool last, const uint64_t *base,
+                      const uint64_t *size, const uint64_t *total, cudaStream_t st) {
+        return hpack_blocks_encode_finish(ctx, first, count, last, records, base[0], size[0], total[0], out, out_capacity,
+                                          out_off, status, st);
+    };
+    return hpack_multi(ctxs, n_ctx, n, weight.data(), run, finish);
 }
 
 }  // namespace
@@ -1952,10 +2274,7 @@ int aws_huffman_batch_concat_offsets(
 // per context drives its shard through that context's own (pipelined) host path into a private buffer, and the
 // host concatenates payloads and offsets. No collective: the shards never talk to each other.
 static int hb_run_multi(struct aws_huffman_batch_ctx *const *ctxs, size_t n_ctx, const struct aws_huffman_batch *b, bool encode) {
-    if (!ctxs || n_ctx == 0) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
-    for (size_t d = 0; d < n_ctx; ++d)
-        if (!ctxs[d]) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
-    if (check_batch(b)) return AWS_OP_ERR;
+    if (check_contexts(ctxs, n_ctx) || check_batch(b)) return AWS_OP_ERR;
     if (b->out_caps) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);  // packed layout only
     const size_t n = b->n;
     if (n == 0) {
@@ -1968,15 +2287,12 @@ static int hb_run_multi(struct aws_huffman_batch_ctx *const *ctxs, size_t n_ctx,
     struct Shard {
         std::vector<uint64_t> in_off, out_off;
         std::vector<uint8_t> out;
-        int rc = AWS_OP_SUCCESS, err = 0;
     };
     std::vector<Shard> shards(n_ctx);
-    std::vector<std::thread> threads;
-    for (size_t d = 0; d < n_ctx; ++d) {
-        threads.emplace_back([&, d]() {
+    if (run_shards(n_ctx, [&](size_t d) -> int {
             Shard &sh = shards[d];
             const size_t a = begin[d], nd = begin[d + 1] - a;
-            if (nd == 0) return;
+            if (nd == 0) return AWS_OP_SUCCESS;
             const uint64_t in0 = b->in_offsets[a], bytes_in = b->in_offsets[a + nd] - in0;
             const uint32_t max_len = std::max<uint32_t>(1, ctxs[d]->tables.max_len), min_len = std::max<uint32_t>(1, ctxs[d]->tables.min_len);
             const uint64_t room = (encode ? bytes_in * ((max_len + 7) / 8) : (bytes_in * 8) / min_len) + 64;
@@ -1999,13 +2315,9 @@ static int hb_run_multi(struct aws_huffman_batch_ctx *const *ctxs, size_t n_ctx,
             if (b->overflow_num_bits) sb.overflow_num_bits = b->overflow_num_bits + a;
             if (b->leftover_working_bits) sb.leftover_working_bits = b->leftover_working_bits + a;
             if (b->leftover_num_bits) sb.leftover_num_bits = b->leftover_num_bits + a;
-            sh.rc = encode ? aws_huffman_encode_batch(ctxs[d], &sb) : aws_huffman_decode_batch(ctxs[d], &sb);
-            if (sh.rc != AWS_OP_SUCCESS) sh.err = aws_last_error();  // (the error slot is per thread)
-        });
-    }
-    for (std::thread &t : threads) t.join();
-    for (const Shard &sh : shards)
-        if (sh.rc != AWS_OP_SUCCESS) return aws_raise_error(sh.err ? sh.err : AWS_ERROR_COMPRESSION_DEVICE_FAILURE);
+            return encode ? aws_huffman_encode_batch(ctxs[d], &sb) : aws_huffman_decode_batch(ctxs[d], &sb);
+        }))
+        return AWS_OP_ERR;
     // the concatenation step
     std::vector<const uint64_t *> ptrs(n_ctx);
     std::vector<size_t> items(n_ctx);
@@ -2029,6 +2341,39 @@ int aws_huffman_encode_batch_multi(
 int aws_huffman_decode_batch_multi(
     struct aws_huffman_batch_ctx *const *ctxs, size_t n_ctx, const struct aws_huffman_batch *batch) {
     return hb_run_multi(ctxs, n_ctx, batch, false);
+}
+
+int aws_hpack_string_encode_batch_multi(
+    struct aws_huffman_batch_ctx *const *ctxs, size_t n_ctx, size_t n, const uint8_t *in, const uint64_t *in_offsets,
+    enum aws_hpack_huffman_mode mode, uint8_t *out, uint64_t out_capacity, uint64_t *out_offsets) {
+    if ((unsigned)mode > (unsigned)AWS_HPACK_HUFFMAN_ALWAYS) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    return hpack_literals_multi(ctxs, n_ctx, true, n, in, in_offsets, (uint32_t)mode, out, out_capacity, out_offsets, nullptr);
+}
+
+int aws_hpack_string_decode_batch_multi(
+    struct aws_huffman_batch_ctx *const *ctxs, size_t n_ctx, size_t n, const uint8_t *in, const uint64_t *in_offsets,
+    uint8_t *out, uint64_t out_capacity, uint64_t *out_offsets, int32_t *status) {
+    return hpack_literals_multi(ctxs, n_ctx, false, n, in, in_offsets, 0, out, out_capacity, out_offsets, status);
+}
+
+int aws_hpack_header_block_decode_batch_multi(
+    struct aws_huffman_batch_ctx *const *ctxs, size_t n_ctx, size_t n, const uint8_t *in, const uint64_t *in_offsets,
+    struct aws_hpack_header_lists *out, int32_t *status) {
+    return hpack_blocks_decode_multi(ctxs, n_ctx, n, in, in_offsets, out, status);
+}
+
+int aws_hpack_header_block_encode_batch_multi(
+    struct aws_huffman_batch_ctx *const *ctxs, size_t n_ctx, const struct aws_hpack_header_lists *in,
+    enum aws_hpack_huffman_mode mode, uint8_t *out, uint64_t out_capacity, uint64_t *out_offsets) {
+    if ((unsigned)mode > (unsigned)AWS_HPACK_HUFFMAN_ALWAYS) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    return hpack_blocks_encode_multi(ctxs, n_ctx, in, false, (uint32_t)mode, out, out_capacity, out_offsets, nullptr);
+}
+
+int aws_hpack_header_block_encode_records_batch_multi(
+    struct aws_huffman_batch_ctx *const *ctxs, size_t n_ctx, const struct aws_hpack_header_lists *in,
+    enum aws_hpack_huffman_mode mode, uint8_t *out, uint64_t out_capacity, uint64_t *out_offsets, int32_t *status) {
+    if ((unsigned)mode > (unsigned)AWS_HPACK_HUFFMAN_ALWAYS) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    return hpack_blocks_encode_multi(ctxs, n_ctx, in, true, (uint32_t)mode, out, out_capacity, out_offsets, status);
 }
 
 int aws_huffman_get_encoded_length_batch_device(

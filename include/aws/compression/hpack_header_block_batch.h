@@ -139,6 +139,48 @@ int aws_hpack_header_block_encode_records_batch(
     int32_t *status);
 
 /*
+ * The three calls above over several contexts, normally one per GPU of the box (contexts on the same device are
+ * allowed; all of them made from the same code table, none used elsewhere during the call). The blocks or lists are
+ * cut into n_ctx contiguous ranges balanced by octets (aws_huffman_batch_plan_shards): decode by block octets, encode
+ * by the lists' string octets. Each range is staged from the caller's arrays, runs on its context on a host thread of
+ * its own, and its records, offsets, status and octets are copied into place in the caller's arrays once every range
+ * knows its bases. The return value, the error and every array written are those of the single-context call on
+ * ctxs[0]: on AWS_ERROR_SHORT_BUFFER the offsets and status the rules above call complete are equal, and nothing is
+ * written past a capacity. A failure in several ranges reports the first range's error. n_ctx == 1 is that call.
+ * Errors of their own: AWS_ERROR_INVALID_ARGUMENT for ctxs == NULL, n_ctx == 0 or a NULL context.
+ */
+AWS_COMPRESSION_API
+int aws_hpack_header_block_decode_batch_multi(
+    struct aws_huffman_batch_ctx *const *ctxs,
+    size_t n_ctx,
+    size_t n,
+    const uint8_t *in,
+    const uint64_t *in_offsets,
+    struct aws_hpack_header_lists *out,
+    int32_t *status);
+
+AWS_COMPRESSION_API
+int aws_hpack_header_block_encode_batch_multi(
+    struct aws_huffman_batch_ctx *const *ctxs,
+    size_t n_ctx,
+    const struct aws_hpack_header_lists *in,
+    enum aws_hpack_huffman_mode mode,
+    uint8_t *out,
+    uint64_t out_capacity,
+    uint64_t *out_offsets);
+
+AWS_COMPRESSION_API
+int aws_hpack_header_block_encode_records_batch_multi(
+    struct aws_huffman_batch_ctx *const *ctxs,
+    size_t n_ctx,
+    const struct aws_hpack_header_lists *in,
+    enum aws_hpack_huffman_mode mode,
+    uint8_t *out,
+    uint64_t out_capacity,
+    uint64_t *out_offsets,
+    int32_t *status);
+
+/*
  * The same with device pointers (every array of `out` / `in` and `in`, `in_offsets`, `status`, `out`, `out_offsets`
  * live on the device); work is enqueued on cuda_stream (NULL = the context's stream). The caller reads the offsets
  * to learn the sizes and checks them against its capacities; nothing is written past a capacity.

@@ -67,6 +67,39 @@ int aws_hpack_string_decode_batch(
     uint64_t *out_offsets,
     int32_t *status);
 
+/*
+ * The same over several contexts, normally one per GPU of the box (contexts on the same device are allowed; all of
+ * them made from the same code table, none used elsewhere during the call). The items are cut into n_ctx contiguous
+ * ranges balanced by input octets (aws_huffman_batch_plan_shards); each range is staged from the caller's arrays, runs
+ * on its context on a host thread of its own and is copied into place in the caller's arrays. The return value, the
+ * error and every array written (out_offsets, out, status) are those of the single-context call on ctxs[0],
+ * AWS_ERROR_SHORT_BUFFER included; a failure in several ranges reports the first range's error. n_ctx == 1 is that
+ * call. Errors of their own: AWS_ERROR_INVALID_ARGUMENT for ctxs == NULL, n_ctx == 0 or a NULL context.
+ */
+AWS_COMPRESSION_API
+int aws_hpack_string_encode_batch_multi(
+    struct aws_huffman_batch_ctx *const *ctxs,
+    size_t n_ctx,
+    size_t n,
+    const uint8_t *in,
+    const uint64_t *in_offsets,
+    enum aws_hpack_huffman_mode mode,
+    uint8_t *out,
+    uint64_t out_capacity,
+    uint64_t *out_offsets);
+
+AWS_COMPRESSION_API
+int aws_hpack_string_decode_batch_multi(
+    struct aws_huffman_batch_ctx *const *ctxs,
+    size_t n_ctx,
+    size_t n,
+    const uint8_t *in,
+    const uint64_t *in_offsets,
+    uint8_t *out,
+    uint64_t out_capacity,
+    uint64_t *out_offsets,
+    int32_t *status);
+
 /* The same with device pointers; work is enqueued on cuda_stream (NULL = the context's stream). in_size ==
  * in_offsets[n] (the offsets live on the device). The caller reads out_offsets[n] to learn the size. */
 AWS_COMPRESSION_API
