@@ -18,6 +18,9 @@ HPACK_HUFFMAN_SMALLEST, HPACK_HUFFMAN_NEVER, HPACK_HUFFMAN_ALWAYS = 0, 1, 2
 # enum aws_hpack_field_kind
 (HPACK_FIELD_INDEXED, HPACK_FIELD_LITERAL_INCREMENTAL, HPACK_FIELD_LITERAL_WITHOUT_INDEXING,
  HPACK_FIELD_LITERAL_NEVER_INDEXED, HPACK_FIELD_TABLE_SIZE_UPDATE, HPACK_FIELD_AUTO) = range(6)
+# enum aws_qpack_field_kind
+(QPACK_FIELD_INDEXED_STATIC, QPACK_FIELD_INDEXED_DYNAMIC, QPACK_FIELD_INDEXED_POST_BASE, QPACK_FIELD_NAME_REF_STATIC,
+ QPACK_FIELD_NAME_REF_DYNAMIC, QPACK_FIELD_NAME_REF_POST_BASE, QPACK_FIELD_LITERAL_NAME, QPACK_FIELD_AUTO) = range(8)
 
 
 class CodecError(RuntimeError):
@@ -95,6 +98,23 @@ class aws_hpack_header_lists(C.Structure):
     ]
 
 
+class aws_qpack_field_sections(C.Structure):
+    _fields_ = [
+        ("n", C.c_size_t),
+        ("encoded_insert_count", C.c_void_p),
+        ("base_sign", C.c_void_p),
+        ("delta_base", C.c_void_p),
+        ("field_offsets", C.c_void_p),
+        ("field_capacity", C.c_uint64),
+        ("field_kind", C.c_void_p),
+        ("field_index", C.c_void_p),
+        ("never_indexed", C.c_void_p),
+        ("strings", C.c_void_p),
+        ("strings_capacity", C.c_uint64),
+        ("string_offsets", C.c_void_p),
+    ]
+
+
 class aws_huffman_table_coder(C.Structure):
     _fields_ = [("coder", aws_huffman_symbol_coder), ("codes", aws_huffman_code * 256),
                 ("lut_entries", C.c_void_p), ("lut_count", C.c_uint32), ("lut_root_bits", C.c_uint8)]
@@ -151,6 +171,9 @@ EXPORTED_SYMBOLS = [
     "aws_hpack_string_encode_batch_multi", "aws_hpack_string_decode_batch_multi",
     "aws_hpack_header_block_decode_batch_multi", "aws_hpack_header_block_encode_batch_multi",
     "aws_hpack_header_block_encode_records_batch_multi",
+    "aws_qpack_field_section_decode_batch", "aws_qpack_field_section_encode_batch",
+    "aws_qpack_field_section_encode_records_batch", "aws_qpack_field_section_decode_batch_device",
+    "aws_qpack_field_section_encode_batch_device", "aws_qpack_field_section_encode_records_batch_device",
 ]
 
 
@@ -269,6 +292,21 @@ class Library:
             getattr(L, name).argtypes = [C.c_void_p] + args
             getattr(L, name + "_multi").argtypes = [C.c_void_p, C.c_size_t] + args
             getattr(L, name).restype = getattr(L, name + "_multi").restype = C.c_int
+        Q = P(aws_qpack_field_sections)
+        qpack = {
+            "aws_qpack_field_section_decode_batch": [C.c_size_t, C.c_void_p, C.c_void_p, Q, C.c_void_p],
+            "aws_qpack_field_section_encode_batch": [Q, C.c_int, C.c_void_p, C.c_uint64, C.c_void_p],
+            "aws_qpack_field_section_encode_records_batch": [Q, C.c_int, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p],
+            "aws_qpack_field_section_decode_batch_device": [C.c_size_t, C.c_void_p, C.c_void_p, C.c_uint64, Q, C.c_void_p,
+                                                            C.c_void_p],
+            "aws_qpack_field_section_encode_batch_device": [Q, C.c_uint64, C.c_uint64, C.c_int, C.c_void_p, C.c_uint64,
+                                                            C.c_void_p, C.c_void_p],
+            "aws_qpack_field_section_encode_records_batch_device": [Q, C.c_uint64, C.c_uint64, C.c_int, C.c_void_p,
+                                                                    C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p],
+        }
+        for name, args in qpack.items():
+            getattr(L, name).argtypes = [C.c_void_p] + args
+            getattr(L, name).restype = C.c_int
 
     def last_error(self):
         return self.lib.aws_last_error()
@@ -667,6 +705,101 @@ class BatchContext:
         self._blocks_call("aws_hpack_header_block_encode_records_batch_device", C.byref(lists), int(num_fields),
                           int(strings_size), mode, _ptr(out), out.numel() if out_capacity is None else int(out_capacity),
                           _ptr(out_offsets), _ptr(status), stream or 0)
+
+    # ---- QPACK field sections (qpack_field_section_batch.h) ----
+    def qpack_decode_sections(self, data, in_offsets, field_capacity=None, strings_capacity=None):
+        """Host buffers. Capacities default to the documented bounds (in_size fields, 69 * in_size octets). On
+        failure the CodecError carries the arrays as `result` (offsets are complete on AWS_ERROR_SHORT_BUFFER)."""
+        data = np.ascontiguousarray(data, dtype=np.uint8)
+        in_offsets = np.ascontiguousarray(in_offsets, dtype=np.uint64)
+        n = len(in_offsets) - 1
+        in_size = int(in_offsets[-1])
+        field_capacity = in_size if field_capacity is None else int(field_capacity)
+        strings_capacity = 69 * in_size if strings_capacity is None else int(strings_capacity)
+        res = {"encoded_insert_count": np.zeros(n, np.uint64), "base_sign": np.zeros(n, np.uint8),
+               "delta_base": np.zeros(n, np.uint64), "field_offsets": np.zeros(n + 1, dtype=np.uint64),
+               "field_kind": np.zeros(max(field_capacity, 1), np.uint8),
+               "field_index": np.zeros(max(field_capacity, 1), np.uint64),
+               "never_indexed": np.zeros(max(field_capacity, 1), np.uint8),
+               "strings": np.zeros(max(strings_capacity, 1), np.uint8),
+               "string_offsets": np.zeros(2 * field_capacity + 1, np.uint64), "status": np.zeros(n, np.int32)}
+        sections = aws_qpack_field_sections(
+            n, _ptr(res["encoded_insert_count"]), _ptr(res["base_sign"]), _ptr(res["delta_base"]),
+            _ptr(res["field_offsets"]), field_capacity, _ptr(res["field_kind"]), _ptr(res["field_index"]),
+            _ptr(res["never_indexed"]), _ptr(res["strings"]), strings_capacity, _ptr(res["string_offsets"]))
+        try:
+            self._blocks_call("aws_qpack_field_section_decode_batch", n, _ptr(data), _ptr(in_offsets), C.byref(sections),
+                              _ptr(res["status"]))
+        except CodecError as err:
+            err.result = res
+            raise
+        return res
+
+    def qpack_encode_sections(self, field_offsets, strings, string_offsets, out_capacity, mode=HPACK_HUFFMAN_SMALLEST,
+                              never_indexed=None, records=None):
+        """Host buffers: header lists in, field sections out ({"out", "out_offsets"}, and "status" for records).
+        records = (encoded_insert_count, base_sign, delta_base, field_kind, field_index): the records encoder
+        (aws_qpack_field_section_encode_records_batch); None: the stateless one. On failure the CodecError carries
+        the arrays as `result`."""
+        field_offsets = np.ascontiguousarray(field_offsets, dtype=np.uint64)
+        strings = np.ascontiguousarray(strings, dtype=np.uint8)
+        string_offsets = np.ascontiguousarray(string_offsets, dtype=np.uint64)
+        if never_indexed is not None:
+            never_indexed = np.ascontiguousarray(never_indexed, dtype=np.uint8)
+        n = len(field_offsets) - 1
+        res = {"out": np.zeros(max(int(out_capacity), 1), dtype=np.uint8), "out_offsets": np.zeros(n + 1, dtype=np.uint64)}
+        prefix, kind, index = (None, None, None), None, None
+        if records is not None:
+            eic, sign, delta, kind, index = records
+            prefix = (np.ascontiguousarray(eic, dtype=np.uint64), np.ascontiguousarray(sign, dtype=np.uint8),
+                      np.ascontiguousarray(delta, dtype=np.uint64))
+            kind = np.ascontiguousarray(kind, dtype=np.uint8)
+            index = np.ascontiguousarray(index, dtype=np.uint64)
+            res["status"] = np.full(n, -1, dtype=np.int32)
+        sections = aws_qpack_field_sections(n, *[_ptr(a) for a in prefix], _ptr(field_offsets), 0, _ptr(kind), _ptr(index),
+                                            _ptr(never_indexed), _ptr(strings), 0, _ptr(string_offsets))
+        try:
+            if records is None:
+                self._blocks_call("aws_qpack_field_section_encode_batch", C.byref(sections), mode, _ptr(res["out"]),
+                                  int(out_capacity), _ptr(res["out_offsets"]))
+            else:
+                self._blocks_call("aws_qpack_field_section_encode_records_batch", C.byref(sections), mode,
+                                  _ptr(res["out"]), int(out_capacity), _ptr(res["out_offsets"]), _ptr(res["status"]))
+        except CodecError as err:
+            err.result = res
+            raise
+        return res
+
+    def qpack_decode_sections_device(self, n, in_, in_offsets, in_size, encoded_insert_count, base_sign, delta_base,
+                                     field_offsets, field_kind, field_index, never_indexed, strings, string_offsets,
+                                     status=None, stream=None, field_capacity=None, strings_capacity=None):
+        """Device pointers (torch CUDA tensors, or objects with data_ptr()); capacities default to the tensors' sizes
+        (field_capacity: (string_offsets.numel() - 1) // 2)."""
+        field_capacity = (string_offsets.numel() - 1) // 2 if field_capacity is None else int(field_capacity)
+        strings_capacity = strings.numel() if strings_capacity is None else int(strings_capacity)
+        sections = aws_qpack_field_sections(n, _ptr(encoded_insert_count), _ptr(base_sign), _ptr(delta_base),
+                                            _ptr(field_offsets), field_capacity, _ptr(field_kind), _ptr(field_index),
+                                            _ptr(never_indexed), _ptr(strings), strings_capacity, _ptr(string_offsets))
+        self._blocks_call("aws_qpack_field_section_decode_batch_device", n, _ptr(in_), _ptr(in_offsets), int(in_size),
+                          C.byref(sections), _ptr(status), stream or 0)
+
+    def qpack_encode_sections_device(self, n, field_offsets, num_fields, strings, string_offsets, strings_size, out,
+                                     out_offsets, mode=HPACK_HUFFMAN_SMALLEST, never_indexed=None, records=None,
+                                     status=None, out_capacity=None, stream=None):
+        """Device pointers; records = (encoded_insert_count, base_sign, delta_base, field_kind, field_index) selects
+        the records encoder. out_capacity defaults to out.numel()."""
+        prefix, kind, index = (None, None, None), None, None
+        if records is not None:
+            prefix, (kind, index) = records[:3], records[3:]
+        sections = aws_qpack_field_sections(n, *[_ptr(a) for a in prefix], _ptr(field_offsets), 0, _ptr(kind), _ptr(index),
+                                            _ptr(never_indexed), _ptr(strings), 0, _ptr(string_offsets))
+        cap = out.numel() if out_capacity is None else int(out_capacity)
+        if records is None:
+            self._blocks_call("aws_qpack_field_section_encode_batch_device", C.byref(sections), int(num_fields),
+                              int(strings_size), mode, _ptr(out), cap, _ptr(out_offsets), stream or 0)
+        else:
+            self._blocks_call("aws_qpack_field_section_encode_records_batch_device", C.byref(sections), int(num_fields),
+                              int(strings_size), mode, _ptr(out), cap, _ptr(out_offsets), _ptr(status), stream or 0)
 
     def encode(self, data, in_offsets, out_capacity, **kw):
         return self._host(True, data, in_offsets, out_capacity, **kw)

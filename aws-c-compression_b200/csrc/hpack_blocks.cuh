@@ -293,7 +293,17 @@ __global__ void hpack_field_records_kernel(
     }
 }
 
-// The strings: item i is string i & 1 (name, value) of parsed field i >> 1. 32 strings per warp.
+// The string source of HPACK fields for hpack_compose_kernel (qpack_sections.cuh has QPACK's).
+struct HpackFieldStrings {
+    __device__ static void get(uint8_t kind, uint64_t index, uint64_t lit, uint32_t which, const uint8_t *dec,
+                               const uint64_t *dec_offsets, const uint8_t *&src, uint64_t &len) {
+        hpack_field_string(kind, index, lit, which, dec, dec_offsets, src, len);
+    }
+};
+
+// The strings: item i is string i & 1 (name, value) of parsed field i >> 1. 32 strings per warp. Strings::get says
+// where a string of a parsed field comes from.
+template <typename Strings>
 __global__ void __launch_bounds__(256) hpack_compose_kernel(
     uint64_t num_parsed, const uint8_t *f_kind, const uint64_t *f_index, const uint32_t *f_block, const uint64_t *f_lits,
     const uint64_t *field_base, const int32_t *status, const uint64_t *field_offsets, uint64_t field_capacity,
@@ -310,7 +320,7 @@ __global__ void __launch_bounds__(256) hpack_compose_kernel(
         if (o != ~0ull) {
             const uint8_t *src;
             uint64_t len;
-            hpack_field_string(f_kind[f], f_index[f], f_lits[2 * f + w], w, dec, dec_offsets, src, len);
+            Strings::get(f_kind[f], f_index[f], f_lits[2 * f + w], w, dec, dec_offsets, src, len);
             const uint64_t o0 = string_offsets[2 * o + w];
             const uint64_t room = o0 < strings_capacity ? strings_capacity - o0 : 0;
             job.src = src;

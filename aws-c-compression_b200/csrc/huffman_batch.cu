@@ -7,6 +7,7 @@
 #include <aws/compression/huffman_batch.h>
 #include <aws/compression/hpack_string_batch.h>
 #include <aws/compression/hpack_header_block_batch.h>
+#include <aws/compression/qpack_field_section_batch.h>
 #include <aws/compression/huffman_table_builder.h>
 
 #include "../host/huffman_lut.h"
@@ -17,6 +18,7 @@
 #include "encode_strings.cuh"
 #include "hpack_literals.cuh"
 #include "hpack_blocks.cuh"
+#include "qpack_sections.cuh"
 #include "decode_fast.cuh"
 
 #include <algorithm>
@@ -103,13 +105,15 @@ struct Lane {
         if (stream) cudaStreamDestroy(stream);
     }
 };
-// HPACK header blocks (hpack_blocks.cuh): per-block counts and bases, parsed fields, literal spans and the decoded
-// literals, encode plans, and the staging of the host entry points' extra arrays.
+// HPACK header blocks (hpack_blocks.cuh) and QPACK field sections (qpack_sections.cuh): per-block counts and bases,
+// parsed fields, literal spans and the decoded literals, encode plans, and the staging of the host entry points' extra
+// arrays.
 struct BlockBufs {
     GrowBuf num_fields, num_lits, lit_bytes, struct_status, out_fields, status, field_base, lit_base, lit_byte_base,
         f_kind, f_index, f_block, f_lits, lit_src, lit_offsets, lits, dec, dec_offsets, lit_status, str_lens, plan,
         plan_index, field_lens, field_pos, framed, framed_offsets, s_field_offsets, s_never, s_kind, s_index,
         s_string_offsets;
+    GrowBuf lit_len, sec_lens, s_eic, s_sign, s_delta;  // QPACK only: literal lengths and H bits, section sizes, prefixes
     uint64_t *h_totals = nullptr;  // pinned: fields, literals, literal octets
     ~BlockBufs() {
         if (h_totals) cudaFreeHost(h_totals);
@@ -1230,7 +1234,7 @@ int hpack_blocks_decode_on_device(
         o.kind, o.index, B.str_lens.as<uint64_t>());
     ++ctx->launches;
     if (launch_scan(ctx, ctx->scratch, B.str_lens.as<uint64_t>(), o.string_offsets, 2 * kept, st)) return AWS_OP_ERR;
-    hb::hpack_compose_kernel<<<grid_of(2 * parsed, 256), 256, 0, st>>>(
+    hb::hpack_compose_kernel<hb::HpackFieldStrings><<<grid_of(2 * parsed, 256), 256, 0, st>>>(
         parsed, f_kind, f_index, f_block, f_lits, field_base, status, o.field_offsets, o.field_capacity, dec, dec_offsets,
         o.strings, o.strings_capacity, o.string_offsets);
     ++ctx->launches;
@@ -1481,6 +1485,355 @@ int hpack_blocks_encode_host(
     cudaStream_t st;
     if (call_begin(ctx, nullptr, &st)) return AWS_OP_ERR;
     return call_end(ctx, st, hpack_blocks_encode_staged(ctx, in, records, mode, out, out_capacity, out_off, status, st));
+}
+
+// ---------------------------------------------------------------------------------------------
+// QPACK field sections (qpack_sections.cuh) over the same literal layer, the same buffers and the same passes as the
+// HPACK header blocks above. Device pointers in, device pointers out.
+// ---------------------------------------------------------------------------------------------
+// stage: `o` holds the prefix arrays and field_offsets (context staging) and the capacities; the per-field outputs go
+// to context staging sized from the totals (the host entry point copies them back).
+int qpack_sections_decode_on_device(
+    aws_huffman_batch_ctx *ctx, uint64_t n, const uint8_t *in, const uint64_t *in_off, aws_qpack_field_sections o,
+    int32_t *status, bool stage, cudaStream_t st) {
+    hb_host::BlockBufs &B = ctx->blk;
+    if (n == 0) {
+        HB_CUDA_TRY(cudaMemsetAsync(o.field_offsets, 0, sizeof(uint64_t), st));
+        if (o.string_offsets && !stage) HB_CUDA_TRY(cudaMemsetAsync(o.string_offsets, 0, sizeof(uint64_t), st));
+        return AWS_OP_SUCCESS;
+    }
+    const unsigned flat = grid_of(n, 256);
+    HB_CUDA_TRY(B.num_fields.reserve(n * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.num_lits.reserve(n * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.lit_bytes.reserve(n * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.out_fields.reserve(n * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.struct_status.reserve(n * sizeof(int32_t)));
+    HB_CUDA_TRY(B.field_base.reserve((n + 1) * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.lit_base.reserve((n + 1) * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.lit_byte_base.reserve((n + 1) * sizeof(uint64_t)));
+    if (!status) {
+        HB_CUDA_TRY(B.status.reserve(n * sizeof(int32_t)));
+        status = B.status.as<int32_t>();
+    }
+    if (!B.h_totals) HB_CUDA_TRY(cudaHostAlloc(reinterpret_cast<void **>(&B.h_totals), 3 * sizeof(uint64_t), cudaHostAllocDefault));
+    uint64_t *field_base = B.field_base.as<uint64_t>(), *lit_base = B.lit_base.as<uint64_t>();
+    uint64_t *lit_byte_base = B.lit_byte_base.as<uint64_t>();
+
+    // 1. structure, counts; 2. their bases, and the totals the later launches are sized from
+    hb::qpack_section_scan_kernel<<<flat, 256, 0, st>>>(
+        n, in, in_off, B.num_fields.as<uint64_t>(), B.num_lits.as<uint64_t>(), B.lit_bytes.as<uint64_t>(), B.struct_status.as<int32_t>());
+    ++ctx->launches;
+    if (launch_scan(ctx, ctx->scratch, B.num_fields.as<uint64_t>(), field_base, n, st)) return AWS_OP_ERR;
+    if (launch_scan(ctx, ctx->scratch, B.num_lits.as<uint64_t>(), lit_base, n, st)) return AWS_OP_ERR;
+    if (launch_scan(ctx, ctx->scratch, B.lit_bytes.as<uint64_t>(), lit_byte_base, n, st)) return AWS_OP_ERR;
+    HB_CUDA_TRY(cudaMemcpyAsync(B.h_totals + 0, field_base + n, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    HB_CUDA_TRY(cudaMemcpyAsync(B.h_totals + 1, lit_base + n, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    HB_CUDA_TRY(cudaMemcpyAsync(B.h_totals + 2, lit_byte_base + n, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    HB_CUDA_TRY(cudaStreamSynchronize(st));
+    const uint64_t parsed = B.h_totals[0], num_lits = B.h_totals[1], lit_total = B.h_totals[2];
+    const uint64_t kept = std::min(parsed, o.field_capacity);  // field slots that can be written
+    const uint32_t min_len = std::max<uint32_t>(1, ctx->tables.min_len);
+    const uint64_t dec_cap = lit_total * 8 / min_len + 64;
+    if (stage) {
+        // (a field's strings are its decoded literals or at most 69 octets of Appendix A)
+        o.strings_capacity = std::min(o.strings_capacity, dec_cap + 69 * kept);
+        HB_CUDA_TRY(B.s_kind.reserve(kept + 1));
+        HB_CUDA_TRY(B.s_index.reserve((kept + 1) * sizeof(uint64_t)));
+        HB_CUDA_TRY(B.s_never.reserve(kept + 1));
+        HB_CUDA_TRY(B.s_string_offsets.reserve((2 * kept + 1) * sizeof(uint64_t)));
+        HB_CUDA_TRY(ctx->s_out.reserve(o.strings_capacity + 16));
+        o.field_kind = B.s_kind.as<uint8_t>();
+        o.field_index = B.s_index.as<uint64_t>();
+        o.never_indexed = B.s_never.as<uint8_t>();
+        o.string_offsets = B.s_string_offsets.as<uint64_t>();
+        o.strings = ctx->s_out.as<uint8_t>();
+    }
+    HB_CUDA_TRY(B.f_kind.reserve(parsed + 1));
+    HB_CUDA_TRY(B.f_index.reserve((parsed + 1) * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.f_block.reserve((parsed + 1) * sizeof(uint32_t)));
+    HB_CUDA_TRY(B.f_lits.reserve((2 * parsed + 1) * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.lit_src.reserve((num_lits + 1) * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.lit_len.reserve((num_lits + 1) * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.lit_offsets.reserve((num_lits + 1) * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.lit_status.reserve((num_lits + 1) * sizeof(int32_t)));
+    HB_CUDA_TRY(B.dec_offsets.reserve((num_lits + 1) * sizeof(uint64_t)));
+    uint8_t *f_kind = B.f_kind.as<uint8_t>();
+    uint64_t *f_index = B.f_index.as<uint64_t>(), *f_lits = B.f_lits.as<uint64_t>();
+    uint32_t *f_block = B.f_block.as<uint32_t>();
+    uint64_t *dec_offsets = B.dec_offsets.as<uint64_t>();
+    int32_t *lit_status = B.lit_status.as<int32_t>();
+
+    // 3. field records and literals in parsed order; 4. the literals, packed and re-framed as RFC 7541 5.2 literals;
+    // 5. decoded by the literal path
+    if (parsed || num_lits) {
+        hb::qpack_section_split_kernel<<<flat, 256, 0, st>>>(
+            n, in, in_off, field_base, lit_base, lit_byte_base, f_kind, f_index, f_block, f_lits, B.lit_src.as<uint64_t>(),
+            B.lit_len.as<uint64_t>(), B.lit_offsets.as<uint64_t>());
+        ++ctx->launches;
+    }
+    if (num_lits) {
+        HB_CUDA_TRY(B.lits.reserve(lit_total + 64));
+        HB_CUDA_TRY(B.dec.reserve(dec_cap + 64));
+        hb::qpack_lit_gather_kernel<<<grid_of(num_lits, 256), 256, 0, st>>>(
+            num_lits, in, B.lit_src.as<uint64_t>(), B.lit_len.as<uint64_t>(), B.lit_offsets.as<uint64_t>(), B.lits.as<uint8_t>());
+        ++ctx->launches;
+        if (hpack_decode_on_device(ctx, num_lits, B.lits.as<uint8_t>(), B.lit_offsets.as<uint64_t>(), lit_total,
+                                   B.dec.as<uint8_t>(), dec_cap, dec_offsets, lit_status, st))
+            return AWS_OP_ERR;
+    }
+    // 6. final status per section, its prefix, field offsets; 7. records, string lengths, string offsets, strings
+    hb::hpack_block_finish_kernel<<<flat, 256, 0, st>>>(
+        n, lit_base, lit_status, B.struct_status.as<int32_t>(), B.num_fields.as<uint64_t>(), status, B.out_fields.as<uint64_t>());
+    ++ctx->launches;
+    hb::qpack_section_prefix_kernel<<<flat, 256, 0, st>>>(n, in, in_off, status, o.encoded_insert_count, o.base_sign,
+                                                           o.delta_base);
+    ++ctx->launches;
+    if (launch_scan(ctx, ctx->scratch, B.out_fields.as<uint64_t>(), o.field_offsets, n, st)) return AWS_OP_ERR;
+    if (!kept) {
+        HB_CUDA_TRY(cudaMemsetAsync(o.string_offsets, 0, sizeof(uint64_t), st));
+        HB_CUDA_TRY(cudaGetLastError());
+        return AWS_OP_SUCCESS;
+    }
+    HB_CUDA_TRY(B.str_lens.reserve(2 * kept * sizeof(uint64_t)));
+    HB_CUDA_TRY(cudaMemsetAsync(B.str_lens.ptr, 0, 2 * kept * sizeof(uint64_t), st));
+    const uint8_t *dec = B.dec.as<uint8_t>();
+    hb::qpack_field_records_kernel<<<grid_of(parsed, 256), 256, 0, st>>>(
+        parsed, f_kind, f_index, f_block, f_lits, field_base, status, o.field_offsets, o.field_capacity, dec, dec_offsets,
+        o.field_kind, o.field_index, o.never_indexed, B.str_lens.as<uint64_t>());
+    ++ctx->launches;
+    if (launch_scan(ctx, ctx->scratch, B.str_lens.as<uint64_t>(), o.string_offsets, 2 * kept, st)) return AWS_OP_ERR;
+    hb::hpack_compose_kernel<hb::QpackFieldStrings><<<grid_of(2 * parsed, 256), 256, 0, st>>>(
+        parsed, f_kind, f_index, f_block, f_lits, field_base, status, o.field_offsets, o.field_capacity, dec, dec_offsets,
+        o.strings, o.strings_capacity, o.string_offsets);
+    ++ctx->launches;
+    HB_CUDA_TRY(cudaGetLastError());
+    return AWS_OP_SUCCESS;
+}
+
+// eic == NULL: stateless (aws_qpack_field_section_encode_batch: field_kind and field_index are NULL too); else the
+// caller's records and prefixes, with the per-section status (optional) of aws_qpack_field_section_encode_records_batch.
+int qpack_sections_encode_on_device(
+    aws_huffman_batch_ctx *ctx, uint64_t n, const uint64_t *field_offsets, uint64_t num_fields, const uint8_t *never_indexed,
+    const uint8_t *field_kind, const uint64_t *field_index, const uint64_t *eic, const uint8_t *sign, const uint64_t *delta,
+    const uint8_t *strings, const uint64_t *string_offsets, uint64_t strings_size, uint32_t mode, uint8_t *out,
+    uint64_t out_capacity, uint64_t *out_offsets, int32_t *status, cudaStream_t st) {
+    hb_host::BlockBufs &B = ctx->blk;
+    if (n == 0) {
+        HB_CUDA_TRY(cudaMemsetAsync(out_offsets, 0, sizeof(uint64_t), st));
+        return AWS_OP_SUCCESS;
+    }
+    const uint64_t F = num_fields;
+    HB_CUDA_TRY(B.sec_lens.reserve(n * sizeof(uint64_t)));
+    const uint64_t *framed_offsets = nullptr;
+    uint64_t *field_pos = nullptr;
+    // 1. every name and value framed; 2. line and size per field (sections without fields skip both)
+    if (F) {
+        const uint64_t expand = mode == hb::kHpackAlways ? (std::max<uint32_t>(1, ctx->tables.max_len) + 7) / 8 : 1;
+        const uint64_t framed_cap = strings_size * expand + 2 * F * 10 + 64;
+        HB_CUDA_TRY(B.framed.reserve(framed_cap + 64));
+        HB_CUDA_TRY(B.framed_offsets.reserve((2 * F + 1) * sizeof(uint64_t)));
+        HB_CUDA_TRY(B.plan.reserve(F));
+        HB_CUDA_TRY(B.plan_index.reserve(F * sizeof(uint64_t)));
+        HB_CUDA_TRY(B.field_lens.reserve(F * sizeof(uint64_t)));
+        HB_CUDA_TRY(B.field_pos.reserve((F + 1) * sizeof(uint64_t)));
+        framed_offsets = B.framed_offsets.as<uint64_t>();
+        field_pos = B.field_pos.as<uint64_t>();
+        if (hpack_encode_on_device(ctx, 2 * F, strings, string_offsets, strings_size, mode, B.framed.as<uint8_t>(), framed_cap,
+                                   B.framed_offsets.as<uint64_t>(), st))
+            return AWS_OP_ERR;
+        hb::qpack_field_plan_kernel<<<grid_of(F, 256), 256, 0, st>>>(
+            F, strings, string_offsets, never_indexed, field_kind, field_index, B.framed.as<uint8_t>(), framed_offsets,
+            B.plan.as<uint8_t>(), B.plan_index.as<uint64_t>(), B.field_lens.as<uint64_t>());
+        ++ctx->launches;
+    }
+    // 3. the section rules and sizes (prefix included); 4. wire positions of sections and fields; 5. prefixes, and
+    // the fields placed behind them; 6. the lines
+    hb::qpack_section_size_kernel<<<grid_of(n, 256), 256, 0, st>>>(
+        n, field_offsets, eic, sign, delta, B.plan.as<uint8_t>(), B.field_lens.as<uint64_t>(), status, B.sec_lens.as<uint64_t>());
+    ++ctx->launches;
+    if (launch_scan(ctx, ctx->scratch, B.sec_lens.as<uint64_t>(), out_offsets, n, st)) return AWS_OP_ERR;
+    if (F && launch_scan(ctx, ctx->scratch, B.field_lens.as<uint64_t>(), field_pos, F, st)) return AWS_OP_ERR;
+    hb::qpack_section_place_kernel<<<grid_of(n, 256), 256, 0, st>>>(n, field_offsets, eic, sign, delta, out_offsets,
+                                                                     field_pos, out, out_capacity);
+    ++ctx->launches;
+    if (F) {
+        hb::qpack_field_emit_kernel<<<grid_of(F, 256), 256, 0, st>>>(
+            F, B.plan.as<uint8_t>(), B.plan_index.as<uint64_t>(), B.framed.as<uint8_t>(), framed_offsets, field_pos, out,
+            out_capacity);
+        ++ctx->launches;
+    }
+    HB_CUDA_TRY(cudaGetLastError());
+    return AWS_OP_SUCCESS;
+}
+
+// The argument rules of check_block_lists, and the prefix arrays: written by a decode, read by a records encode.
+int check_section_lists(const aws_qpack_field_sections *l, bool decode, bool records) {
+    if (!l || (l->n && !l->field_offsets) || !l->string_offsets || l->n > 0xffffffffull)
+        return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    if (decode && ((l->field_capacity && (!l->field_kind || !l->field_index || !l->never_indexed)) ||
+                   (l->strings_capacity && !l->strings)))
+        return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    if ((decode || records) && l->n && (!l->encoded_insert_count || !l->base_sign || !l->delta_base))
+        return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    if (records && (!l->field_kind || !l->field_index)) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    return AWS_OP_SUCCESS;
+}
+
+// Host pointers, run on the device (the way hpack_blocks_decode_slice does): the n sections are staged and decoded into
+// the context's staging, within the capacities given; size[0] receives their fields and, when those fit
+// field_capacity, size[1] their string octets.
+int qpack_sections_decode_slice(
+    aws_huffman_batch_ctx *ctx, size_t n, const uint8_t *in, const uint64_t *in_off, uint64_t field_capacity,
+    uint64_t strings_capacity, uint64_t size[2], cudaStream_t st) {
+    hb_host::BlockBufs &B = ctx->blk;
+    const uint64_t total_in = in_off[n];
+    const uint8_t *d_in = nullptr;
+    uint64_t *d_in_off = nullptr;
+    if (stage_in(ctx->s_in, total_in + 16, in, total_in, st, &d_in) ||
+        stage_in(ctx->s_in_off, (n + 1) * sizeof(uint64_t), in_off, n + 1, st, &d_in_off))
+        return AWS_OP_ERR;
+    aws_qpack_field_sections o{};
+    o.n = n;
+    o.field_capacity = field_capacity;
+    o.strings_capacity = strings_capacity;
+    if (stage_in(B.s_field_offsets, (n + 1) * sizeof(uint64_t), (const uint64_t *)nullptr, 0, st, &o.field_offsets) ||
+        stage_in(B.s_eic, n * sizeof(uint64_t), (const uint64_t *)nullptr, 0, st, &o.encoded_insert_count) ||
+        stage_in(B.s_sign, n, (const uint8_t *)nullptr, 0, st, &o.base_sign) ||
+        stage_in(B.s_delta, n * sizeof(uint64_t), (const uint64_t *)nullptr, 0, st, &o.delta_base))
+        return AWS_OP_ERR;
+    HB_CUDA_TRY(ctx->s_status.reserve(n * sizeof(int32_t)));
+    if (qpack_sections_decode_on_device(ctx, n, d_in, d_in_off, o, ctx->s_status.as<int32_t>(), true, st) ||
+        read_back(o.field_offsets + n, &size[0], st))
+        return AWS_OP_ERR;
+    size[1] = 0;  // (string offsets exist for the fields that fit)
+    return size[0] <= field_capacity ? read_back(B.s_string_offsets.as<uint64_t>() + 2 * size[0], &size[1], st) : AWS_OP_SUCCESS;
+}
+
+// Host pointers, finish into place: prefixes, offsets and status first (complete on AWS_ERROR_SHORT_BUFFER), then the
+// records and strings.
+int qpack_sections_decode_finish(
+    aws_huffman_batch_ctx *ctx, size_t n, const uint64_t size[2], aws_qpack_field_sections *out, int32_t *status,
+    cudaStream_t st) {
+    hb_host::BlockBufs &B = ctx->blk;
+    const uint64_t fields = size[0];
+    HB_CUDA_TRY(cudaMemcpyAsync(out->encoded_insert_count, B.s_eic.ptr, n * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    HB_CUDA_TRY(cudaMemcpyAsync(out->base_sign, B.s_sign.ptr, n, cudaMemcpyDeviceToHost, st));
+    HB_CUDA_TRY(cudaMemcpyAsync(out->delta_base, B.s_delta.ptr, n * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    if (finish_slice(ctx, st, n, true, B.s_field_offsets.as<uint64_t>(), out->field_offsets, 0, nullptr, nullptr, 0, fields,
+                     out->field_capacity, ctx->s_status.as<int32_t>(), status) ||
+        finish_slice(ctx, st, 2 * fields, true, B.s_string_offsets.as<uint64_t>(), out->string_offsets, 0, ctx->s_out.ptr,
+                     out->strings, size[1], size[1], out->strings_capacity))
+        return AWS_OP_ERR;
+    if (fields) {
+        HB_CUDA_TRY(cudaMemcpyAsync(out->field_kind, B.s_kind.ptr, fields, cudaMemcpyDeviceToHost, st));
+        HB_CUDA_TRY(cudaMemcpyAsync(out->field_index, B.s_index.ptr, fields * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+        HB_CUDA_TRY(cudaMemcpyAsync(out->never_indexed, B.s_never.ptr, fields, cudaMemcpyDeviceToHost, st));
+    }
+    HB_CUDA_TRY(cudaStreamSynchronize(st));
+    return AWS_OP_SUCCESS;
+}
+
+// Arguments of the host-pointer decode call; a call with no sections is answered here (*done).
+int qpack_sections_decode_args(size_t n, const uint8_t *in, const uint64_t *in_off, aws_qpack_field_sections *out, bool *done) {
+    *done = false;
+    if ((n && !in_off) || check_section_lists(out, true, false) || out->n != n) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    if (n == 0) {
+        out->field_offsets[0] = 0;
+        out->string_offsets[0] = 0;
+        *done = true;
+        return AWS_OP_SUCCESS;
+    }
+    if ((in_off[n] && !in) || !offsets_sorted(in_off, n + 1)) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    return AWS_OP_SUCCESS;
+}
+
+int qpack_sections_decode_host(
+    aws_huffman_batch_ctx *ctx, size_t n, const uint8_t *in, const uint64_t *in_off, aws_qpack_field_sections *out,
+    int32_t *status) {
+    bool done;
+    if (!ctx) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    if (qpack_sections_decode_args(n, in, in_off, out, &done) || done) return done ? AWS_OP_SUCCESS : AWS_OP_ERR;
+    cudaStream_t st;
+    if (call_begin(ctx, nullptr, &st)) return AWS_OP_ERR;
+    uint64_t size[2];
+    int rc = qpack_sections_decode_slice(ctx, n, in, in_off, out->field_capacity, out->strings_capacity, size, st);
+    if (rc == AWS_OP_SUCCESS) rc = qpack_sections_decode_finish(ctx, n, size, out, status, st);
+    return call_end(ctx, st, rc);
+}
+
+// Host pointers, run on the device: the sections of `in` are staged and encoded into the context's staging,
+// out_capacity octets at most; *size receives the output size. records: the kinds, indices and prefixes are read
+// (aws_qpack_field_section_encode_records_batch) and a status per section is written to the staging.
+int qpack_sections_encode_slice(
+    aws_huffman_batch_ctx *ctx, const aws_qpack_field_sections *in, bool records, uint32_t mode, uint64_t out_capacity,
+    uint64_t *size, cudaStream_t st) {
+    hb_host::BlockBufs &B = ctx->blk;
+    const uint64_t n = in->n, F = in->field_offsets[n], S = in->string_offsets[2 * F];
+    uint64_t *d_field_offsets = nullptr, *d_string_offsets = nullptr;
+    const uint8_t *d_strings = nullptr, *never = nullptr, *kind = nullptr, *sign = nullptr;
+    const uint64_t *index = nullptr, *eic = nullptr, *delta = nullptr;
+    int32_t *d_status = nullptr;
+    if (records) {
+        HB_CUDA_TRY(ctx->s_status.reserve(n * sizeof(int32_t)));
+        d_status = ctx->s_status.as<int32_t>();
+    }
+    if (stage_in(B.s_field_offsets, (n + 1) * sizeof(uint64_t), in->field_offsets, n + 1, st, &d_field_offsets) ||
+        stage_in(ctx->s_in, S + 16, in->strings, S, st, &d_strings) ||
+        stage_in(ctx->s_in_off, (2 * F + 1) * sizeof(uint64_t), in->string_offsets, 2 * F + 1, st, &d_string_offsets) ||
+        (in->never_indexed && F && stage_in(B.s_never, F, in->never_indexed, F, st, &never)) ||
+        (records && (stage_in(B.s_kind, F + 1, in->field_kind, F, st, &kind) ||
+                     stage_in(B.s_index, (F + 1) * sizeof(uint64_t), in->field_index, F, st, &index) ||
+                     stage_in(B.s_eic, n * sizeof(uint64_t), in->encoded_insert_count, n, st, &eic) ||
+                     stage_in(B.s_sign, n, in->base_sign, n, st, &sign) ||
+                     stage_in(B.s_delta, n * sizeof(uint64_t), in->delta_base, n, st, &delta))))
+        return AWS_OP_ERR;
+    HB_CUDA_TRY(ctx->s_out.reserve(out_capacity + 16));
+    HB_CUDA_TRY(ctx->s_out_off.reserve((n + 1) * sizeof(uint64_t)));
+    if (qpack_sections_encode_on_device(ctx, n, d_field_offsets, F, never, kind, index, eic, sign, delta, d_strings,
+                                        d_string_offsets, S, mode, ctx->s_out.as<uint8_t>(), out_capacity,
+                                        ctx->s_out_off.as<uint64_t>(), d_status, st))
+        return AWS_OP_ERR;
+    return read_back(ctx->s_out_off.as<uint64_t>() + n, size, st);
+}
+
+// Arguments of the host-pointer encode calls (those of hpack_blocks_encode_args); a call with no sections is answered
+// here (*done).
+int qpack_sections_encode_args(const aws_qpack_field_sections *in, bool records, const uint8_t *out, uint64_t out_capacity,
+                               uint64_t *out_off, bool *done) {
+    *done = false;
+    if (check_section_lists(in, false, records) || !out_off || (out_capacity && !out))
+        return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    const uint64_t n = in->n;
+    if (n == 0) {
+        out_off[0] = 0;
+        *done = true;
+        return AWS_OP_SUCCESS;
+    }
+    if (in->field_offsets[0] != 0 || !offsets_sorted(in->field_offsets, n + 1)) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    const uint64_t F = in->field_offsets[n];
+    if (in->string_offsets[0] != 0 || !offsets_sorted(in->string_offsets, 2 * F + 1))
+        return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    if (in->string_offsets[2 * F] && !in->strings) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    return AWS_OP_SUCCESS;
+}
+
+int qpack_sections_encode_host(
+    aws_huffman_batch_ctx *ctx, const aws_qpack_field_sections *in, bool records, uint32_t mode, uint8_t *out,
+    uint64_t out_capacity, uint64_t *out_off, int32_t *status) {
+    bool done;
+    if (!ctx || mode > hb::kHpackAlways) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    if (qpack_sections_encode_args(in, records, out, out_capacity, out_off, &done) || done)
+        return done ? AWS_OP_SUCCESS : AWS_OP_ERR;
+    cudaStream_t st;
+    if (call_begin(ctx, nullptr, &st)) return AWS_OP_ERR;
+    uint64_t size = 0;
+    int rc = qpack_sections_encode_slice(ctx, in, records, mode, out_capacity, &size, st);
+    if (rc == AWS_OP_SUCCESS &&
+        (finish_slice(ctx, st, in->n, true, ctx->s_out_off.as<uint64_t>(), out_off, 0, ctx->s_out.ptr, out, size, size,
+                      out_capacity, records ? ctx->s_status.as<int32_t>() : nullptr, status) ||
+         cudaStreamSynchronize(st) != cudaSuccess))
+        rc = AWS_OP_ERR;
+    return call_end(ctx, st, rc);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -2200,6 +2553,67 @@ int aws_hpack_header_block_encode_records_batch_device(
                                                          in->field_kind, in->field_index, in->strings, in->string_offsets,
                                                          strings_size, (uint32_t)mode, out, out_capacity, out_offsets, status,
                                                          st));
+}
+
+int aws_qpack_field_section_decode_batch(
+    struct aws_huffman_batch_ctx *ctx, size_t n, const uint8_t *in, const uint64_t *in_offsets,
+    struct aws_qpack_field_sections *out, int32_t *status) {
+    return qpack_sections_decode_host(ctx, n, in, in_offsets, out, status);
+}
+
+int aws_qpack_field_section_encode_batch(
+    struct aws_huffman_batch_ctx *ctx, const struct aws_qpack_field_sections *in, enum aws_hpack_huffman_mode mode,
+    uint8_t *out, uint64_t out_capacity, uint64_t *out_offsets) {
+    return qpack_sections_encode_host(ctx, in, false, (uint32_t)mode, out, out_capacity, out_offsets, nullptr);
+}
+
+int aws_qpack_field_section_encode_records_batch(
+    struct aws_huffman_batch_ctx *ctx, const struct aws_qpack_field_sections *in, enum aws_hpack_huffman_mode mode,
+    uint8_t *out, uint64_t out_capacity, uint64_t *out_offsets, int32_t *status) {
+    return qpack_sections_encode_host(ctx, in, true, (uint32_t)mode, out, out_capacity, out_offsets, status);
+}
+
+int aws_qpack_field_section_decode_batch_device(
+    struct aws_huffman_batch_ctx *ctx, size_t n, const uint8_t *in, const uint64_t *in_offsets, uint64_t in_size,
+    struct aws_qpack_field_sections *out, int32_t *status, void *cuda_stream) {
+    if (!ctx || (n && !in_offsets) || (in_size && !in) || check_section_lists(out, true, false) || out->n != n)
+        return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    cudaStream_t st;
+    if (call_begin(ctx, cuda_stream, &st)) return AWS_OP_ERR;
+    return call_end(ctx, st, qpack_sections_decode_on_device(ctx, n, in, in_offsets, *out, status, false, st));
+}
+
+int aws_qpack_field_section_encode_batch_device(
+    struct aws_huffman_batch_ctx *ctx, const struct aws_qpack_field_sections *in, uint64_t num_fields,
+    uint64_t strings_size, enum aws_hpack_huffman_mode mode, uint8_t *out, uint64_t out_capacity, uint64_t *out_offsets,
+    void *cuda_stream) {
+    if (!ctx || check_section_lists(in, false, false) || !out_offsets || (out_capacity && !out) ||
+        (strings_size && !in->strings) || (unsigned)mode > (unsigned)AWS_HPACK_HUFFMAN_ALWAYS)
+        return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    cudaStream_t st;
+    if (call_begin(ctx, cuda_stream, &st)) return AWS_OP_ERR;
+    return call_end(ctx, st,
+                    qpack_sections_encode_on_device(ctx, in->n, in->field_offsets, num_fields, in->never_indexed, nullptr,
+                                                    nullptr, nullptr, nullptr, nullptr, in->strings, in->string_offsets,
+                                                    strings_size, (uint32_t)mode, out, out_capacity, out_offsets, nullptr,
+                                                    st));
+}
+
+int aws_qpack_field_section_encode_records_batch_device(
+    struct aws_huffman_batch_ctx *ctx, const struct aws_qpack_field_sections *in, uint64_t num_fields,
+    uint64_t strings_size, enum aws_hpack_huffman_mode mode, uint8_t *out, uint64_t out_capacity, uint64_t *out_offsets,
+    int32_t *status, void *cuda_stream) {
+    if (!ctx || check_section_lists(in, false, true) || !out_offsets || (out_capacity && !out) ||
+        (strings_size && !in->strings) || (unsigned)mode > (unsigned)AWS_HPACK_HUFFMAN_ALWAYS)
+        return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    cudaStream_t st;
+    if (call_begin(ctx, cuda_stream, &st)) return AWS_OP_ERR;
+    return call_end(ctx, st,
+                    qpack_sections_encode_on_device(ctx, in->n, in->field_offsets, num_fields, in->never_indexed,
+                                                    in->field_kind, in->field_index, in->encoded_insert_count,
+                                                    in->base_sign, in->delta_base, in->strings, in->string_offsets,
+                                                    strings_size, (uint32_t)mode, out, out_capacity, out_offsets, status,
+                                                    st));
 }
 
 int aws_huffman_get_encoded_length_batch(

@@ -33,8 +33,11 @@ _spec.loader.exec_module(_blk)
 CUSTOM_NAMES = [b"x-custom-header-%02d" % i for i in range(32)]
 
 
-def synthetic_lists(n, seed, dev):
-    """(field_offsets, strings, string_offsets, never_indexed) as device tensors (int64 offsets, uint8 data)."""
+def synthetic_lists(n, seed, dev, static_table=None):
+    """(field_offsets, strings, string_offsets, never_indexed) as device tensors (int64 offsets, uint8 data).
+    static_table: the (name, value) entries of the exact and name matches (default: RFC 7541 Appendix A)."""
+    static_table = _blk.STATIC_TABLE if static_table is None else static_table
+    entries = len(static_table)
     g = torch.Generator(device=dev)
     g.manual_seed(seed)
     counts = torch.randint(8, 25, (n,), generator=g, device=dev)
@@ -43,20 +46,20 @@ def synthetic_lists(n, seed, dev):
     F = int(fo[-1].item())
     # a pool of fixed strings: the static names and values, then the custom names
     pool, starts, lens = b"", [], []
-    for s in [x for entry in _blk.STATIC_TABLE for x in entry] + CUSTOM_NAMES:
+    for s in [x for entry in static_table for x in entry] + CUSTOM_NAMES:
         starts.append(len(pool))
         lens.append(len(s))
         pool += s
     pool_t = torch.frombuffer(bytearray(pool), dtype=torch.uint8).to(dev)
     p_start = torch.tensor(starts, dtype=torch.int64, device=dev)
     p_len = torch.tensor(lens, dtype=torch.int64, device=dev)
-    with_value = torch.tensor([i for i, (_, v) in enumerate(_blk.STATIC_TABLE) if v], dtype=torch.int64, device=dev)
+    with_value = torch.tensor([i for i, (_, v) in enumerate(static_table) if v], dtype=torch.int64, device=dev)
     r = torch.rand(F, generator=g, device=dev)
     exact = r < 0.25
     custom = r >= 0.70
     entry = torch.where(exact, with_value[torch.randint(0, with_value.numel(), (F,), generator=g, device=dev)],
-                        torch.randint(0, 61, (F,), generator=g, device=dev))
-    name_id = torch.where(custom, 122 + torch.randint(0, 32, (F,), generator=g, device=dev), 2 * entry)
+                        torch.randint(0, entries, (F,), generator=g, device=dev))
+    name_id = torch.where(custom, 2 * entries + torch.randint(0, 32, (F,), generator=g, device=dev), 2 * entry)
     value_len = torch.where(exact, p_len[2 * entry + 1], torch.randint(8, 257, (F,), generator=g, device=dev))
     lens2 = torch.stack([p_len[name_id], value_len], 1).reshape(-1)
     so = torch.zeros(2 * F + 1, dtype=torch.int64, device=dev)
