@@ -21,6 +21,11 @@ HPACK_HUFFMAN_SMALLEST, HPACK_HUFFMAN_NEVER, HPACK_HUFFMAN_ALWAYS = 0, 1, 2
 # enum aws_qpack_field_kind
 (QPACK_FIELD_INDEXED_STATIC, QPACK_FIELD_INDEXED_DYNAMIC, QPACK_FIELD_INDEXED_POST_BASE, QPACK_FIELD_NAME_REF_STATIC,
  QPACK_FIELD_NAME_REF_DYNAMIC, QPACK_FIELD_NAME_REF_POST_BASE, QPACK_FIELD_LITERAL_NAME, QPACK_FIELD_AUTO) = range(8)
+# enum aws_qpack_instruction_stream, enum aws_qpack_instruction_kind
+QPACK_ENCODER_STREAM, QPACK_DECODER_STREAM = 0, 1
+(QPACK_INSERT_NAME_REF_STATIC, QPACK_INSERT_NAME_REF_DYNAMIC, QPACK_INSERT_LITERAL_NAME, QPACK_DUPLICATE,
+ QPACK_SET_CAPACITY, QPACK_SECTION_ACKNOWLEDGMENT, QPACK_STREAM_CANCELLATION, QPACK_INSERT_COUNT_INCREMENT,
+ QPACK_INSERT_AUTO) = range(9)
 
 
 class CodecError(RuntimeError):
@@ -115,6 +120,19 @@ class aws_qpack_field_sections(C.Structure):
     ]
 
 
+class aws_qpack_instructions(C.Structure):
+    _fields_ = [
+        ("n", C.c_size_t),
+        ("instruction_offsets", C.c_void_p),
+        ("instruction_capacity", C.c_uint64),
+        ("kind", C.c_void_p),
+        ("index", C.c_void_p),
+        ("strings", C.c_void_p),
+        ("strings_capacity", C.c_uint64),
+        ("string_offsets", C.c_void_p),
+    ]
+
+
 class aws_huffman_table_coder(C.Structure):
     _fields_ = [("coder", aws_huffman_symbol_coder), ("codes", aws_huffman_code * 256),
                 ("lut_entries", C.c_void_p), ("lut_count", C.c_uint32), ("lut_root_bits", C.c_uint8)]
@@ -174,6 +192,8 @@ EXPORTED_SYMBOLS = [
     "aws_qpack_field_section_decode_batch", "aws_qpack_field_section_encode_batch",
     "aws_qpack_field_section_encode_records_batch", "aws_qpack_field_section_decode_batch_device",
     "aws_qpack_field_section_encode_batch_device", "aws_qpack_field_section_encode_records_batch_device",
+    "aws_qpack_instruction_decode_batch", "aws_qpack_instruction_encode_batch",
+    "aws_qpack_instruction_decode_batch_device", "aws_qpack_instruction_encode_batch_device",
 ]
 
 
@@ -303,6 +323,15 @@ class Library:
                                                             C.c_void_p, C.c_void_p],
             "aws_qpack_field_section_encode_records_batch_device": [Q, C.c_uint64, C.c_uint64, C.c_int, C.c_void_p,
                                                                     C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p],
+            "aws_qpack_instruction_decode_batch": [C.c_int, C.c_size_t, C.c_void_p, C.c_void_p, P(aws_qpack_instructions),
+                                                   C.c_void_p, C.c_void_p],
+            "aws_qpack_instruction_encode_batch": [C.c_int, P(aws_qpack_instructions), C.c_int, C.c_void_p, C.c_uint64,
+                                                   C.c_void_p, C.c_void_p],
+            "aws_qpack_instruction_decode_batch_device": [C.c_int, C.c_size_t, C.c_void_p, C.c_void_p, C.c_uint64,
+                                                          P(aws_qpack_instructions), C.c_void_p, C.c_void_p, C.c_void_p],
+            "aws_qpack_instruction_encode_batch_device": [C.c_int, P(aws_qpack_instructions), C.c_uint64, C.c_uint64,
+                                                          C.c_int, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p,
+                                                          C.c_void_p],
         }
         for name, args in qpack.items():
             getattr(L, name).argtypes = [C.c_void_p] + args
@@ -800,6 +829,76 @@ class BatchContext:
         else:
             self._blocks_call("aws_qpack_field_section_encode_records_batch_device", C.byref(sections), int(num_fields),
                               int(strings_size), mode, _ptr(out), cap, _ptr(out_offsets), _ptr(status), stream or 0)
+
+    # ---- QPACK encoder- and decoder-stream instructions (qpack_instruction_batch.h) ----
+    def qpack_decode_instructions(self, which, data, in_offsets, instruction_capacity=None, strings_capacity=None):
+        """Host buffers. Capacities default to the documented bounds (in_size instructions, 14 * in_size octets). On
+        failure the CodecError carries the arrays as `result` (offsets, consumed and status are complete on
+        AWS_ERROR_SHORT_BUFFER)."""
+        data = np.ascontiguousarray(data, dtype=np.uint8)
+        in_offsets = np.ascontiguousarray(in_offsets, dtype=np.uint64)
+        n = len(in_offsets) - 1
+        in_size = int(in_offsets[-1])
+        cap = in_size if instruction_capacity is None else int(instruction_capacity)
+        strings_capacity = 14 * in_size if strings_capacity is None else int(strings_capacity)
+        res = {"instruction_offsets": np.zeros(n + 1, dtype=np.uint64), "kind": np.zeros(max(cap, 1), np.uint8),
+               "index": np.zeros(max(cap, 1), np.uint64), "strings": np.zeros(max(strings_capacity, 1), np.uint8),
+               "string_offsets": np.zeros(2 * cap + 1, np.uint64), "consumed": np.zeros(n, np.uint64),
+               "status": np.zeros(n, np.int32)}
+        instr = aws_qpack_instructions(n, _ptr(res["instruction_offsets"]), cap, _ptr(res["kind"]), _ptr(res["index"]),
+                                       _ptr(res["strings"]), strings_capacity, _ptr(res["string_offsets"]))
+        try:
+            self._blocks_call("aws_qpack_instruction_decode_batch", which, n, _ptr(data), _ptr(in_offsets),
+                              C.byref(instr), _ptr(res["consumed"]), _ptr(res["status"]))
+        except CodecError as err:
+            err.result = res
+            raise
+        return res
+
+    def qpack_encode_instructions(self, which, instruction_offsets, kind, index, strings, string_offsets, out_capacity,
+                                  mode=HPACK_HUFFMAN_SMALLEST):
+        """Host buffers: instruction records in, chunks of the stream `which` out ({"out", "out_offsets", "status"}).
+        On failure the CodecError carries them as `result`."""
+        instruction_offsets = np.ascontiguousarray(instruction_offsets, dtype=np.uint64)
+        kind = np.ascontiguousarray(kind, dtype=np.uint8)
+        index = np.ascontiguousarray(index, dtype=np.uint64)
+        strings = np.ascontiguousarray(strings, dtype=np.uint8)
+        string_offsets = np.ascontiguousarray(string_offsets, dtype=np.uint64)
+        n = len(instruction_offsets) - 1
+        res = {"out": np.zeros(max(int(out_capacity), 1), dtype=np.uint8), "out_offsets": np.zeros(n + 1, dtype=np.uint64),
+               "status": np.full(n, -1, dtype=np.int32)}
+        instr = aws_qpack_instructions(n, _ptr(instruction_offsets), 0, _ptr(kind), _ptr(index), _ptr(strings), 0,
+                                       _ptr(string_offsets))
+        try:
+            self._blocks_call("aws_qpack_instruction_encode_batch", which, C.byref(instr), mode, _ptr(res["out"]),
+                              int(out_capacity), _ptr(res["out_offsets"]), _ptr(res["status"]))
+        except CodecError as err:
+            err.result = res
+            raise
+        return res
+
+    def qpack_decode_instructions_device(self, which, n, in_, in_offsets, in_size, instruction_offsets, kind, index,
+                                         strings, string_offsets, consumed, status=None, stream=None,
+                                         instruction_capacity=None, strings_capacity=None):
+        """Device pointers (torch CUDA tensors, or objects with data_ptr()); capacities default to the tensors' sizes
+        (instruction_capacity: (string_offsets.numel() - 1) // 2; strings None: capacity 0)."""
+        cap = (string_offsets.numel() - 1) // 2 if instruction_capacity is None else int(instruction_capacity)
+        if strings_capacity is None:
+            strings_capacity = strings.numel() if strings is not None else 0
+        instr = aws_qpack_instructions(n, _ptr(instruction_offsets), cap, _ptr(kind), _ptr(index), _ptr(strings),
+                                       int(strings_capacity), _ptr(string_offsets))
+        self._blocks_call("aws_qpack_instruction_decode_batch_device", which, n, _ptr(in_), _ptr(in_offsets),
+                          int(in_size), C.byref(instr), _ptr(consumed), _ptr(status), stream or 0)
+
+    def qpack_encode_instructions_device(self, which, n, instruction_offsets, num_instructions, kind, index, strings,
+                                         string_offsets, strings_size, out, out_offsets, status=None,
+                                         mode=HPACK_HUFFMAN_SMALLEST, out_capacity=None, stream=None):
+        """Device pointers; out_capacity defaults to out.numel()."""
+        instr = aws_qpack_instructions(n, _ptr(instruction_offsets), 0, _ptr(kind), _ptr(index), _ptr(strings), 0,
+                                       _ptr(string_offsets))
+        cap = out.numel() if out_capacity is None else int(out_capacity)
+        self._blocks_call("aws_qpack_instruction_encode_batch_device", which, C.byref(instr), int(num_instructions),
+                          int(strings_size), mode, _ptr(out), cap, _ptr(out_offsets), _ptr(status), stream or 0)
 
     def encode(self, data, in_offsets, out_capacity, **kw):
         return self._host(True, data, in_offsets, out_capacity, **kw)

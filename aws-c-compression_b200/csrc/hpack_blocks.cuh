@@ -272,7 +272,18 @@ __device__ __forceinline__ uint64_t hpack_out_field(
     return o < field_capacity ? o : ~0ull;
 }
 
-// Thread per parsed field: the record and the lengths of its two strings.
+// The string source of HPACK fields for hpack_field_records_kernel and hpack_compose_kernel (qpack_sections.cuh and
+// qpack_instructions.cuh have QPACK's).
+struct HpackFieldStrings {
+    __device__ static void get(uint8_t kind, uint64_t index, uint64_t lit, uint32_t which, const uint8_t *dec,
+                               const uint64_t *dec_offsets, const uint8_t *&src, uint64_t &len) {
+        hpack_field_string(kind, index, lit, which, dec, dec_offsets, src, len);
+    }
+};
+
+// Thread per parsed field: the record and the lengths of its two strings (Strings::get says where a string of a
+// parsed field comes from).
+template <typename Strings>
 __global__ void hpack_field_records_kernel(
     uint64_t num_parsed, const uint8_t *f_kind, const uint64_t *f_index, const uint32_t *f_block, const uint64_t *f_lits,
     const uint64_t *field_base, const int32_t *status, const uint64_t *field_offsets, uint64_t field_capacity,
@@ -288,18 +299,10 @@ __global__ void hpack_field_records_kernel(
     for (uint32_t w = 0; w < 2; ++w) {
         const uint8_t *src;
         uint64_t len;
-        hpack_field_string(kind, index, f_lits[2 * f + w], w, dec, dec_offsets, src, len);
+        Strings::get(kind, index, f_lits[2 * f + w], w, dec, dec_offsets, src, len);
         str_lens[2 * o + w] = len;
     }
 }
-
-// The string source of HPACK fields for hpack_compose_kernel (qpack_sections.cuh has QPACK's).
-struct HpackFieldStrings {
-    __device__ static void get(uint8_t kind, uint64_t index, uint64_t lit, uint32_t which, const uint8_t *dec,
-                               const uint64_t *dec_offsets, const uint8_t *&src, uint64_t &len) {
-        hpack_field_string(kind, index, lit, which, dec, dec_offsets, src, len);
-    }
-};
 
 // The strings: item i is string i & 1 (name, value) of parsed field i >> 1. 32 strings per warp. Strings::get says
 // where a string of a parsed field comes from.

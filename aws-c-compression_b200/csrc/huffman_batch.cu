@@ -8,6 +8,7 @@
 #include <aws/compression/hpack_string_batch.h>
 #include <aws/compression/hpack_header_block_batch.h>
 #include <aws/compression/qpack_field_section_batch.h>
+#include <aws/compression/qpack_instruction_batch.h>
 #include <aws/compression/huffman_table_builder.h>
 
 #include "../host/huffman_lut.h"
@@ -19,6 +20,7 @@
 #include "hpack_literals.cuh"
 #include "hpack_blocks.cuh"
 #include "qpack_sections.cuh"
+#include "qpack_instructions.cuh"
 #include "decode_fast.cuh"
 
 #include <algorithm>
@@ -1229,7 +1231,7 @@ int hpack_blocks_decode_on_device(
     HB_CUDA_TRY(B.str_lens.reserve(2 * kept * sizeof(uint64_t)));
     HB_CUDA_TRY(cudaMemsetAsync(B.str_lens.ptr, 0, 2 * kept * sizeof(uint64_t), st));
     const uint8_t *dec = B.dec.as<uint8_t>();
-    hb::hpack_field_records_kernel<<<grid_of(parsed, 256), 256, 0, st>>>(
+    hb::hpack_field_records_kernel<hb::HpackFieldStrings><<<grid_of(parsed, 256), 256, 0, st>>>(
         parsed, f_kind, f_index, f_block, f_lits, field_base, status, o.field_offsets, o.field_capacity, dec, dec_offsets,
         o.kind, o.index, B.str_lens.as<uint64_t>());
     ++ctx->launches;
@@ -1657,7 +1659,7 @@ int qpack_sections_encode_on_device(
                                                                      field_pos, out, out_capacity);
     ++ctx->launches;
     if (F) {
-        hb::qpack_field_emit_kernel<<<grid_of(F, 256), 256, 0, st>>>(
+        hb::qpack_field_emit_kernel<hb::QpackFieldLines><<<grid_of(F, 256), 256, 0, st>>>(
             F, B.plan.as<uint8_t>(), B.plan_index.as<uint64_t>(), B.framed.as<uint8_t>(), framed_offsets, field_pos, out,
             out_capacity);
         ++ctx->launches;
@@ -1831,6 +1833,319 @@ int qpack_sections_encode_host(
     if (rc == AWS_OP_SUCCESS &&
         (finish_slice(ctx, st, in->n, true, ctx->s_out_off.as<uint64_t>(), out_off, 0, ctx->s_out.ptr, out, size, size,
                       out_capacity, records ? ctx->s_status.as<int32_t>() : nullptr, status) ||
+         cudaStreamSynchronize(st) != cudaSuccess))
+        rc = AWS_OP_ERR;
+    return call_end(ctx, st, rc);
+}
+
+// ---------------------------------------------------------------------------------------------
+// QPACK encoder- and decoder-stream instructions (qpack_instructions.cuh) over the passes and buffers of the field
+// sections above. Device pointers in, device pointers out.
+// ---------------------------------------------------------------------------------------------
+// stage: `o` holds instruction_offsets (context staging) and the capacities; the per-instruction outputs go to context
+// staging sized from the totals (the host entry point copies them back).
+int qpack_instructions_decode_on_device(
+    aws_huffman_batch_ctx *ctx, uint32_t which, uint64_t n, const uint8_t *in, const uint64_t *in_off,
+    aws_qpack_instructions o, uint64_t *consumed, int32_t *status, bool stage, cudaStream_t st) {
+    hb_host::BlockBufs &B = ctx->blk;
+    if (n == 0) {
+        HB_CUDA_TRY(cudaMemsetAsync(o.instruction_offsets, 0, sizeof(uint64_t), st));
+        if (o.string_offsets && !stage) HB_CUDA_TRY(cudaMemsetAsync(o.string_offsets, 0, sizeof(uint64_t), st));
+        return AWS_OP_SUCCESS;
+    }
+    const unsigned flat = grid_of(n, 256);
+    HB_CUDA_TRY(B.num_fields.reserve(n * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.num_lits.reserve(n * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.lit_bytes.reserve(n * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.out_fields.reserve(n * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.struct_status.reserve(n * sizeof(int32_t)));
+    HB_CUDA_TRY(B.field_base.reserve((n + 1) * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.lit_base.reserve((n + 1) * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.lit_byte_base.reserve((n + 1) * sizeof(uint64_t)));
+    if (!status) {
+        HB_CUDA_TRY(B.status.reserve(n * sizeof(int32_t)));
+        status = B.status.as<int32_t>();
+    }
+    if (!B.h_totals) HB_CUDA_TRY(cudaHostAlloc(reinterpret_cast<void **>(&B.h_totals), 3 * sizeof(uint64_t), cudaHostAllocDefault));
+    uint64_t *instr_base = B.field_base.as<uint64_t>(), *lit_base = B.lit_base.as<uint64_t>();
+    uint64_t *lit_byte_base = B.lit_byte_base.as<uint64_t>();
+
+    // 1. structure, counts, consumed lengths; 2. their bases, and the totals the later launches are sized from
+    hb::qpack_instruction_scan_kernel<<<flat, 256, 0, st>>>(n, which, in, in_off, B.num_fields.as<uint64_t>(),
+                                                             B.num_lits.as<uint64_t>(), B.lit_bytes.as<uint64_t>(), consumed,
+                                                             B.struct_status.as<int32_t>());
+    ++ctx->launches;
+    if (launch_scan(ctx, ctx->scratch, B.num_fields.as<uint64_t>(), instr_base, n, st)) return AWS_OP_ERR;
+    if (launch_scan(ctx, ctx->scratch, B.num_lits.as<uint64_t>(), lit_base, n, st)) return AWS_OP_ERR;
+    if (launch_scan(ctx, ctx->scratch, B.lit_bytes.as<uint64_t>(), lit_byte_base, n, st)) return AWS_OP_ERR;
+    HB_CUDA_TRY(cudaMemcpyAsync(B.h_totals + 0, instr_base + n, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    HB_CUDA_TRY(cudaMemcpyAsync(B.h_totals + 1, lit_base + n, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    HB_CUDA_TRY(cudaMemcpyAsync(B.h_totals + 2, lit_byte_base + n, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    HB_CUDA_TRY(cudaStreamSynchronize(st));
+    const uint64_t parsed = B.h_totals[0], num_lits = B.h_totals[1], lit_total = B.h_totals[2];
+    const uint64_t kept = std::min(parsed, o.instruction_capacity);  // instruction slots that can be written
+    const uint32_t min_len = std::max<uint32_t>(1, ctx->tables.min_len);
+    const uint64_t dec_cap = lit_total * 8 / min_len + 64;
+    if (stage) {
+        // (an instruction's strings are its decoded literals or an Appendix A name, at most 32 octets)
+        o.strings_capacity = std::min(o.strings_capacity, dec_cap + 32 * kept);
+        HB_CUDA_TRY(B.s_kind.reserve(kept + 1));
+        HB_CUDA_TRY(B.s_index.reserve((kept + 1) * sizeof(uint64_t)));
+        HB_CUDA_TRY(B.s_string_offsets.reserve((2 * kept + 1) * sizeof(uint64_t)));
+        HB_CUDA_TRY(ctx->s_out.reserve(o.strings_capacity + 16));
+        o.kind = B.s_kind.as<uint8_t>();
+        o.index = B.s_index.as<uint64_t>();
+        o.string_offsets = B.s_string_offsets.as<uint64_t>();
+        o.strings = ctx->s_out.as<uint8_t>();
+    }
+    HB_CUDA_TRY(B.f_kind.reserve(parsed + 1));
+    HB_CUDA_TRY(B.f_index.reserve((parsed + 1) * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.f_block.reserve((parsed + 1) * sizeof(uint32_t)));
+    HB_CUDA_TRY(B.f_lits.reserve((2 * parsed + 1) * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.lit_src.reserve((num_lits + 1) * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.lit_len.reserve((num_lits + 1) * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.lit_offsets.reserve((num_lits + 1) * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.lit_status.reserve((num_lits + 1) * sizeof(int32_t)));
+    HB_CUDA_TRY(B.dec_offsets.reserve((num_lits + 1) * sizeof(uint64_t)));
+    uint8_t *f_kind = B.f_kind.as<uint8_t>();
+    uint64_t *f_index = B.f_index.as<uint64_t>(), *f_lits = B.f_lits.as<uint64_t>();
+    uint32_t *f_block = B.f_block.as<uint32_t>();
+    uint64_t *dec_offsets = B.dec_offsets.as<uint64_t>();
+    int32_t *lit_status = B.lit_status.as<int32_t>();
+
+    // 3. instruction records and literals in parsed order; 4. the literals, packed and re-framed as RFC 7541 5.2
+    // literals; 5. decoded by the literal path (a decoder-stream batch has no literals)
+    if (parsed || num_lits) {
+        hb::qpack_instruction_split_kernel<<<flat, 256, 0, st>>>(
+            n, which, in, in_off, instr_base, lit_base, lit_byte_base, f_kind, f_index, f_block, f_lits,
+            B.lit_src.as<uint64_t>(), B.lit_len.as<uint64_t>(), B.lit_offsets.as<uint64_t>());
+        ++ctx->launches;
+    }
+    if (num_lits) {
+        HB_CUDA_TRY(B.lits.reserve(lit_total + 64));
+        HB_CUDA_TRY(B.dec.reserve(dec_cap + 64));
+        hb::qpack_lit_gather_kernel<<<grid_of(num_lits, 256), 256, 0, st>>>(
+            num_lits, in, B.lit_src.as<uint64_t>(), B.lit_len.as<uint64_t>(), B.lit_offsets.as<uint64_t>(), B.lits.as<uint8_t>());
+        ++ctx->launches;
+        if (hpack_decode_on_device(ctx, num_lits, B.lits.as<uint8_t>(), B.lit_offsets.as<uint64_t>(), lit_total,
+                                   B.dec.as<uint8_t>(), dec_cap, dec_offsets, lit_status, st))
+            return AWS_OP_ERR;
+    }
+    // 6. final status per chunk, consumed lengths, instruction offsets; 7. records, string lengths, string offsets,
+    // strings
+    hb::hpack_block_finish_kernel<<<flat, 256, 0, st>>>(
+        n, lit_base, lit_status, B.struct_status.as<int32_t>(), B.num_fields.as<uint64_t>(), status, B.out_fields.as<uint64_t>());
+    ++ctx->launches;
+    hb::qpack_instruction_consumed_kernel<<<flat, 256, 0, st>>>(n, status, consumed);
+    ++ctx->launches;
+    if (launch_scan(ctx, ctx->scratch, B.out_fields.as<uint64_t>(), o.instruction_offsets, n, st)) return AWS_OP_ERR;
+    if (!kept) {
+        HB_CUDA_TRY(cudaMemsetAsync(o.string_offsets, 0, sizeof(uint64_t), st));
+        HB_CUDA_TRY(cudaGetLastError());
+        return AWS_OP_SUCCESS;
+    }
+    HB_CUDA_TRY(B.str_lens.reserve(2 * kept * sizeof(uint64_t)));
+    HB_CUDA_TRY(cudaMemsetAsync(B.str_lens.ptr, 0, 2 * kept * sizeof(uint64_t), st));
+    const uint8_t *dec = B.dec.as<uint8_t>();
+    hb::hpack_field_records_kernel<hb::QpackInstructionStrings><<<grid_of(parsed, 256), 256, 0, st>>>(
+        parsed, f_kind, f_index, f_block, f_lits, instr_base, status, o.instruction_offsets, o.instruction_capacity, dec,
+        dec_offsets, o.kind, o.index, B.str_lens.as<uint64_t>());
+    ++ctx->launches;
+    if (launch_scan(ctx, ctx->scratch, B.str_lens.as<uint64_t>(), o.string_offsets, 2 * kept, st)) return AWS_OP_ERR;
+    hb::hpack_compose_kernel<hb::QpackInstructionStrings><<<grid_of(2 * parsed, 256), 256, 0, st>>>(
+        parsed, f_kind, f_index, f_block, f_lits, instr_base, status, o.instruction_offsets, o.instruction_capacity, dec,
+        dec_offsets, o.strings, o.strings_capacity, o.string_offsets);
+    ++ctx->launches;
+    HB_CUDA_TRY(cudaGetLastError());
+    return AWS_OP_SUCCESS;
+}
+
+// The caller's instructions (kind, index; names and values on the encoder stream) into n chunks of the stream `which`,
+// with the per-chunk status (optional) of aws_qpack_instruction_encode_batch.
+int qpack_instructions_encode_on_device(
+    aws_huffman_batch_ctx *ctx, uint32_t which, uint64_t n, const uint64_t *instruction_offsets, uint64_t num_instr,
+    const uint8_t *kind, const uint64_t *index, const uint8_t *strings, const uint64_t *string_offsets,
+    uint64_t strings_size, uint32_t mode, uint8_t *out, uint64_t out_capacity, uint64_t *out_offsets, int32_t *status,
+    cudaStream_t st) {
+    hb_host::BlockBufs &B = ctx->blk;
+    if (n == 0 || num_instr == 0) {
+        HB_CUDA_TRY(cudaMemsetAsync(out_offsets, 0, (n + 1) * sizeof(uint64_t), st));
+        if (status && n) HB_CUDA_TRY(cudaMemsetAsync(status, 0, n * sizeof(int32_t), st));
+        return AWS_OP_SUCCESS;
+    }
+    const uint64_t F = num_instr;
+    HB_CUDA_TRY(B.plan.reserve(F));
+    HB_CUDA_TRY(B.plan_index.reserve(F * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.field_lens.reserve(F * sizeof(uint64_t)));
+    HB_CUDA_TRY(B.field_pos.reserve((F + 1) * sizeof(uint64_t)));
+    uint64_t *field_pos = B.field_pos.as<uint64_t>();
+    const uint8_t *framed = nullptr;
+    const uint64_t *framed_offsets = nullptr;
+    // 1. every name and value framed (encoder stream: the decoder stream sends no literals); 2. instruction and size;
+    // 3. the chunk rule; 4. wire positions of instructions and chunks; 5. the instructions
+    if (which == 0) {
+        const uint64_t expand = mode == hb::kHpackAlways ? (std::max<uint32_t>(1, ctx->tables.max_len) + 7) / 8 : 1;
+        const uint64_t framed_cap = strings_size * expand + 2 * F * 10 + 64;
+        HB_CUDA_TRY(B.framed.reserve(framed_cap + 64));
+        HB_CUDA_TRY(B.framed_offsets.reserve((2 * F + 1) * sizeof(uint64_t)));
+        framed = B.framed.as<uint8_t>();
+        framed_offsets = B.framed_offsets.as<uint64_t>();
+        if (hpack_encode_on_device(ctx, 2 * F, strings, string_offsets, strings_size, mode, B.framed.as<uint8_t>(),
+                                   framed_cap, B.framed_offsets.as<uint64_t>(), st))
+            return AWS_OP_ERR;
+    }
+    hb::qpack_instruction_plan_kernel<<<grid_of(F, 256), 256, 0, st>>>(
+        F, which, strings, string_offsets, kind, index, framed, framed_offsets, B.plan.as<uint8_t>(),
+        B.plan_index.as<uint64_t>(), B.field_lens.as<uint64_t>());
+    ++ctx->launches;
+    hb::qpack_instruction_check_kernel<<<grid_of(n, 256), 256, 0, st>>>(n, instruction_offsets, B.plan.as<uint8_t>(),
+                                                                         B.field_lens.as<uint64_t>(), status);
+    ++ctx->launches;
+    if (launch_scan(ctx, ctx->scratch, B.field_lens.as<uint64_t>(), field_pos, F, st)) return AWS_OP_ERR;
+    hb::hpack_block_offsets_kernel<<<grid_of(n + 1, 256), 256, 0, st>>>(n, instruction_offsets, field_pos, out_offsets);
+    ++ctx->launches;
+    hb::qpack_field_emit_kernel<hb::QpackInstructionLines><<<grid_of(F, 256), 256, 0, st>>>(
+        F, B.plan.as<uint8_t>(), B.plan_index.as<uint64_t>(), framed, framed_offsets, field_pos, out, out_capacity);
+    ++ctx->launches;
+    HB_CUDA_TRY(cudaGetLastError());
+    return AWS_OP_SUCCESS;
+}
+
+// The argument rules of the instruction calls that need no device memory read. Decode writes kind, index, strings and
+// string_offsets; encode reads kind and index, and on the encoder stream string_offsets.
+int check_instruction_lists(const aws_qpack_instructions *l, uint32_t which, bool decode) {
+    if (!l || which > 1 || (l->n && !l->instruction_offsets) || l->n > 0xffffffffull)
+        return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    if (decode && (!l->string_offsets || (l->instruction_capacity && (!l->kind || !l->index)) ||
+                   (l->strings_capacity && !l->strings)))
+        return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    if (!decode && (!l->kind || !l->index || (which == 0 && !l->string_offsets)))
+        return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    return AWS_OP_SUCCESS;
+}
+
+// Host pointers, run on the device (the way qpack_sections_decode_slice does): the n chunks are staged and decoded
+// into the context's staging, within the capacities given; size[0] receives their instructions and, when those fit
+// instruction_capacity, size[1] their string octets.
+int qpack_instructions_decode_slice(
+    aws_huffman_batch_ctx *ctx, uint32_t which, size_t n, const uint8_t *in, const uint64_t *in_off,
+    uint64_t instruction_capacity, uint64_t strings_capacity, uint64_t size[2], cudaStream_t st) {
+    hb_host::BlockBufs &B = ctx->blk;
+    const uint64_t total_in = in_off[n];
+    const uint8_t *d_in = nullptr;
+    uint64_t *d_in_off = nullptr, *d_consumed = nullptr;
+    aws_qpack_instructions o{};
+    o.n = n;
+    o.instruction_capacity = instruction_capacity;
+    o.strings_capacity = strings_capacity;
+    if (stage_in(ctx->s_in, total_in + 16, in, total_in, st, &d_in) ||
+        stage_in(ctx->s_in_off, (n + 1) * sizeof(uint64_t), in_off, n + 1, st, &d_in_off) ||
+        stage_in(B.s_field_offsets, (n + 1) * sizeof(uint64_t), (const uint64_t *)nullptr, 0, st, &o.instruction_offsets) ||
+        stage_in(ctx->s_consumed, n * sizeof(uint64_t), (const uint64_t *)nullptr, 0, st, &d_consumed))
+        return AWS_OP_ERR;
+    HB_CUDA_TRY(ctx->s_status.reserve(n * sizeof(int32_t)));
+    if (qpack_instructions_decode_on_device(ctx, which, n, d_in, d_in_off, o, d_consumed, ctx->s_status.as<int32_t>(),
+                                            true, st) ||
+        read_back(o.instruction_offsets + n, &size[0], st))
+        return AWS_OP_ERR;
+    size[1] = 0;  // (string offsets exist for the instructions that fit)
+    return size[0] <= instruction_capacity ? read_back(B.s_string_offsets.as<uint64_t>() + 2 * size[0], &size[1], st)
+                                           : AWS_OP_SUCCESS;
+}
+
+// Host pointers, finish into place: consumed lengths, offsets and status first (complete on AWS_ERROR_SHORT_BUFFER),
+// then the records and strings.
+int qpack_instructions_decode_finish(
+    aws_huffman_batch_ctx *ctx, size_t n, const uint64_t size[2], aws_qpack_instructions *out, uint64_t *consumed,
+    int32_t *status, cudaStream_t st) {
+    hb_host::BlockBufs &B = ctx->blk;
+    const uint64_t instr = size[0];
+    HB_CUDA_TRY(cudaMemcpyAsync(consumed, ctx->s_consumed.ptr, n * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    if (finish_slice(ctx, st, n, true, B.s_field_offsets.as<uint64_t>(), out->instruction_offsets, 0, nullptr, nullptr, 0,
+                     instr, out->instruction_capacity, ctx->s_status.as<int32_t>(), status) ||
+        finish_slice(ctx, st, 2 * instr, true, B.s_string_offsets.as<uint64_t>(), out->string_offsets, 0, ctx->s_out.ptr,
+                     out->strings, size[1], size[1], out->strings_capacity))
+        return AWS_OP_ERR;
+    if (instr) {
+        HB_CUDA_TRY(cudaMemcpyAsync(out->kind, B.s_kind.ptr, instr, cudaMemcpyDeviceToHost, st));
+        HB_CUDA_TRY(cudaMemcpyAsync(out->index, B.s_index.ptr, instr * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    }
+    HB_CUDA_TRY(cudaStreamSynchronize(st));
+    return AWS_OP_SUCCESS;
+}
+
+int qpack_instructions_decode_host(
+    aws_huffman_batch_ctx *ctx, uint32_t which, size_t n, const uint8_t *in, const uint64_t *in_off,
+    aws_qpack_instructions *out, uint64_t *consumed, int32_t *status) {
+    if (!ctx || (n && (!in_off || !consumed)) || check_instruction_lists(out, which, true) || out->n != n)
+        return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    if (n == 0) {
+        out->instruction_offsets[0] = 0;
+        out->string_offsets[0] = 0;
+        return AWS_OP_SUCCESS;
+    }
+    if ((in_off[n] && !in) || !offsets_sorted(in_off, n + 1)) return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    cudaStream_t st;
+    if (call_begin(ctx, nullptr, &st)) return AWS_OP_ERR;
+    uint64_t size[2];
+    int rc = qpack_instructions_decode_slice(ctx, which, n, in, in_off, out->instruction_capacity, out->strings_capacity,
+                                             size, st);
+    if (rc == AWS_OP_SUCCESS) rc = qpack_instructions_decode_finish(ctx, n, size, out, consumed, status, st);
+    return call_end(ctx, st, rc);
+}
+
+// Host pointers: the chunks of `in` are staged and encoded into the context's staging, out_capacity octets at most;
+// *size receives the output size and the status per chunk goes to the staging.
+int qpack_instructions_encode_slice(
+    aws_huffman_batch_ctx *ctx, uint32_t which, const aws_qpack_instructions *in, uint32_t mode, uint64_t out_capacity,
+    uint64_t *size, cudaStream_t st) {
+    const uint64_t n = in->n, F = in->instruction_offsets[n], S = which == 0 ? in->string_offsets[2 * F] : 0;
+    hb_host::BlockBufs &B = ctx->blk;
+    uint64_t *d_offsets = nullptr, *d_string_offsets = nullptr;
+    const uint8_t *d_strings = nullptr, *d_kind = nullptr;
+    const uint64_t *d_index = nullptr;
+    HB_CUDA_TRY(ctx->s_status.reserve(n * sizeof(int32_t)));
+    if (stage_in(B.s_field_offsets, (n + 1) * sizeof(uint64_t), in->instruction_offsets, n + 1, st, &d_offsets) ||
+        stage_in(B.s_kind, F + 1, in->kind, F, st, &d_kind) ||
+        stage_in(B.s_index, (F + 1) * sizeof(uint64_t), in->index, F, st, &d_index) ||
+        (which == 0 && (stage_in(ctx->s_in, S + 16, in->strings, S, st, &d_strings) ||
+                        stage_in(ctx->s_in_off, (2 * F + 1) * sizeof(uint64_t), in->string_offsets, 2 * F + 1, st,
+                                 &d_string_offsets))))
+        return AWS_OP_ERR;
+    HB_CUDA_TRY(ctx->s_out.reserve(out_capacity + 16));
+    HB_CUDA_TRY(ctx->s_out_off.reserve((n + 1) * sizeof(uint64_t)));
+    if (qpack_instructions_encode_on_device(ctx, which, n, d_offsets, F, d_kind, d_index, d_strings, d_string_offsets, S,
+                                            mode, ctx->s_out.as<uint8_t>(), out_capacity, ctx->s_out_off.as<uint64_t>(),
+                                            ctx->s_status.as<int32_t>(), st))
+        return AWS_OP_ERR;
+    return read_back(ctx->s_out_off.as<uint64_t>() + n, size, st);
+}
+
+int qpack_instructions_encode_host(
+    aws_huffman_batch_ctx *ctx, uint32_t which, const aws_qpack_instructions *in, uint32_t mode, uint8_t *out,
+    uint64_t out_capacity, uint64_t *out_off, int32_t *status) {
+    if (!ctx || mode > hb::kHpackAlways || check_instruction_lists(in, which, false) || !out_off ||
+        (out_capacity && !out))
+        return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    const uint64_t n = in->n;
+    if (n == 0) {
+        out_off[0] = 0;
+        return AWS_OP_SUCCESS;
+    }
+    // (instructions are numbered from 0 and every one is encoded: chunks start at instruction 0, strings at octet 0)
+    if (in->instruction_offsets[0] != 0 || !offsets_sorted(in->instruction_offsets, n + 1))
+        return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    const uint64_t F = in->instruction_offsets[n];
+    if (which == 0 && (in->string_offsets[0] != 0 || !offsets_sorted(in->string_offsets, 2 * F + 1) ||
+                       (in->string_offsets[2 * F] && !in->strings)))
+        return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    cudaStream_t st;
+    if (call_begin(ctx, nullptr, &st)) return AWS_OP_ERR;
+    uint64_t size = 0;
+    int rc = qpack_instructions_encode_slice(ctx, which, in, mode, out_capacity, &size, st);
+    if (rc == AWS_OP_SUCCESS &&
+        (finish_slice(ctx, st, n, true, ctx->s_out_off.as<uint64_t>(), out_off, 0, ctx->s_out.ptr, out, size, size,
+                      out_capacity, ctx->s_status.as<int32_t>(), status) ||
          cudaStreamSynchronize(st) != cudaSuccess))
         rc = AWS_OP_ERR;
     return call_end(ctx, st, rc);
@@ -2614,6 +2929,48 @@ int aws_qpack_field_section_encode_records_batch_device(
                                                     in->base_sign, in->delta_base, in->strings, in->string_offsets,
                                                     strings_size, (uint32_t)mode, out, out_capacity, out_offsets, status,
                                                     st));
+}
+
+int aws_qpack_instruction_decode_batch(
+    struct aws_huffman_batch_ctx *ctx, enum aws_qpack_instruction_stream which, size_t n, const uint8_t *in,
+    const uint64_t *in_offsets, struct aws_qpack_instructions *out, uint64_t *consumed, int32_t *status) {
+    return qpack_instructions_decode_host(ctx, (uint32_t)which, n, in, in_offsets, out, consumed, status);
+}
+
+int aws_qpack_instruction_encode_batch(
+    struct aws_huffman_batch_ctx *ctx, enum aws_qpack_instruction_stream which, const struct aws_qpack_instructions *in,
+    enum aws_hpack_huffman_mode mode, uint8_t *out, uint64_t out_capacity, uint64_t *out_offsets, int32_t *status) {
+    return qpack_instructions_encode_host(ctx, (uint32_t)which, in, (uint32_t)mode, out, out_capacity, out_offsets, status);
+}
+
+int aws_qpack_instruction_decode_batch_device(
+    struct aws_huffman_batch_ctx *ctx, enum aws_qpack_instruction_stream which, size_t n, const uint8_t *in,
+    const uint64_t *in_offsets, uint64_t in_size, struct aws_qpack_instructions *out, uint64_t *consumed, int32_t *status,
+    void *cuda_stream) {
+    if (!ctx || (n && (!in_offsets || !consumed)) || (in_size && !in) || check_instruction_lists(out, (uint32_t)which, true) ||
+        out->n != n)
+        return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    cudaStream_t st;
+    if (call_begin(ctx, cuda_stream, &st)) return AWS_OP_ERR;
+    return call_end(ctx, st, qpack_instructions_decode_on_device(ctx, (uint32_t)which, n, in, in_offsets, *out, consumed,
+                                                                 status, false, st));
+}
+
+int aws_qpack_instruction_encode_batch_device(
+    struct aws_huffman_batch_ctx *ctx, enum aws_qpack_instruction_stream which, const struct aws_qpack_instructions *in,
+    uint64_t num_instructions, uint64_t strings_size, enum aws_hpack_huffman_mode mode, uint8_t *out,
+    uint64_t out_capacity, uint64_t *out_offsets, int32_t *status, void *cuda_stream) {
+    if (!ctx || check_instruction_lists(in, (uint32_t)which, false) || !out_offsets || (out_capacity && !out) ||
+        (which == AWS_QPACK_ENCODER_STREAM && strings_size && !in->strings) ||
+        (unsigned)mode > (unsigned)AWS_HPACK_HUFFMAN_ALWAYS)
+        return aws_raise_error(AWS_ERROR_INVALID_ARGUMENT);
+    cudaStream_t st;
+    if (call_begin(ctx, cuda_stream, &st)) return AWS_OP_ERR;
+    return call_end(ctx, st,
+                    qpack_instructions_encode_on_device(ctx, (uint32_t)which, in->n, in->instruction_offsets,
+                                                        num_instructions, in->kind, in->index, in->strings,
+                                                        in->string_offsets, which == AWS_QPACK_ENCODER_STREAM ? strings_size : 0,
+                                                        (uint32_t)mode, out, out_capacity, out_offsets, status, st));
 }
 
 int aws_huffman_get_encoded_length_batch(

@@ -201,6 +201,29 @@ __global__ void qpack_section_scan_kernel(uint64_t n, const uint8_t *in, const u
     lit_bytes[b] = nbytes;
 }
 
+// The literal spans of one walked line (or instruction) whose item starts at in[a]: literal l (payload offset into
+// `in`, length << 1 | H, offset of the re-framed literal in the packed batch) for its name and then its value, those
+// read in full; name and value receive their literal ids, or kNoLiteral.
+__device__ __forceinline__ void qpack_split_literals(const SectionField &fd, uint64_t a, uint64_t &l, uint64_t &o,
+                                                     uint64_t *lit_src, uint64_t *lit_len, uint64_t *lit_offsets,
+                                                     uint64_t &name, uint64_t &value) {
+    name = value = kNoLiteral;
+    if (fd.name_lit) {
+        name = l;
+        lit_src[l] = a + fd.name_pay;
+        lit_len[l] = fd.name_len << 1 | fd.name_huff;
+        lit_offsets[l++] = o;
+        o += qpack_reframed_bytes(fd.name_len);
+    }
+    if (fd.value_lit) {
+        value = l;
+        lit_src[l] = a + fd.value_pay;
+        lit_len[l] = fd.value_len << 1 | fd.value_huff;
+        lit_offsets[l++] = o;
+        o += qpack_reframed_bytes(fd.value_len);
+    }
+}
+
 // Pass 2, thread per section, the same walk: field records (kind with the N bit, index, section, the literal ids of
 // name and value) in parsed order from field_base[b], and literals (payload offset into `in`, length << 1 | H, offset
 // of the re-framed literal in the packed batch) from lit_base[b] / lit_byte_base[b].
@@ -213,21 +236,8 @@ __global__ void qpack_section_split_kernel(
     const uint64_t a = in_offsets[b];
     uint64_t f = field_base[b], l = lit_base[b], o = lit_byte_base[b];
     qpack_walk_section(in + a, in_offsets[b + 1] - a, [&](const SectionField &fd) {
-        uint64_t name = kNoLiteral, value = kNoLiteral;
-        if (fd.name_lit) {
-            name = l;
-            lit_src[l] = a + fd.name_pay;
-            lit_len[l] = fd.name_len << 1 | fd.name_huff;
-            lit_offsets[l++] = o;
-            o += qpack_reframed_bytes(fd.name_len);
-        }
-        if (fd.value_lit) {
-            value = l;
-            lit_src[l] = a + fd.value_pay;
-            lit_len[l] = fd.value_len << 1 | fd.value_huff;
-            lit_offsets[l++] = o;
-            o += qpack_reframed_bytes(fd.value_len);
-        }
+        uint64_t name, value;
+        qpack_split_literals(fd, a, l, o, lit_src, lit_len, lit_offsets, name, value);
         if (!fd.complete) return;
         f_kind[f] = fd.kind | (fd.never ? kQNeverBit : 0);
         f_index[f] = fd.index;
@@ -326,6 +336,22 @@ __global__ void qpack_section_prefix_kernel(uint64_t n, const uint8_t *in, const
 // payload's length).
 constexpr uint8_t kQPlanNever = 64;
 
+// Record f's name and value (strings[string_offsets[2f] .. string_offsets[2f + 2])) against Appendix A: name_match is
+// the lowest entry with that name, exact the lowest with that name and value (kQpackStaticEntries: none).
+__device__ __forceinline__ void qpack_static_match(const uint8_t *strings, const uint64_t *string_offsets, uint64_t f,
+                                                   uint32_t &name_match, uint32_t &exact) {
+    const uint64_t n0 = string_offsets[2 * f], v0 = string_offsets[2 * f + 1], v1 = string_offsets[2 * f + 2];
+    const uint8_t *name = strings + n0, *value = strings + v0;
+    const uint64_t name_len = v0 - n0, value_len = v1 - v0;
+    name_match = exact = kQpackStaticEntries;
+    for (uint32_t e = 0; e < kQpackStaticEntries && exact == kQpackStaticEntries; ++e) {
+        const uint32_t s0 = kQpackStaticOff[2 * e], s1 = kQpackStaticOff[2 * e + 1], s2 = kQpackStaticOff[2 * e + 2];
+        if (s1 - s0 != name_len || !hpack_bytes_equal(name, kQpackStaticBlob + s0, name_len)) continue;
+        if (name_match == kQpackStaticEntries) name_match = e;
+        if (s2 - s1 == value_len && hpack_bytes_equal(value, kQpackStaticBlob + s1, value_len)) exact = e;
+    }
+}
+
 // Thread per field: the line and its size on the wire from the framed literals (framed_offsets: name of field f is
 // framed item 2f, its value 2f + 1). field_kind == NULL: every field is kQAuto; else the caller's kind and
 // field_index[f] as given (ignored for a literal name). Static indices >= 99, unknown kinds and integers that
@@ -341,16 +367,8 @@ __global__ void qpack_field_plan_kernel(
     uint8_t p;
     uint64_t index = 0;
     if (kind == kQAuto) {
-        const uint64_t n0 = string_offsets[2 * f], v0 = string_offsets[2 * f + 1], v1 = string_offsets[2 * f + 2];
-        const uint8_t *name = strings + n0, *value = strings + v0;
-        const uint64_t name_len = v0 - n0, value_len = v1 - v0;
-        uint32_t name_match = kQpackStaticEntries, exact = kQpackStaticEntries;
-        for (uint32_t e = 0; e < kQpackStaticEntries && exact == kQpackStaticEntries; ++e) {
-            const uint32_t s0 = kQpackStaticOff[2 * e], s1 = kQpackStaticOff[2 * e + 1], s2 = kQpackStaticOff[2 * e + 2];
-            if (s1 - s0 != name_len || !hpack_bytes_equal(name, kQpackStaticBlob + s0, name_len)) continue;
-            if (name_match == kQpackStaticEntries) name_match = e;
-            if (s2 - s1 == value_len && hpack_bytes_equal(value, kQpackStaticBlob + s1, value_len)) exact = e;
-        }
+        uint32_t name_match, exact;
+        qpack_static_match(strings, string_offsets, f, name_match, exact);
         if (!never && exact < kQpackStaticEntries) {
             p = kQIndexedStatic;
             index = exact;
@@ -452,9 +470,21 @@ __global__ void qpack_section_place_kernel(uint64_t n, const uint64_t *field_off
     for (uint64_t f = f0; f < f1; ++f) field_pos[f] += shift;
 }
 
-// A warp takes 32 fields: every lane writes its field's first-octet flags and integer, then the warp copies the 32
-// name payloads (re-framed: their H bit and 3-bit-prefix length went into the first octet) and the 32 framed value
-// literals. Fields marked kPlanSkip write nothing. Never writes at or after out + out_capacity.
+// The wire format of field lines for qpack_field_emit_kernel (qpack_instructions.cuh has the instructions'): prefix
+// bits and first-octet flags per plan byte, and the H bit of a name literal, whose length takes the line's prefix.
+struct QpackFieldLines {
+    static constexpr uint8_t kNameHuff = 0x08;
+    __device__ static uint32_t prefix_bits(uint32_t kind) { return qpack_prefix_bits(kind); }
+    __device__ static uint8_t flags(uint8_t plan) {
+        return qpack_prefix_flags(plan & 7) | ((plan & kQPlanNever) ? qpack_never_flag(plan & 7) : 0);
+    }
+};
+
+// A warp takes 32 lines: every lane writes its line's first-octet flags and integer, then the warp copies the 32
+// name payloads (re-framed: their H bit and prefix-integer length went into the first octet) and the 32 framed value
+// literals. Lines marked kPlanSkip write nothing. Never writes at or after out + out_capacity. Lines says what the
+// first octet holds (QpackFieldLines: field lines).
+template <typename Lines>
 __global__ void __launch_bounds__(256) qpack_field_emit_kernel(
     uint64_t num_fields, const uint8_t *plan, const uint64_t *plan_index, const uint8_t *framed,
     const uint64_t *framed_offsets, const uint64_t *field_pos, uint8_t *out, uint64_t out_capacity) {
@@ -466,9 +496,9 @@ __global__ void __launch_bounds__(256) qpack_field_emit_kernel(
         const uint8_t p = plan[f], kind = p & 7;
         const uint64_t index = plan_index[f];
         uint64_t pos = field_pos[f];
-        uint8_t flags = qpack_prefix_flags(kind) | ((p & kQPlanNever) ? qpack_never_flag(kind) : 0);
-        if ((p & kPlanNameLit) && (framed[framed_offsets[2 * f]] & 0x80)) flags |= 0x08;
-        const uint32_t prefix_bits = qpack_prefix_bits(kind);
+        uint8_t flags = Lines::flags(p);
+        if ((p & kPlanNameLit) && (framed[framed_offsets[2 * f]] & 0x80)) flags |= Lines::kNameHuff;
+        const uint32_t prefix_bits = Lines::prefix_bits(kind);
         hpack_put_int(out, pos, out_capacity, index, prefix_bits, flags);
         pos += hpack_int_bytes(index, prefix_bits);
         if (p & kPlanNameLit) {
